@@ -2,6 +2,7 @@
 """bench.py -- alignment DP cells/s and audio-hours/s of the B200 forced-alignment decoder.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c4|c4j|c5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (emission -> DP -> backtrace/intervals -> compact results on
 the host) over one workload of synthetic logits.
@@ -55,6 +56,7 @@ WORKLOADS = {
 CORPUS_CHUNK_CELLS = 600_000_000     # workspace bound of a corpus chunk (~8000 utterances, ~5.5 GB): measured on
                                      # one B200, 32768 utterances: 9.44 / 8.72 / 8.58 / 8.63 ms per pass with
                                      # chunks of 150M / 300M / 600M / 1200M cells (tools/gpu/r2_chunks2.sh)
+DUMP_SAMPLE = 4096                   # corpus utterances whose results --dump-outputs writes
 
 
 def workload_shapes(name: str, seed: int, corpus: int = 0):
@@ -219,14 +221,16 @@ def run_reference(args, rank, world):
     for _ in range(args.warmup):
         run()
     times = []
-    t_all = time.perf_counter()
     for _ in range(args.steps):
         t0 = time.perf_counter()
         out = run()
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_all > 120:       # bound the whole run to a few minutes
-            break
     assert out["bad"] == 0
+    if args.dump_outputs:
+        seg = segment_slots(out["seg_off"], out["n_seg"])
+        write_outputs(args.dump_outputs, {"status": out["status"], "n_seg": out["n_seg"], "total_conf": out["total_conf"],
+                                          "ph_idx_seq": out["ph_idx_seq"][seg], "ph_time_int": out["ph_time_int"][seg],
+                                          "intervals": out["intervals"].reshape(-1, 2)[seg]})
     k = len(times)
     sec = float(np.sum(times))
     val = cells * k / sec
@@ -265,6 +269,36 @@ def verify_against_oracle(T, S, V, ids_list, head_np, row_off, get_result, sampl
                     "only be a few-ulp near-tie between the two softmax implementations (tests/: tier 2)"}
 
 
+def segment_slots(seg_off, n_seg):
+    """Result-blob slots that hold segments: utterance b owns the slots from seg_off[b] on, and the first n_seg[b]
+    of them are written (the rest are not, so they never go into a dump)."""
+    return np.concatenate([np.zeros(0, np.int64)] + [np.arange(o, o + k, dtype=np.int64) for o, k in zip(seg_off, n_seg)])
+
+
+def write_outputs(path, arrays: dict) -> None:
+    """--dump-outputs: DIR/<name>.npy per array; integers are stored as float64 (exactly) so that every file is
+    float32 or float64."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a if a.dtype.kind == "f" else a.astype(np.float64)))
+
+
+def corpus_outputs(cp, host, n_utt: int) -> dict:
+    """--dump-outputs of the corpus arm: the results of a fixed, seeded sample of DUMP_SAMPLE utterances (all of
+    them would be hundreds of MB at the default corpus size)."""
+    from hubertfa_b200.corpus import read_results
+    utt = np.sort(np.random.default_rng(0).choice(n_utt, size=min(n_utt, DUMP_SAMPLE), replace=False))
+    res = read_results(cp, host, utt)
+    r = [res[int(b)] for b in utt]
+    return {"utterance": utt, "status": [x["status"] for x in r], "n_seg": [len(x["ph_idx_seq"]) for x in r],
+            "final_score": np.array([x["final_score"] for x in r], np.float32),
+            "total_conf": np.array([x["total_conf"] for x in r], np.float32),
+            "ph_idx_seq": np.concatenate([x["ph_idx_seq"] for x in r]),
+            "ph_time_int": np.concatenate([x["ph_time_int"] for x in r]),
+            "intervals": np.concatenate([x["intervals"] for x in r])}
+
+
 def kernel_source_stamp():
     h = hashlib.sha1()
     for f in ("hfa_dp.cu", "hfa_dp_skew.cu", "hfa_common.cuh"):
@@ -289,6 +323,9 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--e2e-chunks", type=int, default=0,
                     help="equal-sized upload/compute chunks of the e2e leg (0: the library's default shares)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / "
+                         "float64; the corpus workload: a fixed sample of %d utterances)" % DUMP_SAMPLE)
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -296,6 +333,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.steps is None:
         args.steps = 400 if max(world, args.gpus) <= 1 else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup is None:
         args.warmup = 10 if max(world, args.gpus) <= 1 else 3
     if args.impl == "reference":
@@ -346,7 +385,7 @@ def main():
     # -----------------------------------------------------------------------------------------
     # one ragged batch (configs[0..3]): every rank aligns its own batch of the same shape
     # -----------------------------------------------------------------------------------------
-    def measure_batch(workload: str, steps: int, warmup: int, do_e2e: bool, seed_rank: int):
+    def measure_batch(workload: str, steps: int, warmup: int, do_e2e: bool, seed_rank: int, dump: bool = False):
         seed = synth.SEED0 + 100003 * seed_rank
         T, S, V, desc = workload_shapes(workload, seed)
         ids_list = synth.make_ids_batch(T, S, V, seed=seed)
@@ -446,6 +485,11 @@ def main():
         kk = (steps - 1) % n_sets
         v = plan.views(host_res[kk].numpy())
         assert (v["status"] == 0).all() and (v["n_seg"] > 0).all()
+        outputs = None
+        if dump:
+            seg = segment_slots(plan.seg_off[:-1], v["n_seg"])
+            outputs = {k: v[k].copy() for k in ("status", "n_seg", "end_state", "final_score", "total_conf")}
+            outputs.update({k: v[k][seg] for k in ("ph_idx_seq", "ph_time_int", "intervals")})
         verified = None
         if rank == 0:
             sample = np.unique(np.linspace(0, len(T) - 1, min(16, len(T))).astype(np.int64))
@@ -500,7 +544,7 @@ def main():
                     launches=launches_per_step * steps,
                     launch_mode=("cuda graph replay, one launch per step" if use_graph
                                  else "eager launches, result download on a side stream"),
-                    e2e=e2e, alg=alg, alg_8d=alg_8d, design=design, verified=verified, n_sets=n_sets,
+                    e2e=e2e, alg=alg, alg_8d=alg_8d, design=design, verified=verified, n_sets=n_sets, outputs=outputs,
                     bytes_per_set=int(heads_host[0].numel() * 4 + plan.workspace_bytes))
 
     def roofline(m, wl):
@@ -555,7 +599,8 @@ def main():
     # -----------------------------------------------------------------------------------------
     # the corpus (configs[4]): sharded by cost, chunked, gathered on rank 0's host
     # -----------------------------------------------------------------------------------------
-    def measure_corpus(n_utt: int, steps: int, warmup: int, ranks: int, my_rank: int, do_e2e: bool, tag: str):
+    def measure_corpus(n_utt: int, steps: int, warmup: int, ranks: int, my_rank: int, do_e2e: bool, tag: str,
+                       dump: bool = False):
         """ranks = 1: this process alone runs the whole corpus (the strong-scaling reference)."""
         from hubertfa_b200.corpus import CorpusAligner, CorpusPlan, SharedHostBuffer, all_status_ok, read_results
         T, S, V, desc = workload_shapes("c5", synth.SEED0, n_utt)
@@ -615,6 +660,8 @@ def main():
             sample = np.unique(np.linspace(0, n_utt - 1, 24).astype(np.int64))
             out["results"] = read_results(cp, host, sample)
             out["sample"] = sample
+            if dump:          # before the e2e leg below writes its own passes into the same host segment
+                out["outputs"] = corpus_outputs(cp, host, n_utt)
             sub_rows = torch.cat([head[row_off[b]:row_off[b + 1]] for b in sample]).cpu().numpy()
             sub_off = np.concatenate([[0], np.cumsum(T[sample].astype(np.int64))])
             res = out["results"]
@@ -685,7 +732,9 @@ def main():
     # =========================================================================================
     if world == 1 and (args.workload or "c2") != "c5":
         wl = args.workload or "c2"
-        m = measure_batch(wl, args.steps, args.warmup, do_e2e=True, seed_rank=0)
+        m = measure_batch(wl, args.steps, args.warmup, do_e2e=True, seed_rank=0, dump=bool(args.dump_outputs))
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, m["outputs"])
         sec = m["ms"] * 1e-3
         m["e2e"]["value"] = m["cells"] * args.steps / m["e2e"].pop("seconds")
         line = {
@@ -737,7 +786,8 @@ def main():
         return
 
     # ---- the corpus arm: N ranks (or --workload c5 on one GPU) ----
-    c = measure_corpus(args.corpus, args.steps, args.warmup, world, rank, do_e2e=True, tag="m")
+    c = measure_corpus(args.corpus, args.steps, args.warmup, world, rank, do_e2e=True, tag="m",
+                       dump=bool(args.dump_outputs))
     cp = c["cp"]
     sec = c["ms"] * 1e-3
     line = None
@@ -760,6 +810,8 @@ def main():
             "clocks": c["clk"], "e2e": c["e2e"], "gpu_launches": int(c["launches"]),
             "all_status_ok": c["ok"], "verified": c["verified"], "cpu_baseline": None,
         }
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, c["outputs"])
     first = c.get("results")
     sample = c.get("sample")
     c["host"].close()

@@ -8,6 +8,9 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+
+from golden_format import unpack_prob_log  # noqa: E402
 
 
 def pytest_configure(config):
@@ -40,6 +43,7 @@ class Golden:
     def case(self, name):
         m = next(x for x in self.meta if x["name"] == name)
         d = {k.split("/", 1)[1]: self.z[k] for k in self.z.files if k.startswith(name + "/")}
+        d["prob_log"] = unpack_prob_log(d["frame"], d["ids"], d.pop("prob_log_offset"), d.pop("prob_log_xor"))
         d["meta"] = m
         return d
 

@@ -1,11 +1,14 @@
 """Generates tests/golden/reference_cases.npz by running the UNMODIFIED reference decoder
-(/root/reference/tools/alignment_decoder.py, imported with a matplotlib stub) on seeded synthetic
-logits.  Only runs where the reference tree exists (the build container):
+(tools/alignment_decoder.py of the reference tree, see oracle/reference_import.py; imported with a
+matplotlib stub) on seeded synthetic logits.  Only runs where the reference tree exists:
 
     PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
 
 Every case stores its inputs (so nothing depends on RNG reproducibility), the reference's values at
-the `_decode` boundary (ph_prob_log gathered by ph_seq_id, edge_prob) and every output of `decode`.
+the `_decode` boundary (ph_prob_log gathered by ph_seq_id, in the compact form of
+golden_format.pack_prob_log; edge_prob) and every output of `decode`.  The ctc logits are not stored: the
+test of `ctc()` draws them again from the case's seed and first checks that the same draw reproduces
+the stored frame and edge logits.
 """
 import json
 import os
@@ -17,6 +20,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 
+from golden_format import pack_prob_log  # noqa: E402  (next to this script)
 from hubertfa_b200 import synth  # noqa: E402
 from oracle.reference_import import load_reference_decoder  # noqa: E402
 
@@ -89,7 +93,8 @@ def main():
         out[pre + "edge"] = edge[0].numpy()
         out[pre + "ctc_argmax"] = dec.ctc().astype(np.int64)
         out[pre + "ids"] = ids.astype(np.int32)
-        out[pre + "prob_log"] = np.ascontiguousarray(captured["ph_prob_log"][:, ids])  # ad:239
+        packed = pack_prob_log(frame[0].numpy(), captured["ph_prob_log"][:, ids], ids)      # ad:239
+        out.update({pre + k: v for k, v in packed.items()})
         out[pre + "edge_prob"] = captured["edge_prob"]
         out[pre + "ph_seq_pred"] = np.asarray(r[0]).astype("U")
         out[pre + "ph_intervals_pred"] = np.asarray(r[1], dtype=np.float64)
@@ -106,7 +111,7 @@ def main():
         out[pre + "plot_ph_intervals_int"] = np.asarray(a[2]).astype(np.int32)
         out[pre + "plot_ph_idx_frame"] = np.asarray(a[5]).astype(np.int64)
         out[pre + "plot_ph_frame_prob_sum"] = np.asarray(a[4], dtype=np.float64).sum(axis=0)   # [S]: a digest of [T, S]
-        meta.append(dict(name=name, T=T, S=S, V=V, style=style, planted=planted, hop=hop, sr=sr,
+        meta.append(dict(name=name, seed=9000 + ci, T=T, S=S, V=V, style=style, planted=planted, hop=hop, sr=sr,
                          wav_length=wav_length, ph_seq=ph_seq, word_seq=word_seq,
                          ph_idx_to_word_idx=[int(x) for x in ph2w]))
         print(name, "segments", len(dec.ph_idx_seq), "conf", float(r[4]))

@@ -1,6 +1,6 @@
 """CPU: both oracles reproduce the reference outputs stored in tests/golden (and the live reference
-where /root/reference exists).  This is what pins the oracle; the GPU tests then compare the CUDA
-path with the oracle."""
+where its tree is provided, see oracle/reference_import.py).  This is what pins the oracle; the GPU
+tests then compare the CUDA path with the oracle."""
 import numpy as np
 import pytest
 import torch
@@ -100,6 +100,19 @@ def test_c_oracle_batch_driver_matches_single(golden):
         r = oc.decode(c["ids"], e, el, ne)
         assert np.array_equal(out["ph_idx_seq"][o:o + k], r["ph_idx_seq"])
         assert np.array_equal(out["ph_time_int"][o:o + k], r["ph_time_int"])
+
+
+@pytest.mark.parametrize("name", golden_names())
+def test_ctc_greedy_matches_golden(golden, name):
+    """The reference's greedy CTC decode (ad:145-150) of its ctc logits, trimmed to the frames it aligned.
+    The logits are drawn again from the case's seed; the same draw must reproduce the stored inputs."""
+    c = golden.case(name)
+    m = c["meta"]
+    frame, edge, ctc = synth.make_logits(m["seed"], m["T"], m["V"], c["ids"], m["planted"])
+    assert np.array_equal(_bits(frame[0].numpy()), _bits(c["frame"]))
+    assert np.array_equal(_bits(edge[0].numpy()), _bits(c["edge"]))
+    T = c["prob_log"].shape[0]
+    assert np.array_equal(onp.ctc_greedy(ctc[0, :T].numpy()), c["ctc_argmax"])
 
 
 @pytest.mark.skipif(load_reference_decoder() is None, reason="reference tree not present")
