@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "libhfa_align.so")
 HFA_OK = 0
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 UTT_OK, UTT_EMPTY, UTT_BAD_ID, UTT_NO_STATES, UTT_INFEASIBLE, UTT_TOO_MANY_STATES = range(6)
-MAX_STATES = 8192
+MAX_STATES = 1 << 20   # include/hfa_align.h HFA_MAX_STATES
 ABI_VERSION = 2
 
 

@@ -288,7 +288,9 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         p->total_states = p->seg_off[n_utt];
         p->ids.assign(ph_ids, ph_ids + p->total_states);
 
-        std::vector<int32_t> lists[HFA_NUM_CLASSES + 1], invalid;
+        // giant: S > HFA_CTA_MAX_S, beyond the CTA kernel -- always in the skewed strips (or halo bands), routed
+        // after everything else so that the other utterances of the batch are placed as if it were not there
+        std::vector<int32_t> lists[HFA_NUM_CLASSES + 1], invalid, giant;
         int64_t emis = 0, edge = 0, words = 0, cells = 0, frames = 0;
         for (int32_t b = 0; b < n_utt; ++b) {
             HfaUtt &m = p->utt[b];
@@ -325,6 +327,7 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                 p->row_blocks[b + 1] = p->row_blocks[b] + (t + HFA_EMIS_ROWS - 1) / HFA_EMIS_ROWS;
                 p->max_sp = std::max(p->max_sp, m.Sp);
                 if (m.Sp <= HFA_WARP_MAX_S) lists[(m.Sp + 31) / 32 - 1].push_back(b);
+                else if (s > HFA_CTA_MAX_S) giant.push_back(b);
                 else {
                     lists[HFA_NUM_CLASSES].push_back(b);
                     p->cta_max_sp = std::max(p->cta_max_sp, m.Sp);
@@ -353,6 +356,7 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
             p->order.insert(p->order.end(), lists[c].begin(), lists[c].end());
             all.insert(all.end(), lists[c].begin(), lists[c].end());
         }
+        all.insert(all.end(), giant.begin(), giant.end());
         // Routing.  The recurrence is a serial chain in t, so a batch that cannot fill the machine
         // with one warp per utterance (BASELINE configs 1-3) is bounded by the per-frame latency of
         // its longest utterances.  Such batches go to the banded kernel (hfa_dp_band_kernel): every
@@ -459,6 +463,18 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                 big_band = lists[HFA_NUM_CLASSES];
                 lists[HFA_NUM_CLASSES].clear();
                 p->class_count[HFA_NUM_CLASSES] = 0;
+            }
+            // The giants join that list whatever the budget.  When it is otherwise empty (the other long
+            // utterances, if any, stay in the CTA kernel) it becomes strips, or 2-states-per-lane halo bands
+            // without tensor maps.  When it already holds the batch's other long utterances it keeps their kernel:
+            // strips, or halo bands if those won the budget or HFA_BIG_K / the missing tensor maps chose them.
+            if (!giant.empty()) {
+                if (big_band.empty()) {
+                    p->band_k[1] = skew_d > 0 ? 1 : 2;
+                    p->band_skew[1] = skew_d;
+                }
+                big_band.insert(big_band.end(), giant.begin(), giant.end());
+                std::sort(big_band.begin(), big_band.end(), by_len);
             }
         }
         bool keep_dp = true;
@@ -1007,7 +1023,9 @@ static bool fused_ok(const hfa_plan *p, const void *workspace, int32_t dtype)
     const bool all_banded = p->warp_all_count == 0 &&
                             p->class_count[HFA_NUM_CLASSES] == 0 && !p->band_items.empty();
     const bool skewed = p->band_skew[0] > 0 || p->band_skew[1] > 0;   // no producer warp there to fuse into
-    return all_banded && !skewed && p->dp_store_elems > 0 && dtype == HFA_DTYPE_F32 && max_row_stride > 0 &&
+    // max_sp: the fused band kernel is not shown to handle utterances beyond the CTA kernel's range
+    return all_banded && !skewed && p->max_sp <= HFA_CTA_MAX_S && p->dp_store_elems > 0 && dtype == HFA_DTYPE_F32 &&
+           max_row_stride > 0 &&
            p->vocab <= 256 && max_row_stride * 4 * HFA_TILE_T <= 48 * 1024;
 }
 

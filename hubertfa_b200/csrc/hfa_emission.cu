@@ -49,6 +49,18 @@ __device__ __forceinline__ float lds_f32(uint32_t addr)
     return v;
 }
 
+// The emission kernels stage an utterance's ids in shared memory for at most this many states (sp_cap =
+// min(largest Sp of the batch, HFA_EMIS_ID_CAP)), so one long utterance cannot lower the occupancy of its whole
+// batch.  The ids of the states past the staged ones (S > HFA_CTA_MAX_S only) are read from global memory.
+#define HFA_EMIS_ID_CAP 8192
+
+// ids of states s4 .. s4 + 3 (pads past S -> V), straight from global memory
+__device__ __forceinline__ int4 hfa_ids4(const int32_t *ids, int S, int V, int s4)
+{
+    return make_int4(s4 < S ? __ldg(ids + s4) : V, s4 + 1 < S ? __ldg(ids + s4 + 1) : V,
+                     s4 + 2 < S ? __ldg(ids + s4 + 2) : V, s4 + 3 < S ? __ldg(ids + s4 + 3) : V);
+}
+
 // One edge logit per frame out of a [T, V+2] head output is a 4-byte load every row stride: by default the L2
 // fetches the whole 128-byte line around it from HBM (ncu, config 4: 460 MB read for 3.7 M frames).  The 64-byte
 // fetch-granularity hint is the smallest PTX offers; the rest of the line belongs to the emission kernel's copy.
@@ -159,7 +171,7 @@ hfa_emission_block_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
     const int32_t *ids = compact ? ws.col_ids + m.seg_off + 4 * (int64_t)u : ws.ids + m.seg_off;
     for (int s = tid; s < Sp; s += blockDim.x) {
         const int id = (s < S) ? ids[s] : V;
-        ids_sm[s] = id;
+        if (s < sp_cap) ids_sm[s] = id;
         if (id < V) atomicOr(&mask_sm[id >> 5], 1u << (id & 31));
     }
     __syncthreads();
@@ -225,11 +237,21 @@ hfa_emission_block_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
             }
         }
         if (Sp > 256) {                                                      // long phoneme sequences
+            const int s_sm = min(Sp, sp_cap);
             for (int r = 0; r < rows_here; ++r) {
                 const int rr = warp + HFA_EMIS_WARPS * r;
                 const float2 st = stat_sm[rr];
-                for (int s4 = lane * 4 + 256; s4 < Sp; s4 += 128) {
+                for (int s4 = lane * 4 + 256; s4 < s_sm; s4 += 128) {
                     const int4 id4 = *reinterpret_cast<const int4 *>(ids_sm + s4);
+                    float4 o;
+                    o.x = __fsub_rn(__fsub_rn(xs[rr * VP + id4.x], st.x), st.y);
+                    o.y = __fsub_rn(__fsub_rn(xs[rr * VP + id4.y], st.x), st.y);
+                    o.z = __fsub_rn(__fsub_rn(xs[rr * VP + id4.z], st.x), st.y);
+                    o.w = __fsub_rn(__fsub_rn(xs[rr * VP + id4.w], st.x), st.y);
+                    *reinterpret_cast<float4 *>(dst + r * dst_step + (s4 - lane * 4)) = o;
+                }
+                for (int s4 = lane * 4 + s_sm; s4 < Sp; s4 += 128) {        // past the staged ids
+                    const int4 id4 = hfa_ids4(ids, S, V, s4);
                     float4 o;
                     o.x = __fsub_rn(__fsub_rn(xs[rr * VP + id4.x], st.x), st.y);
                     o.y = __fsub_rn(__fsub_rn(xs[rr * VP + id4.y], st.x), st.y);
@@ -361,7 +383,7 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
             const int32_t *ids = compact ? ws.col_ids + m.seg_off + 4 * (int64_t)u : ws.ids + m.seg_off;
             for (int q = tid; q < Sp; q += blockDim.x) {
                 const int id = (q < S) ? ids[q] : V;
-                ids_sm[q] = id;
+                if (q < sp_cap) ids_sm[q] = id;
                 if (id < V) atomicOr(&mask_sm[id >> 5], 1u << (id & 31));
             }
             if (compact && tid == 0 && blk == ws.row_blocks[u]) ws.emis_mode[u] = 1;
@@ -479,16 +501,28 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
             }
             }
             if (Sp > 256) {                                                  // long phoneme sequences
+                const int s_sm = min(Sp, sp_cap);
                 for (int r = 0; r < rows_here; ++r) {
                     const int rr = RPW * warp + r;
                     const float2 st = stat_sm[rr];
                     const TIn *row = xs + rr * row_st;
-                    for (int s4 = lane * 4 + 256; s4 < Sp; s4 += 128) {
+                    for (int s4 = lane * 4 + 256; s4 < s_sm; s4 += 128) {
                         const int4 id4 = *reinterpret_cast<const int4 *>(ids_sm + s4);
                         float4 o;
                         o.x = val(row, (uint32_t)id4.x, st); o.y = val(row, (uint32_t)id4.y, st);
                         o.z = val(row, (uint32_t)id4.z, st); o.w = val(row, (uint32_t)id4.w, st);
                         *reinterpret_cast<float4 *>(dst + r * dst_step + (s4 - lane * 4)) = o;
+                    }
+                    if (Sp > s_sm) {                                         // past the staged ids
+                        const int32_t *ids = m.Dp > 0 ? ws.col_ids + m.seg_off + 4 * (int64_t)cur_u
+                                                      : ws.ids + m.seg_off;
+                        for (int s4 = lane * 4 + s_sm; s4 < Sp; s4 += 128) {
+                            const int4 id4 = hfa_ids4(ids, S, V, s4);
+                            float4 o;
+                            o.x = val(row, (uint32_t)id4.x, st); o.y = val(row, (uint32_t)id4.y, st);
+                            o.z = val(row, (uint32_t)id4.z, st); o.w = val(row, (uint32_t)id4.w, st);
+                            *reinterpret_cast<float4 *>(dst + r * dst_step + (s4 - lane * 4)) = o;
+                        }
                     }
                 }
             }
@@ -529,7 +563,7 @@ hfa_emission_wide_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
     const int32_t *ids = compact ? ws.col_ids + m.seg_off + 4 * (int64_t)u : ws.ids + m.seg_off;
     for (int s = tid; s < Sp; s += blockDim.x) {
         const int id = (s < S) ? ids[s] : V;
-        ids_sm[s] = id;
+        if (s < sp_cap) ids_sm[s] = id;
         if (id < V) atomicOr(&mask_sm[id >> 5], 1u << (id & 31));
     }
     __syncthreads();
@@ -555,7 +589,8 @@ hfa_emission_wide_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
         __syncwarp();
         float *dst = g_out + (int64_t)t * Sp;
         for (int s4 = lane * 4; s4 < Sp; s4 += 128) {
-            const int4 id4 = *reinterpret_cast<const int4 *>(ids_sm + s4);
+            const int4 id4 = s4 < sp_cap ? *reinterpret_cast<const int4 *>(ids_sm + s4)
+                                         : hfa_ids4(ids, S, V, s4);           // past the staged ids
             float4 o;
             o.x = __fsub_rn(__fsub_rn(rowbuf[id4.x], mr), l);
             o.y = __fsub_rn(__fsub_rn(rowbuf[id4.y], mr), l);
@@ -583,8 +618,8 @@ hfa_pack_kernel(HfaWs ws, int n_utt, const float *__restrict__ prob_log,
     const float *src = prob_log + m.cell_off + (int64_t)t_base * S;
     float *dst = ws.emis + m.emis_off + (int64_t)t_base * Sp;
     if (m.Dp > 0 && t_base == 0 && tid == 0) ws.emis_mode[u] = 0;     // per-state values: plain rows
-    for (int i = tid; i < rows * Sp; i += blockDim.x) {
-        const int r = i / Sp, s = i - r * Sp;
+    for (int64_t i = tid; i < (int64_t)rows * Sp; i += blockDim.x) {
+        const int r = (int)(i / Sp), s = (int)(i - (int64_t)r * Sp);
         dst[i] = (s < S) ? src[(int64_t)r * S + s] : HFA_NEG_INF;
     }
     if (tid < rows) {
@@ -605,8 +640,8 @@ hfa_unpack_emis_kernel(HfaWs ws, float *__restrict__ out)
     const int t_base = (blockIdx.x - ws.row_blocks[u]) * HFA_EMIS_ROWS;
     const int rows = min(HFA_EMIS_ROWS, m.T - t_base);
     const uint8_t *cm = ws.colmap + m.seg_off;
-    for (int i = threadIdx.x; i < rows * S; i += blockDim.x) {
-        const int r = i / S, s = i - r * S;
+    for (int64_t i = threadIdx.x; i < (int64_t)rows * S; i += blockDim.x) {
+        const int r = (int)(i / S), s = (int)(i - (int64_t)r * S);
         out[m.cell_off + (int64_t)(t_base + r) * S + s] =
             ws.emis[m.emis_off + (int64_t)(t_base + r) * Ep + (compact ? cm[s] : s)];
     }
@@ -627,6 +662,7 @@ static cudaError_t launch_emission_t(const HfaLaunchCtx &c, int blocks, int max_
 {
     *n_launched = 1;
     const int V = c.vocab;
+    max_sp = max_sp < HFA_EMIS_ID_CAP ? max_sp : HFA_EMIS_ID_CAP;      // = sp_cap of the kernels
     cudaError_t e;
     // max_row_stride > 0: every utterance has unit column stride and rows at most that many elements
     // apart -> a 64-row block is one contiguous range and can travel by TMA

@@ -48,13 +48,22 @@ enum {
     HFA_UTT_NO_STATES = 3,   /* S < 1: reference raises IndexError at :250                         */
     HFA_UTT_INFEASIBLE = 4,  /* best path has score -inf (T too short); outputs still follow the
                                 reference (single segment, NaN confidence), flagged for callers    */
-    HFA_UTT_TOO_MANY_STATES = 5 /* S > HFA_MAX_STATES: not covered by the kernels yet              */
+    HFA_UTT_TOO_MANY_STATES = 5 /* S > HFA_MAX_STATES (see there)                                  */
 };
 
 /* element type of the logits handed to hfa_emission (the reference applies .float(), :57,:63,:69) */
 enum { HFA_DTYPE_F32 = 0, HFA_DTYPE_F16 = 1, HFA_DTYPE_BF16 = 2 };
 
-#define HFA_MAX_STATES 8192 /* one CTA of 1024 threads x 8 states; larger S -> HFA_ERR_UNSUPPORTED */
+/* Largest S the library aligns (2^20).  Utterances with S <= HFA_CTA_MAX_S (8192: one CTA of 1024 threads x 8
+ * states) may run in any forward kernel; longer ones always run in the skewed-wavefront strips (halo bands without
+ * TMA tensor maps), whose shared memory does not depend on S.  The bound is what every index provably handles:
+ * state indices, strip / band counts per utterance and the emission, backpointer and exchange row strides
+ * (Sp, 16-frame words x Sp) are int32 and stay below 2^21 here; every offset that multiplies a frame index by
+ * a state count or stride is int64 (cells, emissions, backpointer words, kept dp); the per-utterance kept-dp /
+ * exchange sizes of one utterance (T < 2^31 frames x 2^20 states) fit int64 with room to spare.  Larger S ->
+ * HFA_UTT_TOO_MANY_STATES. */
+#define HFA_MAX_STATES (1 << 20)
+#define HFA_CTA_MAX_S 8192
 
 typedef struct hfa_plan hfa_plan; /* opaque, host side: collation + bucketing of one ragged batch */
 
