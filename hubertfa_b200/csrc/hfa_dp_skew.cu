@@ -14,8 +14,11 @@
 // iteration is just   dp -> FADD -> FADD -> FMNMX -> FMNMX.   The conversions, the f64 add and the
 // shuffles are pipelined work, off the chain.  Cost: T + 31 D iterations per strip instead of T.
 //
-// Mapping.  One warp (= one CTA) per STRIP of 32 columns, one state per lane.  Strip 0 owns states
-// 0..31.  Strip w > 0 starts at column 30 w: lanes 0 and 1 are GHOSTS of the left strip's last two
+// Mapping.  One CTA per STRIP of 32 columns: a compute warp with one state per lane and a producer warp.
+// The compute warp only runs the recurrence: wait for the block's stage (READY), run the block, arrive
+// on DONE.  The producer does everything else off that serial chain -- TMA ring, exchange wait, ghost
+// columns, publication, kept-dp bulk store -- and runs ahead of it.  Strip 0 owns states 0..31.
+// Strip w > 0 starts at column 30 w: lanes 0 and 1 are GHOSTS of the left strip's last two
 // states -- they inject the advance scores the left strip published -- and lanes 2..31 own 30 states.
 // A strip publishes {adv[31](t), adv[30](t)} once per iteration (lane 31 has both in registers) into a
 // per-frame slot in HBM/L2: two 64-bit words {f32 bits | tag << 32}, tag = t + 1, each read and written
@@ -85,7 +88,8 @@ __device__ __forceinline__ void sk_mbar_arrive(uint32_t bar)
 {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void sk_mbar_wait(uint32_t bar, uint32_t parity)
+// `limit` polls, then trap: a phase that never completes is a bug -- fail loudly, do not hang
+__device__ __forceinline__ void sk_mbar_wait(uint32_t bar, uint32_t parity, uint32_t limit)
 {
     uint32_t spins = 0;
     for (;;) {
@@ -100,8 +104,23 @@ __device__ __forceinline__ void sk_mbar_wait(uint32_t bar, uint32_t parity)
             : "r"(bar), "r"(parity)
             : "memory");
         if (ok) return;
-        if (++spins > (1u << 24)) __trap();       // a copy that never lands is a bug: fail loudly, do not hang
+        if (++spins > limit) __trap();
     }
+}
+// non-blocking: has the phase of this parity completed?
+__device__ __forceinline__ bool sk_mbar_test(uint32_t bar, uint32_t parity)
+{
+    uint32_t ok;
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+        "selp.u32 %0, 1, 0, p;\n"
+        "}\n"
+        : "=r"(ok)
+        : "r"(bar), "r"(parity)
+        : "memory");
+    return ok != 0;
 }
 __device__ __forceinline__ void sk_bulk_load(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
 {
@@ -134,6 +153,7 @@ __device__ __forceinline__ bool sk_elect_one()
     return pred != 0;
 }
 __device__ __forceinline__ void sk_bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
+__device__ __forceinline__ void sk_bulk_wait_read_0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 
 // exchange slot of one frame: {adv31 bits | tag << 32, adv30 bits | tag << 32}
 __device__ __forceinline__ ulonglong2 sk_ld_slot(const ulonglong2 *p)
@@ -224,21 +244,24 @@ constexpr uint32_t SK_EDGE_B = BLK * 8u;             // edge pairs of a stage
 constexpr uint32_t SK_DPST_B = BLK * 128u;           // one dp staging tile
 constexpr uint32_t SK_PUB_B = (2 * BLK + BLK + 32) * 4u;   // adv31 [BLK], adv30 [BLK], scratch [BLK + 32]
 constexpr int SK_LOOK = 3;                           // operands are loaded this many iterations ahead
+constexpr int SK_NBUF = 3;                           // dp and publication staging buffers: block j reuses block j - 3's
 static_assert(BLK == 16 || BLK == 32, "a block is one or two backpointer words long");
 
 // shared-memory map (byte offsets from the 128-byte aligned base)
 template <int NSTG> struct SkSmem {
     static constexpr uint32_t TILE = 0;                                   // [(NSTG + 1) x BLK][36] f32 (+1: mirror of stage 0)
     static constexpr uint32_t EDGE = TILE + (NSTG + 1) * SK_STG_B;        // [(NSTG + 1) x BLK] float2
-    static constexpr uint32_t DPST = EDGE + (NSTG + 1) * SK_EDGE_B;       // 2 x [BLK][32] f32: kept-dp staging
-    static constexpr uint32_t PUB = DPST + 2 * SK_DPST_B;                 // 2 x publication staging
-    static constexpr uint32_t FULL = PUB + 2 * SK_PUB_B;                  // NSTG mbarriers
-    static constexpr uint32_t SLOT = FULL + NSTG * 8;                     // work-item ticket
+    static constexpr uint32_t DPST = EDGE + (NSTG + 1) * SK_EDGE_B;       // SK_NBUF x [BLK][32] f32: kept-dp staging
+    static constexpr uint32_t PUB = DPST + SK_NBUF * SK_DPST_B;           // SK_NBUF x publication staging
+    static constexpr uint32_t FULL = PUB + SK_NBUF * SK_PUB_B;            // NSTG mbarriers: the tile has landed
+    static constexpr uint32_t READY = FULL + NSTG * 8;                    // NSTG: ... and its ghost columns are in
+    static constexpr uint32_t DONE = READY + NSTG * 8;                    // NSTG: the compute warp is done with a block
+    static constexpr uint32_t SLOT = DONE + NSTG * 8;                     // work-item ticket, role swap
     static constexpr uint32_t BYTES = SLOT + 16;
 };
 
 template <int D, int NSTG, bool KEEP, bool DUMP>
-__global__ void __launch_bounds__(32)
+__global__ void __launch_bounds__(64)
 hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict__ dp_dump, int force_slow)
 {
     using SM = SkSmem<NSTG>;
@@ -254,14 +277,28 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         asm volatile("mov.u32 %0, %1;" : "=r"(sm0) : "r"(a));
     }
 
-    const int lane = threadIdx.x;
-    if (lane == 0) {
+    // Which of the two warps computes?  As in hfa_dp_band_kernel: the warps of a 2-warp CTA land on an
+    // aligned pair of warp slots (slot % 4 = scheduler partition), so "warp 0 computes" would put every
+    // compute warp of the SM on partitions 0 and 2; swapping the roles in every other pair spreads them.
+    if (threadIdx.x == 0) {
+        unsigned hw_slot;
+        asm volatile("mov.u32 %0, %%warpid;" : "=r"(hw_slot));
+        sk_sts_i32(sm0 + SM::SLOT + 4u, (int)((hw_slot >> 2) & 1u));
         sk_sts_i32(sm0 + SM::SLOT, (int)atomicInc(reinterpret_cast<unsigned int *>(ticket), gridDim.x - 1));   // self-resetting
 #pragma unroll
-        for (int s = 0; s < NSTG; ++s) sk_mbar_init(sm0 + SM::FULL + 8u * s, 1);
+        for (int s = 0; s < NSTG; ++s) {
+            sk_mbar_init(sm0 + SM::FULL + 8u * s, 1);      // the copy issuer (+ the TMA bytes)
+            sk_mbar_init(sm0 + SM::READY + 8u * s, 32);    // every producer lane, after the ghost columns
+            sk_mbar_init(sm0 + SM::DONE + 8u * s, 32);     // every compute lane, after the block
+        }
         hfa_fence_mbar_init();
     }
-    __syncwarp();
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    // (broadcast from lane 0 so that the compiler knows the role is warp-uniform: without it, the compute
+    // warp's shuffles are compiled for a possibly diverged warp)
+    const bool producer =
+        __shfl_sync(0xffffffffu, (threadIdx.x >> 5) ^ (unsigned)sk_lds_i32(sm0 + SM::SLOT + 4u), 0) != 0;
     const int item = item_begin + sk_lds_i32(sm0 + SM::SLOT);
     const HfaBandItem bi = ws.band_items[item];
     const int u = bi.utt, w = bi.band;
@@ -269,14 +306,156 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     const int T = m.T, S = m.S, Sp = m.Sp;
     const bool has_left = w > 0, has_right = w + 1 < hfa_skew_strips(Sp);
     const int c0 = HFA_SKEW_OWN * w;
+    const int NB = hfa_skew_blocks(D, T);
+
+    if (producer) {
+        // ---------------- producer: TMA ring, left exchange -> ghost columns, publication, dp store ----------------
+        // Block a is PREPARED (tile landed, the left strip's advance scores stored over the ghost columns:
+        // READY) and block b RETIRED (after DONE: its advance scores published, its dp rows stored, the
+        // stage it read last refilled).  Retiring comes first -- the right strip waits for it -- and
+        // neither step blocks the other: the loop polls both.  Preparing runs ahead as far as the left
+        // strip, the ring (tile a is fetched when block a - PF - 1 retires) and the staging buffers (block
+        // a writes the ones block a - SK_NBUF wrote: a <= b + SK_NBUF - 1) allow.
+        const float2 *g_edge = ws.edge2 + m.edge_off;
+        const unsigned char *tmap = static_cast<const unsigned char *>(ws.tmaps) + (size_t)m.tmap * 128;
+        float *g_dp = (KEEP && m.dp_off >= 0) ? ws.dp_store + m.dp_off + (int64_t)w * NB * (BLK * 32) : nullptr;
+        // tile i -> stage st (= i % NSTG, kept as a running counter); executed by ONE elected lane.  The edge
+        // pairs of an utterance are padded to a multiple of 16 frames: the last copy of a 32-frame block may be short.
+        const int edge_len = (T + 15) & ~15;
+        auto issue = [&](int i, int st) {
+            const int t0 = i * BLK;
+            const uint32_t bar = sm0 + SM::FULL + 8u * (uint32_t)st;
+            if (t0 >= T) {                                     // nothing to fetch: complete the phase
+                sk_mbar_arrive(bar);
+                return;
+            }
+            const uint32_t ebytes = (uint32_t)min(BLK, edge_len - t0) * 8u;
+            const uint32_t bytes = SK_STG_B + ebytes;
+            sk_mbar_expect_tx(bar, st == 0 ? 2u * bytes : bytes);
+            sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)st * SK_STG_B, tmap, c0 & ~3, t0, bar);
+            sk_bulk_load(sm0 + SM::EDGE + (uint32_t)st * SK_EDGE_B, g_edge + t0, ebytes, bar);
+            if (st == 0) {                                     // the mirror behind the last stage
+                sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)NSTG * SK_STG_B, tmap, c0 & ~3, t0, bar);
+                sk_bulk_load(sm0 + SM::EDGE + (uint32_t)NSTG * SK_EDGE_B, g_edge + t0, ebytes, bar);
+            }
+        };
+        static_assert(PF + 1 <= NSTG, "prologue fills distinct stages");
+        if (sk_elect_one())
+            for (int i = 0; i <= PF && i < NB; ++i) issue(i, i);   // tiles 0 .. PF (tile b + PF + 1 follows block b)
+
+        const ulonglong2 *left_x = reinterpret_cast<const ulonglong2 *>(ws.band_xchg) +
+                                   (has_left ? ws.band_items[item - 1].xoff : 0);
+        ulonglong2 *my_x = reinterpret_cast<ulonglong2 *>(ws.band_xchg) + bi.xoff;
+        auto slot_needed = [&](int jj) { const int t = BLK * jj + lane; return has_left && lane < BLK && t >= 1 && t < T; };
+        // exchange slots of the block being prepared, fetched one block early (the left strip is normally
+        // that far ahead)
+        ulonglong2 xv = make_ulonglong2(0ull, 0ull);
+        if (slot_needed(0)) xv = sk_ld_slot(left_x + lane);
+
+        int a = 0, st_a = 0, buf_b = 0;
+        uint32_t par_a = 0;
+        int b = 0, st_b = 0;
+        uint32_t par_b = 0;
+        int st_issue = (PF + 1) % NSTG;                        // stage of the next tile to fetch
+        uint32_t spins = 0;
+        while (b < NB) {
+            if (b < a && __all_sync(0xffffffffu, sk_mbar_test(sm0 + SM::DONE + 8u * (uint32_t)st_b, par_b))) {
+                if (has_right) {
+                    // the advance scores lanes 31 and 30 have parked: published as tagged 64-bit words, adv31 of
+                    // frame BLK b + i - 31 D into .x, adv30 of frame BLK b + i - 30 D into .y (frames 1 .. T-1 only)
+#pragma unroll
+                    for (int q = lane; q < 2 * BLK; q += 32) {
+                        const int half = q / BLK, i = q % BLK;
+                        const int t = BLK * b + i - (31 - half) * D;
+                        if (t >= 1 && t < T)
+                            sk_st_word(reinterpret_cast<unsigned long long *>(my_x + t) + half,
+                                       sk_pack(sk_lds_f32(sm0 + SM::PUB + (uint32_t)buf_b * SK_PUB_B + 4u * (uint32_t)q),
+                                               (uint32_t)t + 1u));
+                    }
+                }
+                if (sk_elect_one()) {
+                    if (KEEP && g_dp != nullptr) {             // the block's rows of dp leave as one bulk store
+                        sk_bulk_store(g_dp + (int64_t)b * (BLK * 32), sm0 + SM::DPST + (uint32_t)buf_b * SK_DPST_B,
+                                      SK_DPST_B);
+                        hfa_bulk_commit();
+                    }
+                    if (b + PF + 1 < NB) issue(b + PF + 1, st_issue);   // into the stage block b read last
+                }
+                if (++st_issue == NSTG) st_issue = 0;
+                if (++st_b == NSTG) {
+                    st_b = 0;
+                    par_b ^= 1u;
+                }
+                if (++buf_b == SK_NBUF) buf_b = 0;
+                ++b;
+                spins = 0;
+                continue;
+            }
+            if (a < NB && a <= b + SK_NBUF - 1 &&
+                __all_sync(0xffffffffu, sk_mbar_test(sm0 + SM::FULL + 8u * (uint32_t)st_a, par_a))) {
+                bool go = true;
+                if (has_left) {
+                    // The left strip's advance scores for frames BLK a .. BLK a + BLK - 1 go where the ghost lanes
+                    // look for their "emission": ghost lane 0 (the left strip's state 30) reads column c0 of row t
+                    // of the tile, ghost lane 1 (state 31) column c0 + 1 -- the emissions TMA put there are of no
+                    // use to anybody.
+                    const int t = BLK * a + lane;
+                    const bool need = slot_needed(a);
+                    ulonglong2 *src = const_cast<ulonglong2 *>(left_x) + t;
+                    const uint32_t tag = (uint32_t)t + 1u;
+                    const bool ok = !need || ((uint32_t)(xv.x >> 32) == tag && (uint32_t)(xv.y >> 32) == tag);
+                    go = __all_sync(0xffffffffu, ok);
+                    if (!go) {
+                        if (!ok) xv = sk_ld_slot(src);
+                    } else {
+                        const ulonglong2 v = xv;
+                        xv = slot_needed(a + 1) ? sk_ld_slot(src + BLK) : make_ulonglong2(0ull, 0ull);
+                        if (lane < BLK) {
+                            const float a30 = need ? __uint_as_float((uint32_t)v.y) : 0.0f;
+                            const float a31 = need ? __uint_as_float((uint32_t)v.x) : 0.0f;
+                            const uint32_t row_sa = sm0 + SM::TILE + (uint32_t)st_a * SK_STG_B + (uint32_t)lane * SK_ROW_B +
+                                                    4u * (uint32_t)(c0 & 3);
+                            sk_sts_f32(row_sa, a30);
+                            sk_sts_f32(row_sa + 4u, a31);
+                            if (st_a == 0) {                                       // and its mirror
+                                sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B, a30);
+                                sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B + 4u, a31);
+                            }
+                            if (need) sk_st_slot(src, 0ull, 0ull);                 // leave the table clean
+                        }
+                        hfa_fence_async_smem();   // generic writes into a stage the TMA engine will refill later
+                    }
+                }
+                if (go) {
+                    // block a overwrites the dp staging of block a - SK_NBUF: that bulk store must have been read
+                    // out (stores 0 .. b - 1 are in flight; a - SK_NBUF <= b - 2 unless a = b + SK_NBUF - 1)
+                    if (KEEP && a >= SK_NBUF && sk_elect_one()) {
+                        if (a == b + SK_NBUF - 1) sk_bulk_wait_read_0();
+                        else sk_bulk_wait_read_1();
+                    }
+                    sk_mbar_arrive(sm0 + SM::READY + 8u * (uint32_t)st_a);
+                    if (++st_a == NSTG) {
+                        st_a = 0;
+                        par_a ^= 1u;
+                    }
+                    ++a;
+                    spins = 0;
+                    continue;
+                }
+            }
+            // neither step can go: the compute warp is inside its block, or the left strip is behind
+            if (++spins > (1u << 26)) __trap();
+        }
+        if (KEEP && sk_elect_one()) hfa_bulk_wait_all();
+        return;
+    }
+
+    // ---------------- compute warp: the recurrence, nothing else ----------------
     const int s = c0 + lane;                                   // this lane's state
     const bool ghost = has_left && lane < 2;
     const bool real = !ghost && s < Sp;                        // owns a column of the padded matrices
-    const int NB = hfa_skew_blocks(D, T);
     const int n_rows = (T + 15) >> 4;
-    const float2 *g_edge = ws.edge2 + m.edge_off;
     uint32_t *g_bp = ws.bp + m.bp_off;
-    const unsigned char *tmap = static_cast<const unsigned char *>(ws.tmaps) + (size_t)m.tmap * 128;
     const double ratio = __ddiv_rn((double)T, (double)S);      // T / S (:186)
     const float NEG = HFA_NEG_INF, POS = __uint_as_float(0x7f800000u);
 
@@ -292,32 +471,9 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     const bool seeded = !ghost && (s == 0 || (s == 1 && lead_sp));
     const float cap1 = (s == 0) ? NEG : POS;                   // nothing to the left of state 0
 
-    // tile i -> stage st (= i % NSTG, kept as a running counter); executed by ONE elected lane.  The edge
-    // pairs of an utterance are padded to a multiple of 16 frames: the last copy of a 32-frame block may be short.
-    const int edge_len = (T + 15) & ~15;
-    auto issue = [&](int i, int st) {
-        const int t0 = i * BLK;
-        const uint32_t bar = sm0 + SM::FULL + 8u * (uint32_t)st;
-        if (t0 >= T) {                                         // nothing to fetch: complete the phase
-            sk_mbar_arrive(bar);
-            return;
-        }
-        const uint32_t ebytes = (uint32_t)min(BLK, edge_len - t0) * 8u;
-        const uint32_t bytes = SK_STG_B + ebytes;
-        sk_mbar_expect_tx(bar, st == 0 ? 2u * bytes : bytes);
-        sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)st * SK_STG_B, tmap, c0 & ~3, t0, bar);
-        sk_bulk_load(sm0 + SM::EDGE + (uint32_t)st * SK_EDGE_B, g_edge + t0, ebytes, bar);
-        if (st == 0) {                                         // the mirror behind the last stage
-            sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)NSTG * SK_STG_B, tmap, c0 & ~3, t0, bar);
-            sk_bulk_load(sm0 + SM::EDGE + (uint32_t)NSTG * SK_EDGE_B, g_edge + t0, ebytes, bar);
-        }
-    };
-    static_assert(PF + 1 <= NSTG, "prologue fills distinct stages");
-    if (sk_elect_one())
-        for (int i = 0; i <= PF && i < NB; ++i) issue(i, i);   // tiles 0 .. PF (tile j + PF + 1 follows block j)
-    int st_issue = (PF + 1) % NSTG;                            // stage of the next tile to fetch
     int st_wait = 0;                                           // stage and phase parity of the current block's tile
     uint32_t par_wait = 0;
+    int buf = 0;                                               // staging buffer of the current block (j % SK_NBUF)
 
     // loop-carried state
     float dp = NEG;
@@ -331,7 +487,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
 
     // per-lane ring position of the first row of the current block: (BLK j - lane D) mod R
     int u_row = ((-lane * D) % R + R) % R;
-    // (a ghost lane's "emission" is the left strip's advance score: written over its column of the tile, below)
+    // (a ghost lane's "emission" is the left strip's advance score: the producer writes it over its column)
     const uint32_t tile_sa = sm0 + SM::TILE + 4u * (uint32_t)(lane + (c0 & 3));
     const uint32_t edge_sa = sm0 + SM::EDGE;
     const uint32_t dpst_sa = sm0 + SM::DPST + 4u * (uint32_t)lane;
@@ -341,9 +497,6 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     const uint32_t m16 = o_res ? ((0xffffu << (16 - o_res)) & 0xffffu) : 0xffffu;
     const uint32_t hi_mask = m16 | (m16 << 16);
     const uint32_t mrot0 = 0x00010001u << ((16 - o_res) & 15);
-    const ulonglong2 *left_x = reinterpret_cast<const ulonglong2 *>(ws.band_xchg) +
-                               (has_left ? ws.band_items[item - 1].xoff : 0);
-    ulonglong2 *my_x = reinterpret_cast<ulonglong2 *>(ws.band_xchg) + bi.xoff;
     // publication staging: every iteration each lane parks its advance score at [its base + 4 k]; only the
     // rows of lanes 31 and 30 are read back (the other lanes write to a scratch area, one column each)
     const uint32_t pub_sa = sm0 + SM::PUB +
@@ -352,12 +505,6 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     // running pointer of this lane's backpointer word of row (16-frame half-block index) - q_rows
     uint32_t *bp_ptr = g_bp + (int64_t)(-q_rows) * Sp + s;
     int bp_row = -q_rows;
-    float *g_dp = (KEEP && m.dp_off >= 0) ? ws.dp_store + m.dp_off + (int64_t)w * NB * (BLK * 32) : nullptr;
-
-    // exchange slots of the NEXT block, fetched one block early (the left strip is normally that far ahead)
-    ulonglong2 xv_next = make_ulonglong2(0ull, 0ull);
-    auto slot_needed = [&](int jj) { const int t = BLK * jj + lane; return has_left && lane < BLK && t >= 1 && t < T; };
-    if (slot_needed(0)) xv_next = sk_ld_slot(left_x + lane);
 
     // one 16-frame backpointer word: `bits` holds the first part of row bp_row (from the previous half-block),
     // its last part is acc[hi_mask]; the rest of acc opens the next row
@@ -369,50 +516,18 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     };
 
     for (int j = 0; j < NB; ++j) {
-        sk_mbar_wait(sm0 + SM::FULL + 8u * (uint32_t)st_wait, par_wait);
+        // READY covers the producer's wait for the left strip as well as the copy: the exchange bound
+        sk_mbar_wait(sm0 + SM::READY + 8u * (uint32_t)st_wait, par_wait, 1u << 26);
         const int st_cur = st_wait;                            // stage that holds frames BLK j .. BLK j + BLK - 1
         if (++st_wait == NSTG) {
             st_wait = 0;
             par_wait ^= 1u;
         }
 
-        if (has_left) {
-            // The left strip's advance scores for frames BLK j .. BLK j + BLK - 1 go where the ghost lanes look for
-            // their "emission": ghost lane 0 (the left strip's state 30) reads column c0 of row t of the tile,
-            // ghost lane 1 (state 31) column c0 + 1 -- the emissions TMA put there are of no use to anybody.
-            const int t = BLK * j + lane;
-            const bool need = slot_needed(j);
-            ulonglong2 *src = const_cast<ulonglong2 *>(left_x) + t;
-            const uint32_t tag = (uint32_t)t + 1u;
-            ulonglong2 v = xv_next;
-            uint32_t spins = 0;
-            for (;;) {
-                const bool ok = !need || ((uint32_t)(v.x >> 32) == tag && (uint32_t)(v.y >> 32) == tag);
-                if (__all_sync(0xffffffffu, ok)) break;
-                if (++spins > (1u << 26)) __trap();
-                if (!ok) v = sk_ld_slot(src);
-            }
-            if (slot_needed(j + 1)) xv_next = sk_ld_slot(src + BLK);           // consumed one block later
-            if (lane < BLK) {
-                const float a30 = need ? __uint_as_float((uint32_t)v.y) : 0.0f;
-                const float a31 = need ? __uint_as_float((uint32_t)v.x) : 0.0f;
-                const uint32_t row_sa = sm0 + SM::TILE + (uint32_t)st_cur * SK_STG_B + (uint32_t)lane * SK_ROW_B +
-                                        4u * (uint32_t)(c0 & 3);
-                sk_sts_f32(row_sa, a30);
-                sk_sts_f32(row_sa + 4u, a31);
-                if (st_cur == 0) {                                             // and its mirror
-                    sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B, a30);
-                    sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B + 4u, a31);
-                }
-                if (need) sk_st_slot(src, 0ull, 0ull);                         // leave the table clean
-            }
-            hfa_fence_async_smem();       // generic writes into a stage the TMA engine will refill later
-            __syncwarp();
-        }
         const uint32_t e_sa = tile_sa + (uint32_t)u_row * SK_ROW_B;
         const uint32_t d_sa = edge_sa + (uint32_t)u_row * 8u;
-        const uint32_t k_sa = dpst_sa + (uint32_t)(j & 1) * SK_DPST_B;
-        const uint32_t p_sa = pub_sa + (uint32_t)(j & 1) * SK_PUB_B;
+        const uint32_t k_sa = dpst_sa + (uint32_t)buf * SK_DPST_B;
+        const uint32_t p_sa = pub_sa + (uint32_t)buf * SK_PUB_B;
         // all 32 lanes inside frames 1 .. T-1 for all BLK iterations?
         const bool steady = (BLK * j - 31 * D >= 1) && (BLK * j + BLK - 1 <= T - 1);
 
@@ -539,33 +654,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             for (int i = 0; i < 2 * D; ++i) q2[i] = r2[BLK + i];
         }
         if (KEEP) hfa_fence_async_smem();                      // this block's dp rows -> visible to the bulk store
-        __syncwarp();                                          // every lane is done with this block's stage reads,
-                                                               // staging writes and the stage refilled below
-        if (has_right) {
-            // the advance scores lanes 31 and 30 have parked: published as tagged 64-bit words, adv31 of frame
-            // BLK j + i - 31 D into .x, adv30 of frame BLK j + i - 30 D into .y (frames 1 .. T-1 only; the
-            // staging is double-buffered)
-#pragma unroll
-            for (int q = lane; q < 2 * BLK; q += 32) {
-                const int half = q / BLK, i = q % BLK;
-                const int t = BLK * j + i - (31 - half) * D;
-                if (steady || (t >= 1 && t < T))
-                    sk_st_word(reinterpret_cast<unsigned long long *>(my_x + t) + half,
-                               sk_pack(sk_lds_f32(sm0 + SM::PUB + (uint32_t)(j & 1) * SK_PUB_B + 4u * (uint32_t)q),
-                                       (uint32_t)t + 1u));
-            }
-        }
-        if (sk_elect_one()) {
-            if (KEEP && g_dp != nullptr) {
-                // the block's rows of dp leave as one bulk store; the staging tile written two blocks
-                // ago must have been read out before the next block overwrites it
-                sk_bulk_store(g_dp + (int64_t)j * (BLK * 32), sm0 + SM::DPST + (uint32_t)(j & 1) * SK_DPST_B, SK_DPST_B);
-                hfa_bulk_commit();
-                sk_bulk_wait_read_1();
-            }
-            if (j + PF + 1 < NB) issue(j + PF + 1, st_issue);  // into the stage last read during this block
-        }
-        if (++st_issue == NSTG) st_issue = 0;
+        sk_mbar_arrive(sm0 + SM::DONE + 8u * (uint32_t)st_cur);   // the stage, the staging rows: the producer's now
+        if (++buf == SK_NBUF) buf = 0;
         u_row += BLK;
         if (u_row >= R) u_row -= R;
     }
@@ -576,7 +666,6 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         if (s == S - 1) ws.dp_last[2 * u] = dp;
         if (s == S - 2) ws.dp_last[2 * u + 1] = dp;
     }
-    if (KEEP && sk_elect_one()) hfa_bulk_wait_all();
 }
 
 template <int D, int NSTG, bool KEEP, bool DUMP>
@@ -587,7 +676,7 @@ cudaError_t launch_skew(const HfaLaunchCtx &c, int item_begin, int n_items, int3
     cudaError_t e = cudaFuncSetAttribute(hfa_dp_skew_kernel<D, NSTG, KEEP, DUMP>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    hfa_dp_skew_kernel<D, NSTG, KEEP, DUMP><<<n_items, 32, smem, c.stream>>>(c.ws, item_begin, ticket, dp_dump,
+    hfa_dp_skew_kernel<D, NSTG, KEEP, DUMP><<<n_items, 64, smem, c.stream>>>(c.ws, item_begin, ticket, dp_dump,
                                                                             force_slow);
     return cudaGetLastError();
 }
@@ -605,7 +694,7 @@ cudaError_t launch_skew_d(const HfaLaunchCtx &c, int item_begin, int n_items, in
 
 }  // namespace
 
-// skewed kernel: items [item_begin, item_begin + n_items) of the plan's strip table, one warp each.
+// skewed kernel: items [item_begin, item_begin + n_items) of the plan's strip table, one 2-warp CTA each.
 // d = frames of skew per state (2 or 3, fixed when the plan was made: the dp store layout depends on it)
 cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int item_begin, int n_items, int32_t *ticket,
                                bool keep_dp, float *dp_dump)
