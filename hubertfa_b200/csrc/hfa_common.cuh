@@ -93,8 +93,10 @@ struct HfaWs {
     int32_t *emis_mode;          // [n_utt]
     const HfaBandItem *band_items;   // banded kernel work list (see hfa_dp_band_kernel)
     int32_t *band_ticket;        // [2] work-item tickets of the two band lists (self-resetting)
-    uint4 *band_xchg;            // {dp, tag, p.lo, tag}{p.hi, tag, 0, tag} of a band's last 32 states per tile;
-                                 // all-zero between calls (zeroed by hfa_plan_upload, then by its readers)
+    uint4 *band_xchg;            // 16-byte slots of tagged 64-bit words (hfa_ld_xchg): per band, tile and state of
+                                 // its last 32, {dp | tag << 32, p.lo | tag << 32}{p.hi | tag << 32, tag << 32};
+                                 // per strip and frame, {adv31 | tag << 32, adv30 | tag << 32}.
+                                 // All-zero between calls (zeroed by hfa_plan_upload, then by its readers)
 };
 
 #define HFA_NEG_INF __uint_as_float(0xff800000u)
@@ -114,7 +116,7 @@ __host__ __device__ __forceinline__ int64_t hfa_dp_store_index(int K, int T, int
 // advance scores of the left strip's last two states, lanes 2..31 own states 30 w + 2 .. 30 w + 31.
 #define HFA_SKEW_OWN 30
 #define HFA_SKEW_BOX 36          // columns of its TMA box: the box starts at (30 w) & ~3, a 16-byte boundary
-#define HFA_SKEW_BLK 32          // frames per block (TMA tile rows, exchange batch, dp staging tile): 16 or 32
+#define HFA_SKEW_BLK 32          // frames per block (TMA tile rows, exchange batch, dp staging tile)
 __host__ __device__ __forceinline__ int hfa_skew_strips(int Sp)
 {
     return Sp <= 32 ? 1 : 1 + (Sp - 32 + HFA_SKEW_OWN - 1) / HFA_SKEW_OWN;
@@ -135,56 +137,127 @@ __host__ __device__ __forceinline__ int64_t hfa_skew_dp_index(int D, int T, int 
 }
 
 // ---------------------------------------------------------------------------------------------
-// PTX helpers: mbarrier + 1-D bulk async copy (TMA engine, SASS: UBLKCP)
+// PTX primitives.  Shared memory is addressed through 32-bit shared::cta window addresses: a generic
+// pointer costs an S2UR + ULEA at every use on sm_100, so a kernel converts once (hfa_smem_u32) and
+// works on offsets from there.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t hfa_smem_u32(const void *p)
 {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
-__device__ __forceinline__ void hfa_mbar_init(uint64_t *bar, uint32_t count)
+__device__ __forceinline__ float hfa_lds_f32(uint32_t addr)
 {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(hfa_smem_u32(bar)), "r"(count)
-                 : "memory");
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ float2 hfa_lds_f2(uint32_t addr)
+{
+    float2 v;
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ int hfa_lds_s32(uint32_t addr)
+{
+    int v;
+    asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
+    return v;
+}
+__device__ __forceinline__ void hfa_sts_f32(uint32_t addr, float v)
+{
+    asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
+}
+__device__ __forceinline__ void hfa_sts_s32(uint32_t addr, int v)
+{
+    asm volatile("st.shared.s32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+
+// mbarriers
+__device__ __forceinline__ void hfa_mbar_init(uint32_t bar, uint32_t count)
+{
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
 __device__ __forceinline__ void hfa_fence_mbar_init()
 {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
-__device__ __forceinline__ void hfa_mbar_expect_tx(uint64_t *bar, uint32_t bytes)
+__device__ __forceinline__ void hfa_mbar_expect_tx(uint32_t bar, uint32_t bytes)
 {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(hfa_smem_u32(bar)),
-                 "r"(bytes)
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void hfa_mbar_arrive(uint32_t bar)
+{
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+// non-blocking: has the phase of this parity completed?
+__device__ __forceinline__ bool hfa_mbar_test_wait(uint32_t bar, uint32_t parity)
+{
+    uint32_t ok;
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+        "selp.u32 %0, 1, 0, p;\n"
+        "}\n"
+        : "=r"(ok)
+        : "r"(bar), "r"(parity)
+        : "memory");
+    return ok != 0;
+}
+// Poll bounds of the spin waits (DESIGN §8 item 4).  A phase that never completes is a bug: fail loudly
+// rather than hang the GPU.  Every bound counts the polls of ONE wait and none grows with T.
+constexpr uint32_t HFA_POLLS_COPY = 1u << 24;      // one TMA copy of one tile
+constexpr uint32_t HFA_POLLS_EXCHANGE = 1u << 26;  // one exchange with the left neighbour (an L2 round trip per poll)
+// try_wait suspends the thread for a hardware time slice per poll; `limit` polls, then trap
+__device__ __forceinline__ void hfa_mbar_wait(uint32_t bar, uint32_t parity, uint32_t limit)
+{
+    uint32_t spins = 0;
+    for (;;) {
+        uint32_t ok;
+        asm volatile(
+            "{\n"
+            ".reg .pred p;\n"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
+            "selp.u32 %0, 1, 0, p;\n"
+            "}\n"
+            : "=r"(ok)
+            : "r"(bar), "r"(parity)
+            : "memory");
+        if (ok) return;
+        if (++spins > limit) __trap();
+    }
+}
+
+// bulk async copies (TMA engine): 1-D global -> shared (SASS UBLKCP), completing on an mbarrier
+__device__ __forceinline__ void hfa_bulk_load(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
+{
+    asm volatile("cp.async.bulk.shared::cta.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                 "l"(src), "r"(bytes), "r"(bar)
                  : "memory");
 }
-__device__ __forceinline__ void hfa_bulk_load(void *dst_smem, const void *src_gmem, uint32_t bytes,
-                                              uint64_t *bar)
+// 2-D tensor tile global -> shared (SASS UTMALDG): box position {x = column, y = row}
+__device__ __forceinline__ void hfa_tensor_load_2d(uint32_t dst, const void *tmap, int x, int y, uint32_t bar)
 {
     asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-            "r"(hfa_smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(hfa_smem_u32(bar))
+        "cp.async.bulk.tensor.2d.shared::cta.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
+        "l"(tmap), "r"(x), "r"(y), "r"(bar)
         : "memory");
 }
-// shared -> global bulk copy (TMA store), tracked by the issuing thread's bulk async-group
-__device__ __forceinline__ void hfa_bulk_store(void *dst_gmem, const void *src_smem, uint32_t bytes)
+// shared -> global (TMA store), tracked by the issuing thread's bulk async-group
+__device__ __forceinline__ void hfa_bulk_store(void *dst, uint32_t src, uint32_t bytes)
 {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem),
-                 "r"(hfa_smem_u32(src_smem)), "r"(bytes)
-                 : "memory");
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void hfa_bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void hfa_bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void hfa_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void hfa_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// 2-D tensor tile copy global -> shared (TMA, SASS UTMALDG): box position {x = column, y = row}
-__device__ __forceinline__ void hfa_tensor_load_2d(void *dst_smem, const void *tmap, int x, int y, uint64_t *bar)
+// at most N committed stores may still be reading their shared-memory source
+template <int N> __device__ __forceinline__ void hfa_bulk_wait_read()
 {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(hfa_smem_u32(dst_smem)), "l"(tmap), "r"(x), "r"(y), "r"(hfa_smem_u32(bar))
-        : "memory");
+    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
 }
+__device__ __forceinline__ void hfa_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// generic-proxy shared-memory writes -> visible to the async proxy (a bulk store, a later TMA refill)
+__device__ __forceinline__ void hfa_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // one lane of a CONVERGED warp (ptxas then emits TMA / bulk instructions once, from uniform registers, instead of
 // an ELECT / R2UR / BRA.U.ANY loop of ~20 instructions per copy)
 __device__ __forceinline__ bool hfa_elect_one()
@@ -199,47 +272,6 @@ __device__ __forceinline__ bool hfa_elect_one()
         : "=r"(pred));
     return pred != 0;
 }
-__device__ __forceinline__ bool hfa_mbar_try_wait(uint64_t *bar, uint32_t parity)
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(ok)
-        : "r"(hfa_smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ bool hfa_mbar_test_wait(uint64_t *bar, uint32_t parity)   // non-blocking
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(ok)
-        : "r"(hfa_smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void hfa_mbar_arrive(uint64_t *bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(hfa_smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void hfa_mbar_wait(uint64_t *bar, uint32_t parity)
-{
-    // try_wait suspends the thread for a hardware time slice; a copy that never lands (a bug) must
-    // not hang the GPU, so give up loudly after ~seconds of polling.
-    uint32_t spins = 0;
-    while (!hfa_mbar_try_wait(bar, parity)) {
-        if (++spins > (1u << 24)) __trap();
-    }
-}
 
 // Scattered 4-byte gathers (one value out of a row or a column per frame): by default the L2 fetches the whole
 // 128-byte line from HBM; the 64-byte fetch-granularity hint (SASS: LDG.E.LTC64B) is the smallest PTX offers.
@@ -250,26 +282,34 @@ __device__ __forceinline__ float hfa_ldg_f32_64B(const float *p)
     return v;
 }
 
+// Exchange words between the CTAs of one utterance (band and strip kernels, HfaWs::band_xchg): every 64-bit
+// word is {payload bits | tag << 32} and is read and written as ONE access, so it is single-copy atomic and
+// valid iff its tag matches -- no flag, no fence.  Readers zero what they consumed: the table is all-zero
+// between calls.
+__device__ __forceinline__ ulonglong2 hfa_ld_xchg(const ulonglong2 *p)
+{
+    ulonglong2 v;
+    asm volatile("ld.relaxed.gpu.global.v2.u64 {%0, %1}, [%2];" : "=l"(v.x), "=l"(v.y) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void hfa_st_xchg(ulonglong2 *p, unsigned long long a, unsigned long long b)
+{
+    asm volatile("st.relaxed.gpu.global.v2.u64 [%0], {%1, %2};" ::"l"(p), "l"(a), "l"(b) : "memory");
+}
+__device__ __forceinline__ void hfa_st_xchg_word(unsigned long long *p, unsigned long long a)
+{
+    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(a) : "memory");
+}
+__device__ __forceinline__ unsigned long long hfa_tagged(uint32_t bits, uint32_t tag)
+{
+    return (unsigned long long)bits | ((unsigned long long)tag << 32);
+}
+
 // the one mixed-precision operation of the recurrence (alignment_decoder.py:182-187):
 // f32( f64(a) + f64(curr) * ratio ), multiply and add rounded separately (no FMA contraction).
 __device__ __forceinline__ float hfa_advance(float a, float curr, double ratio)
 {
     return __double2float_rn(__dadd_rn((double)a, __dmul_rn((double)curr, ratio)));
-}
-
-// exp(x) for x <= 0 in the softmax normaliser (alignment_decoder.py:62-65).  Default: expf (1 ulp).
-// -DHFA_FAST_EXP: ex2.approx of x * log2(e), two instructions instead of eight, still inside the 4e-6 the
-// emission tests allow -- MEASURED on B200 config 4: no gain (emission stage 0.470 -> 0.481 ms: the kernel
-// waits on HBM, not on these instructions), so the exact one stays.
-__device__ __forceinline__ float hfa_exp_neg(float x)
-{
-#ifndef HFA_FAST_EXP
-    return expf(x);
-#else
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(__fmul_rn(x, 1.4426950408889634f)));
-    return y;
-#endif
 }
 
 template <typename T> __device__ __forceinline__ float hfa_to_float(T v);

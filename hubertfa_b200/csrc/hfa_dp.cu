@@ -154,32 +154,6 @@ template <int K> __device__ __forceinline__ void hfa_lds_row(uint32_t addr, floa
             asm volatile("ld.shared.f32 %0, [%1];" : "=f"(e[k]) : "r"(addr + 4u * k));
     }
 }
-__device__ __forceinline__ float2 hfa_lds_f2(uint32_t addr)
-{
-    float2 v;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
-    return v;
-}
-
-// exchange slot of one state: two 16-byte words {dp bits, tag, p.lo, tag} {p.hi, tag, 0, tag},
-// tag = tile + 1.  Every 8-byte half carries its own tag (8-byte accesses are single-copy atomic),
-// so the reader needs no flag and no fence: a half is valid iff its tag matches.  The reader zeroes
-// a slot after use, so the table is all-zero between calls (zeroed once by hfa_plan_upload).
-__device__ __forceinline__ uint4 hfa_ld_slot(const uint4 *p)
-{
-    uint4 v;
-    asm volatile("ld.relaxed.gpu.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                 : "l"(p)
-                 : "memory");
-    return v;
-}
-__device__ __forceinline__ void hfa_st_slot(uint4 *p, uint4 v)
-{
-    asm volatile("st.relaxed.gpu.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y),
-                 "r"(v.z), "r"(v.w)
-                 : "memory");
-}
 
 // One frame of K states with curr carried as p = f64(curr) * ratio (see above).
 //   e / pe : this frame's emissions and f64(e) * ratio;  ed = {edge_log, not_edge_log}
@@ -241,11 +215,10 @@ __device__ __forceinline__ void hfa_frame_p(const float (&e)[K], const double (&
 // warp per utterance
 // ---------------------------------------------------------------------------------------------
 constexpr int HFA_WARP_TILE = 8;      // frames per TMA stage (two stages = one backpointer word)
-#ifndef HFA_WARP_NSTAGES
-#define HFA_WARP_NSTAGES 2      // measured on config 4 (B200): 13 -> 20 resident warps per SM, DP stage 0.370 -> 0.362 ms (pairs),
-                                // 0.480 -> 0.457 ms (plain); the next tile still has a whole tile time (~1 us) to land
-#endif
-constexpr int HFA_WARP_STAGES = HFA_WARP_NSTAGES;    // the copy of tile i+3 is issued when tile i has been consumed
+// 2 stages, measured on config 4 (B200) against 3: 13 -> 20 resident warps per SM, DP stage 0.370 -> 0.362 ms
+// (pairs), 0.480 -> 0.457 ms (plain); the next tile still has a whole tile time (~1 us) to land.  The copy of
+// tile i + 2 is issued when tile i has been consumed.
+constexpr int HFA_WARP_STAGES = 2;
 
 template <int K> constexpr size_t hfa_warp_smem_bytes()
 {
@@ -285,14 +258,17 @@ __device__ __forceinline__ void hfa_dp_warp_body(const HfaWs &ws, const int u,
         const int t0 = i * TT;
         const int rows = min(TT, T - t0);
         const uint32_t bytes = (uint32_t)rows * (uint32_t)Sp * 4u;
-        hfa_mbar_expect_tx(&bar[st], bytes + TT * (uint32_t)sizeof(float2));
-        hfa_bulk_load(tile0 + st * TILE_FLOATS, g_emis + (int64_t)t0 * Sp, bytes, &bar[st]);
-        hfa_bulk_load(edge0 + st * TT, g_edge + t0, TT * (uint32_t)sizeof(float2), &bar[st]);
+        const uint32_t tx = bytes + TT * (uint32_t)sizeof(float2);
+        hfa_mbar_expect_tx(hfa_smem_u32(&bar[st]), tx);
+        const float *src = g_emis + (int64_t)t0 * Sp;
+        hfa_bulk_load(hfa_smem_u32(tile0 + st * TILE_FLOATS), src, bytes, hfa_smem_u32(&bar[st]));
+        const float2 *esrc = g_edge + t0;
+        hfa_bulk_load(hfa_smem_u32(edge0 + st * TT), esrc, TT * (uint32_t)sizeof(float2), hfa_smem_u32(&bar[st]));
     };
 
     if (lane == 0) {
 #pragma unroll
-        for (int s = 0; s < NST; ++s) hfa_mbar_init(&bar[s], 1);
+        for (int s = 0; s < NST; ++s) hfa_mbar_init(hfa_smem_u32(&bar[s]), 1);
         hfa_fence_mbar_init();
         for (int i = 0; i < NST && i < n_tiles; ++i) issue(i);
     }
@@ -317,7 +293,7 @@ __device__ __forceinline__ void hfa_dp_warp_body(const HfaWs &ws, const int u,
     int st = 0;
     uint32_t phase = 0;
     for (int i = 0; i < n_tiles; ++i) {
-        hfa_mbar_wait(&bar[st], phase);
+        hfa_mbar_wait(hfa_smem_u32(&bar[st]), phase, HFA_POLLS_COPY);
         const uint32_t tl = tile_sa + (uint32_t)st * (TILE_FLOATS * 4u);
         const uint32_t et = edge_sa + (uint32_t)st * (TT * 8u);
         const int rows = min(TT, T - i * TT);
@@ -428,16 +404,15 @@ __device__ __forceinline__ void hfa_dp_warp_body(const HfaWs &ws, const int u,
 // through the guarded body.
 // Eligibility (hfa_plan_create): no two adjacent SPs, pairs <= 32 * HFA_PAIR_MAX_K, cheaper than the
 // K-states-per-lane body.
-#ifndef HFA_PAIR_UNROLL
-#define HFA_PAIR_UNROLL 8        // measured on config 4 (B200, every utterance in pairs): DP stage 0.382 / 0.390 / 0.370 ms
-#endif                           // with 2 / 4 / 8 frames per chunk
 
 template <int KP, bool DUMP>
 __device__ __forceinline__ void hfa_dp_pair_body(const HfaWs &ws, const int u, float *__restrict__ dp_dump,
                                                  unsigned char *smem_raw)
 {
     constexpr int TT = HFA_WARP_TILE, NST = HFA_WARP_STAGES;
-    constexpr int UNR = HFA_PAIR_UNROLL;                      // frames per unrolled chunk (2, 4 or 8)
+    // frames per unrolled chunk: measured on config 4 (B200, every utterance in pairs), DP stage 0.382 / 0.390 /
+    // 0.370 ms with 2 / 4 / 8
+    constexpr int UNR = 8;
     const int lane = threadIdx.x & 31;
     const HfaUtt m = ws.utt[u];
     const int T = m.T, S = m.S, Sp = m.Sp;
@@ -469,14 +444,17 @@ __device__ __forceinline__ void hfa_dp_pair_body(const HfaWs &ws, const int u, f
         const int t0 = i * TT;
         const int rows = min(TT, T - t0);
         const uint32_t bytes = (uint32_t)rows * row_bytes;
-        hfa_mbar_expect_tx(&bar[st], bytes + TT * (uint32_t)sizeof(float2));
-        hfa_bulk_load(tile0 + st * TT * Ep, g_emis + (int64_t)t0 * Ep, bytes, &bar[st]);
-        hfa_bulk_load(edge0 + st * TT, g_edge + t0, TT * (uint32_t)sizeof(float2), &bar[st]);
+        const uint32_t tx = bytes + TT * (uint32_t)sizeof(float2);
+        hfa_mbar_expect_tx(hfa_smem_u32(&bar[st]), tx);
+        const float *src = g_emis + (int64_t)t0 * Ep;
+        hfa_bulk_load(hfa_smem_u32(tile0 + st * TT * Ep), src, bytes, hfa_smem_u32(&bar[st]));
+        const float2 *esrc = g_edge + t0;
+        hfa_bulk_load(hfa_smem_u32(edge0 + st * TT), esrc, TT * (uint32_t)sizeof(float2), hfa_smem_u32(&bar[st]));
     };
 
     if (lane == 0) {
 #pragma unroll
-        for (int s = 0; s < NST; ++s) hfa_mbar_init(&bar[s], 1);
+        for (int s = 0; s < NST; ++s) hfa_mbar_init(hfa_smem_u32(&bar[s]), 1);
         hfa_fence_mbar_init();
     }
     for (int q = lane; q < 32 * KP; q += 32) {
@@ -522,8 +500,8 @@ __device__ __forceinline__ void hfa_dp_pair_body(const HfaWs &ws, const int u, f
     auto load = [&](uint32_t off, uint32_t eoff, float (&eA)[KP], float (&eB)[KP], float2 &ed) {
 #pragma unroll
         for (int k = 0; k < KP; ++k) {
-            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(eA[k]) : "r"(aA[k] + off));
-            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(eB[k]) : "r"(aB[k] + off));
+            eA[k] = hfa_lds_f32(aA[k] + off);
+            eB[k] = hfa_lds_f32(aB[k] + off);
         }
         ed = hfa_lds_f2(edge_sa + eoff);
     };
@@ -609,7 +587,7 @@ __device__ __forceinline__ void hfa_dp_pair_body(const HfaWs &ws, const int u, f
     int st = 0;
     uint32_t phase = 0;
     for (int i = 0; i < n_tiles; ++i) {
-        hfa_mbar_wait(&bar[st], phase);
+        hfa_mbar_wait(hfa_smem_u32(&bar[st]), phase, HFA_POLLS_COPY);
         const uint32_t tl = (uint32_t)st * tile_bytes;        // row 0 of this stage (uniform)
         const uint32_t et = (uint32_t)st * (TT * 8u);
         const int rows = min(TT, T - i * TT);
@@ -750,14 +728,16 @@ hfa_dp_cta_kernel(HfaWs ws, const int32_t *__restrict__ order, int tile_t, int s
         const int t0 = i * tile_t;
         const int rows = min(tile_t, T - t0);
         const uint32_t bytes = (uint32_t)rows * (uint32_t)Sp * 4u;
-        hfa_mbar_expect_tx(&bar[st], bytes + edge_bytes);
-        hfa_bulk_load(tile0 + st * stage_floats, g_emis + (int64_t)t0 * Sp, bytes, &bar[st]);
-        hfa_bulk_load(edge0 + st * HFA_TILE_T, g_edge + (t0 & ~(HFA_TILE_T - 1)), edge_bytes,
-                      &bar[st]);
+        const uint32_t tx = bytes + edge_bytes;
+        hfa_mbar_expect_tx(hfa_smem_u32(&bar[st]), tx);
+        const float *src = g_emis + (int64_t)t0 * Sp;
+        hfa_bulk_load(hfa_smem_u32(tile0 + st * stage_floats), src, bytes, hfa_smem_u32(&bar[st]));
+        const float2 *esrc = g_edge + (t0 & ~(HFA_TILE_T - 1));
+        hfa_bulk_load(hfa_smem_u32(edge0 + st * HFA_TILE_T), esrc, edge_bytes, hfa_smem_u32(&bar[st]));
     };
 
     if (tid == 0) {
-        for (int s = 0; s < HFA_CTA_STAGES; ++s) hfa_mbar_init(&bar[s], 1);
+        for (int s = 0; s < HFA_CTA_STAGES; ++s) hfa_mbar_init(hfa_smem_u32(&bar[s]), 1);
         hfa_fence_mbar_init();
         for (int i = 0; i < HFA_CTA_STAGES && i < n_tiles; ++i) issue(i);
     }
@@ -778,7 +758,8 @@ hfa_dp_cta_kernel(HfaWs ws, const int32_t *__restrict__ order, int tile_t, int s
 
     for (int i = 0; i < n_tiles; ++i) {
         const int st = i % HFA_CTA_STAGES;
-        hfa_mbar_wait(&bar[st], (uint32_t)((i / HFA_CTA_STAGES) & 1));
+        const uint32_t parity = (i / HFA_CTA_STAGES) & 1;
+        hfa_mbar_wait(hfa_smem_u32(&bar[st]), parity, HFA_POLLS_COPY);
         // threads past the last padded state still run the loop (they take part in the barriers)
         // but read row 0 of the stage instead of running off its end
         const float *tl = tile0 + st * stage_floats + (first < Sp ? first : 0);
@@ -875,6 +856,11 @@ hfa_dp_cta_kernel(HfaWs ws, const int32_t *__restrict__ order, int tile_t, int s
 // Warp 0 is the CONSUMER: it only waits on that barrier, runs the recurrence, stores backpointer
 // words and publishes its own last 32 states.  Work items are claimed through an atomic ticket, so
 // a band's left neighbour has always started before the band itself; band 0 never waits.
+// Exchange slot of one state after tile i: two 16-byte halves of tagged 64-bit words (hfa_ld_xchg),
+// {dp | tag << 32, p.lo | tag << 32} {p.hi | tag << 32, tag << 32}, tag = i + 1.  Every word is
+// read and written as ONE access (single-copy atomic), so a word is valid iff its tag matches: no
+// flag, no fence.  The reader zeroes the slot after use, so the table is all-zero between calls
+// (zeroed once by hfa_plan_upload).
 //
 // The serial chain per frame is  FADD, FADD, F2F, DADD, F2F, SHFL, 3 x FMNMX  (~85 cycles):
 //   * curr[] is carried as the f64 product p = f64(curr) * ratio.  ratio > 0 and rounding is
@@ -929,8 +915,8 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         *slot = (int)atomicInc(reinterpret_cast<unsigned int *>(ticket), gridDim.x - 1);   // self-resetting
 #pragma unroll
         for (int s = 0; s < NST; ++s) {
-            hfa_mbar_init(&full[s], 2);          // the copy issuer + the halo relay
-            hfa_mbar_init(&empty[s], 1);         // the compute warp
+            hfa_mbar_init(hfa_smem_u32(&full[s]), 2);    // the copy issuer + the halo relay
+            hfa_mbar_init(hfa_smem_u32(&empty[s]), 1);   // the compute warp
         }
         hfa_fence_mbar_init();
     }
@@ -976,8 +962,9 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             const uint32_t shift = (uint32_t)(reinterpret_cast<uintptr_t>(src) & 15u);
             const uint32_t bytes = (shift + (uint32_t)(((int64_t)(rows - 1) * row_st + V) * 4) + 15u) & ~15u;
             shift_sm[ls] = (int32_t)shift;
-            hfa_mbar_expect_tx(&lbar[ls], bytes);
-            hfa_bulk_load(lstage0 + (size_t)ls * lstage_bytes, src - shift, bytes, &lbar[ls]);
+            hfa_mbar_expect_tx(hfa_smem_u32(&lbar[ls]), bytes);
+            hfa_bulk_load(hfa_smem_u32(lstage0 + (size_t)ls * lstage_bytes), src - shift, bytes,
+                          hfa_smem_u32(&lbar[ls]));
         };
         if constexpr (FUSED) {
             const HfaInput in = ws.inputs[u];
@@ -986,8 +973,8 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             const int32_t *ids = ws.ids + m.seg_off;
             if (lane < 8) mask_sm[lane] = (lane == 0) ? 1u : 0u;             // id 0 always kept (:39)
             if (lane == 0) {
-                hfa_mbar_init(&lbar[0], 1);
-                hfa_mbar_init(&lbar[1], 1);
+                hfa_mbar_init(hfa_smem_u32(&lbar[0]), 1);
+                hfa_mbar_init(hfa_smem_u32(&lbar[1]), 1);
                 hfa_fence_mbar_init();
             }
             __syncwarp();
@@ -1018,7 +1005,8 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         }
         const unsigned char *tmap = (ws.tmaps != nullptr && m.tmap >= 0)
                                         ? static_cast<const unsigned char *>(ws.tmaps) + (size_t)m.tmap * 128 : nullptr;
-        uint4 *left_x = ws.band_xchg + (has_left ? ws.band_items[item - 1].xoff : 0) + 2 * lane;
+        ulonglong2 *left_x =
+            reinterpret_cast<ulonglong2 *>(ws.band_xchg) + (has_left ? ws.band_items[item - 1].xoff : 0) + 2 * lane;
         // dp store: the compute warp leaves dp[t][.] of a tile in the stage it has just consumed (in
         // place of the emissions); before the stage is refilled the tile goes out as one bulk store.
         // every band keeps its WHOLE window ([T][W] block of its own, the halo columns included --
@@ -1027,27 +1015,29 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         for (int i = 0; i < n_tiles + NST; ++i) {
             const int st = i % NST;
             if (i >= NST) {
-                hfa_mbar_wait(&empty[st], (uint32_t)(((i / NST) - 1) & 1));
+                hfa_mbar_wait(hfa_smem_u32(&empty[st]), (uint32_t)(((i / NST) - 1) & 1), HFA_POLLS_COPY);
                 const int j = i - NST;                         // the tile that sat in this stage
                 if (g_dp != nullptr && lane == 0) {
-                    hfa_bulk_store(g_dp + (int64_t)j * TT * W, tile0 + st * TILE_FLOATS,
+                    hfa_bulk_store(g_dp + (int64_t)j * TT * W, hfa_smem_u32(tile0 + st * TILE_FLOATS),
                                    (uint32_t)min(TT, T - j * TT) * (uint32_t)W * 4u);
                     hfa_bulk_commit();
-                    hfa_bulk_wait_read();                      // the stage may be overwritten
+                    hfa_bulk_wait_read<0>();                   // the stage may be overwritten
                 }
                 __syncwarp();
             }
             if (i >= n_tiles) continue;
             const int t0 = i * TT;
             const int rows = min(TT, T - t0);
+            const uint32_t full_sa = hfa_smem_u32(&full[st]), edge_sa = hfa_smem_u32(edge0 + st * TT);
+            constexpr uint32_t edge_bytes = TT * (uint32_t)sizeof(float2);
             if constexpr (FUSED) {
                 if (lane == 0) {
-                    hfa_mbar_expect_tx(&full[st], TT * (uint32_t)sizeof(float2));
-                    hfa_bulk_load(edge0 + st * TT, g_edge + t0, TT * (uint32_t)sizeof(float2), &full[st]);
+                    hfa_mbar_expect_tx(full_sa, edge_bytes);
+                    hfa_bulk_load(edge_sa, g_edge + t0, edge_bytes, full_sa);
                     if (i + 1 < n_tiles) issue_logits(i + 1);     // its stage was read during tile i-1
                 }
                 const int ls = i & 1;
-                hfa_mbar_wait(&lbar[ls], (uint32_t)((i >> 1) & 1));
+                hfa_mbar_wait(hfa_smem_u32(&lbar[ls]), (uint32_t)((i >> 1) & 1), HFA_POLLS_COPY);
                 const float *xs = reinterpret_cast<const float *>(lstage0 + (size_t)ls * lstage_bytes + shift_sm[ls]);
                 // normaliser: lane -> (row = 8 * pass + lane / 4, part = lane % 4), kept ids only.
                 // The lane's kept ids sit in registers (kreg, <= 16 of them: up to 64 kept ids) so
@@ -1072,13 +1062,13 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
 #pragma unroll
                         for (int j = 0; j < 16; ++j)     // entries past the end are -inf: exp = +0, sum unchanged
-                            sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(xv[j], mx)));
+                            sum = __fadd_rn(sum, expf(__fsub_rn(xv[j], mx)));
                     } else {
                         for (int k = part; k < n_kept; k += 4) mx = fmaxf(mx, row[kept_sm[k]]);
                         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
                         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
                         for (int k = part; k < n_kept; k += 4)
-                            sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(row[kept_sm[k]], mx)));
+                            sum = __fadd_rn(sum, expf(__fsub_rn(row[kept_sm[k]], mx)));
                     }
                     sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
                     sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
@@ -1122,38 +1112,39 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                 // ONE tensor-tile copy per stage: box = 16 frames x W columns at {c0, t0} of emis[t][s]
                 // (rows past T and columns past Sp are zero-filled and never used)
                 if (lane == 0) {
-                    hfa_mbar_expect_tx(&full[st], (uint32_t)(TILE_FLOATS * 4) + TT * (uint32_t)sizeof(float2));
-                    hfa_bulk_load(edge0 + st * TT, g_edge + t0, TT * (uint32_t)sizeof(float2), &full[st]);
-                    hfa_tensor_load_2d(tile0 + st * TILE_FLOATS, tmap, c0, t0, &full[st]);
+                    hfa_mbar_expect_tx(full_sa, (uint32_t)(TILE_FLOATS * 4) + edge_bytes);
+                    hfa_bulk_load(edge_sa, g_edge + t0, edge_bytes, full_sa);
+                    hfa_tensor_load_2d(hfa_smem_u32(tile0 + st * TILE_FLOATS), tmap, c0, t0, full_sa);
                 }
             } else {
                 if (lane == 0) {
-                    hfa_mbar_expect_tx(&full[st], (uint32_t)rows * row_b + TT * (uint32_t)sizeof(float2));
-                    hfa_bulk_load(edge0 + st * TT, g_edge + t0, TT * (uint32_t)sizeof(float2), &full[st]);
+                    hfa_mbar_expect_tx(full_sa, (uint32_t)rows * row_b + edge_bytes);
+                    hfa_bulk_load(edge_sa, g_edge + t0, edge_bytes, full_sa);
                 }
                 __syncwarp();
                 if (lane < rows)
-                    hfa_bulk_load(tile0 + st * TILE_FLOATS + lane * W, g_emis + (int64_t)(t0 + lane) * Sp, row_b,
-                                  &full[st]);
+                    hfa_bulk_load(hfa_smem_u32(tile0 + st * TILE_FLOATS + lane * W), g_emis + (int64_t)(t0 + lane) * Sp, row_b,
+                                  full_sa);
             }
             if (has_left && i > 0) {
                 // the window's first 32 states at the start of tile i = the left band's last 32
                 // after its tile i-1: lane j relays state j
-                uint4 *src = left_x + (int64_t)(i - 1) * 64;
+                ulonglong2 *src = left_x + (int64_t)(i - 1) * 64;
                 const uint32_t tag = (uint32_t)i;
-                uint4 a = hfa_ld_slot(src), b = hfa_ld_slot(src + 1);
+                ulonglong2 a = hfa_ld_xchg(src), b = hfa_ld_xchg(src + 1);
                 uint32_t spins = 0;
-                while (a.y != tag || a.w != tag || b.y != tag || b.w != tag) {
-                    if (++spins > (1u << 26)) __trap();
-                    a = hfa_ld_slot(src);
-                    b = hfa_ld_slot(src + 1);
+                while ((uint32_t)(a.x >> 32) != tag || (uint32_t)(a.y >> 32) != tag || (uint32_t)(b.x >> 32) != tag ||
+                       (uint32_t)(b.y >> 32) != tag) {
+                    if (++spins > HFA_POLLS_EXCHANGE) __trap();
+                    a = hfa_ld_xchg(src);
+                    b = hfa_ld_xchg(src + 1);
                 }
-                halo0[st * 32 + lane] = make_uint4(a.x, 0u, a.z, b.x);
-                hfa_st_slot(src, make_uint4(0u, 0u, 0u, 0u));   // leave the table clean for the next call
-                hfa_st_slot(src + 1, make_uint4(0u, 0u, 0u, 0u));
+                halo0[st * 32 + lane] = make_uint4((uint32_t)a.x, 0u, (uint32_t)a.y, (uint32_t)b.x);
+                hfa_st_xchg(src, 0ull, 0ull);   // leave the table clean for the next call
+                hfa_st_xchg(src + 1, 0ull, 0ull);
             }
             __syncwarp();
-            if (lane == 0) hfa_mbar_arrive(&full[st]);
+            if (lane == 0) hfa_mbar_arrive(full_sa);
         }
         hfa_bulk_wait_all();
         return;
@@ -1164,7 +1155,7 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     const bool owner = !has_left || lane >= HL;                // lanes whose states this band owns
     uint32_t *g_bp = ws.bp + m.bp_off;
     const double ratio = __ddiv_rn((double)T, (double)S);
-    uint4 *my_x = ws.band_xchg + bi.xoff + 2 * ((lane - (32 - HL)) * K);
+    ulonglong2 *my_x = reinterpret_cast<ulonglong2 *>(ws.band_xchg) + bi.xoff + 2 * ((lane - (32 - HL)) * K);
 
     uint32_t sp_hi[K];
     float jump_cap[K];
@@ -1216,7 +1207,7 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     int st = 0;
     uint32_t phase = 0;
     for (int i = 0; i < n_tiles; ++i) {
-        hfa_mbar_wait(&full[st], phase);
+        hfa_mbar_wait(hfa_smem_u32(&full[st]), phase, HFA_POLLS_COPY);
         const uint32_t tl = tile_sa + (uint32_t)st * (TILE_FLOATS * 4u);
         const uint32_t et = edge_sa + (uint32_t)st * (TT * 8u);
         const int rows = min(TT, T - i * TT);
@@ -1289,14 +1280,15 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             const uint32_t tag = (uint32_t)i + 1u;
 #pragma unroll
             for (int k = 0; k < K; ++k) {
-                uint4 *dst = my_x + (int64_t)i * 64 + 2 * k;
-                hfa_st_slot(dst, make_uint4(__float_as_uint(dp[k]), tag, (uint32_t)__double2loint(p[k]), tag));
-                hfa_st_slot(dst + 1, make_uint4((uint32_t)__double2hiint(p[k]), tag, 0u, tag));
+                ulonglong2 *dst = my_x + (int64_t)i * 64 + 2 * k;
+                hfa_st_xchg(dst, hfa_tagged(__float_as_uint(dp[k]), tag),
+                            hfa_tagged((uint32_t)__double2loint(p[k]), tag));
+                hfa_st_xchg(dst + 1, hfa_tagged((uint32_t)__double2hiint(p[k]), tag), hfa_tagged(0u, tag));
             }
         }
         if (keep) hfa_fence_async_smem();                    // dp rows -> visible to the bulk store
         __syncwarp();                                        // every lane is done with stage `st`
-        if (lane == 0) hfa_mbar_arrive(&empty[st]);
+        if (lane == 0) hfa_mbar_arrive(hfa_smem_u32(&empty[st]));
         if (++st == NST) {
             st = 0;
             phase ^= 1u;

@@ -20,27 +20,27 @@
 // columns, publication, kept-dp bulk store -- and runs ahead of it.  Strip 0 owns states 0..31.
 // Strip w > 0 starts at column 30 w: lanes 0 and 1 are GHOSTS of the left strip's last two
 // states -- they inject the advance scores the left strip published -- and lanes 2..31 own 30 states.
-// A strip publishes {adv[31](t), adv[30](t)} once per iteration (lane 31 has both in registers) into a
-// per-frame slot in HBM/L2: two 64-bit words {f32 bits | tag << 32}, tag = t + 1, each read and written
-// as ONE 64-bit access (single-copy atomic), so a word is valid iff its tag matches -- no flag, no
-// fence; the reader zeroes the slot after use and the table is all-zero between calls.  The right
-// strip fetches 16 frames of slots per 16 iterations and simply runs that far behind.  Work items are
-// claimed through an atomic ticket in (utterance, strip) order, so a strip's left neighbour has
-// always started; strip 0 never waits.
+// A strip publishes {adv[31](t), adv[30](t)} for every frame into a per-frame slot in HBM/L2: lanes 31 and
+// 30 park them in shared memory each iteration, and once per block the producer writes two tagged 64-bit
+// words {f32 bits | tag << 32}, tag = t + 1, per frame (hfa_st_xchg_word: single-copy atomic, so a word
+// is valid iff its tag matches -- no flag, no fence); the reader zeroes the slot after use and the table
+// is all-zero between calls.  The right strip fetches BLK frames of slots per block and simply runs that
+// far behind.  Work items are claimed through an atomic ticket in (utterance, strip) order, so a strip's
+// left neighbour has always started; strip 0 never waits.
 //
 // All shared-memory traffic uses 32-bit shared-window addresses derived from ONE base computed at kernel
 // start (forming generic pointers costs an S2UR + ULEA per use on sm_100).
 //
-// Emissions: ONE TMA tensor-tile copy (cp.async.bulk.tensor.2d, 16 frames x 36 columns: the box must
+// Emissions: ONE TMA tensor-tile copy (cp.async.bulk.tensor.2d, 32 frames x 36 columns: the box must
 // start at a 16-byte boundary, 30 w rounded down to a multiple of 4, so it is 4 columns wider than the
-// strip) per 16 iterations into a ring of NSTG stages (the 32 lanes of a strip span 31 D frames = 4-6 tiles), plus a
-// 128-byte bulk copy of the edge pairs; stage 0 is copied twice, the second time behind the last
-// stage, so a lane's 16 rows of a block are always contiguous and every shared-memory load of the
-// unrolled block is [per-lane base + constant].  Kept dp (for the table backtrace): each iteration's 32
-// values form one 128-byte row of a staging tile that leaves as one 2 KB bulk store per block
-// (hfa_skew_dp_index) -- no halo columns, nothing stored twice.
+// strip) per block of BLK = 32 iterations into a ring of NSTG = 5 stages (the 32 lanes of a strip span
+// 31 D frames = 2-3 tiles), plus a bulk copy of the block's 256 bytes of edge pairs; stage 0 is copied
+// twice, the second time behind the last stage, so a lane's 32 rows of a block are always contiguous and
+// every shared-memory load of the unrolled block is [per-lane base + constant].  Kept dp (for the table
+// backtrace): each iteration's 32 values form one 128-byte row of a staging tile that leaves as one 4 KB
+// bulk store per block (hfa_skew_dp_index) -- no halo columns, nothing stored twice.
 //
-// Three block bodies: the unrolled steady-state one (all 32 lanes inside frames 1 .. T-1 for all 16
+// Three block bodies: the unrolled steady-state one (all 32 lanes inside frames 1 .. T-1 for all 32
 // iterations), the same with a per-lane `live` predicate for the ramps at both ends (and for every block
 // of a dp-dump run), and a rolled one for the single block that seeds frame 0.
 #include <cstdlib>
@@ -48,132 +48,6 @@
 #include "hfa_common.cuh"
 
 namespace {
-
-// ---- shared-memory / mbarrier / TMA helpers on 32-bit shared::cta addresses ----
-__device__ __forceinline__ float sk_lds_f32(uint32_t addr)
-{
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ float2 sk_lds_f2(uint32_t addr)
-{
-    float2 v;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sk_sts_f32(uint32_t addr, float v)
-{
-    asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ int sk_lds_i32(uint32_t addr)
-{
-    int v;
-    asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
-    return v;
-}
-__device__ __forceinline__ void sk_sts_i32(uint32_t addr, int v)
-{
-    asm volatile("st.shared.s32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void sk_mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void sk_mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void sk_mbar_arrive(uint32_t bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// `limit` polls, then trap: a phase that never completes is a bug -- fail loudly, do not hang
-__device__ __forceinline__ void sk_mbar_wait(uint32_t bar, uint32_t parity, uint32_t limit)
-{
-    uint32_t spins = 0;
-    for (;;) {
-        uint32_t ok;
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(ok)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (ok) return;
-        if (++spins > limit) __trap();
-    }
-}
-// non-blocking: has the phase of this parity completed?
-__device__ __forceinline__ bool sk_mbar_test(uint32_t bar, uint32_t parity)
-{
-    uint32_t ok;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void sk_bulk_load(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cta.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ void sk_tensor_load_2d(uint32_t dst, const void *tmap, int x, int y, uint32_t bar)
-{
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cta.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-        "l"(tmap), "r"(x), "r"(y), "r"(bar)
-        : "memory");
-}
-__device__ __forceinline__ void sk_bulk_store(void *dst, uint32_t src, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
-}
-// one lane of a converged warp (ptxas then emits the TMA / bulk instructions once, without an ELECT loop)
-__device__ __forceinline__ bool sk_elect_one()
-{
-    uint32_t pred;
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "elect.sync _|p, 0xffffffff;\n"
-        "selp.u32 %0, 1, 0, p;\n"
-        "}\n"
-        : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void sk_bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void sk_bulk_wait_read_0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-
-// exchange slot of one frame: {adv31 bits | tag << 32, adv30 bits | tag << 32}
-__device__ __forceinline__ ulonglong2 sk_ld_slot(const ulonglong2 *p)
-{
-    ulonglong2 v;
-    asm volatile("ld.relaxed.gpu.global.v2.u64 {%0, %1}, [%2];" : "=l"(v.x), "=l"(v.y) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void sk_st_slot(ulonglong2 *p, unsigned long long a, unsigned long long b)
-{
-    asm volatile("st.relaxed.gpu.global.v2.u64 [%0], {%1, %2};" ::"l"(p), "l"(a), "l"(b) : "memory");
-}
-__device__ __forceinline__ void sk_st_word(unsigned long long *p, unsigned long long a)
-{
-    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(a) : "memory");
-}
-__device__ __forceinline__ unsigned long long sk_pack(float v, uint32_t tag)
-{
-    return (unsigned long long)__float_as_uint(v) | ((unsigned long long)tag << 32);
-}
 
 // One frame of one state with curr carried as P = f64(curr) * ratio (alignment_decoder.py:210-228).
 // Value: max of the three candidates (up2 is already capped where a two-state jump is not allowed).
@@ -245,7 +119,6 @@ constexpr uint32_t SK_DPST_B = BLK * 128u;           // one dp staging tile
 constexpr uint32_t SK_PUB_B = (2 * BLK + BLK + 32) * 4u;   // adv31 [BLK], adv30 [BLK], scratch [BLK + 32]
 constexpr int SK_LOOK = 3;                           // operands are loaded this many iterations ahead
 constexpr int SK_NBUF = 3;                           // dp and publication staging buffers: block j reuses block j - 3's
-static_assert(BLK == 16 || BLK == 32, "a block is one or two backpointer words long");
 
 // shared-memory map (byte offsets from the 128-byte aligned base)
 template <int NSTG> struct SkSmem {
@@ -283,13 +156,14 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     if (threadIdx.x == 0) {
         unsigned hw_slot;
         asm volatile("mov.u32 %0, %%warpid;" : "=r"(hw_slot));
-        sk_sts_i32(sm0 + SM::SLOT + 4u, (int)((hw_slot >> 2) & 1u));
-        sk_sts_i32(sm0 + SM::SLOT, (int)atomicInc(reinterpret_cast<unsigned int *>(ticket), gridDim.x - 1));   // self-resetting
+        hfa_sts_s32(sm0 + SM::SLOT + 4u, (int)((hw_slot >> 2) & 1u));
+        hfa_sts_s32(sm0 + SM::SLOT,
+                    (int)atomicInc(reinterpret_cast<unsigned int *>(ticket), gridDim.x - 1));   // self-resetting
 #pragma unroll
         for (int s = 0; s < NSTG; ++s) {
-            sk_mbar_init(sm0 + SM::FULL + 8u * s, 1);      // the copy issuer (+ the TMA bytes)
-            sk_mbar_init(sm0 + SM::READY + 8u * s, 32);    // every producer lane, after the ghost columns
-            sk_mbar_init(sm0 + SM::DONE + 8u * s, 32);     // every compute lane, after the block
+            hfa_mbar_init(sm0 + SM::FULL + 8u * s, 1);      // the copy issuer (+ the TMA bytes)
+            hfa_mbar_init(sm0 + SM::READY + 8u * s, 32);    // every producer lane, after the ghost columns
+            hfa_mbar_init(sm0 + SM::DONE + 8u * s, 32);     // every compute lane, after the block
         }
         hfa_fence_mbar_init();
     }
@@ -298,8 +172,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
     // (broadcast from lane 0 so that the compiler knows the role is warp-uniform: without it, the compute
     // warp's shuffles are compiled for a possibly diverged warp)
     const bool producer =
-        __shfl_sync(0xffffffffu, (threadIdx.x >> 5) ^ (unsigned)sk_lds_i32(sm0 + SM::SLOT + 4u), 0) != 0;
-    const int item = item_begin + sk_lds_i32(sm0 + SM::SLOT);
+        __shfl_sync(0xffffffffu, (threadIdx.x >> 5) ^ (unsigned)hfa_lds_s32(sm0 + SM::SLOT + 4u), 0) != 0;
+    const int item = item_begin + hfa_lds_s32(sm0 + SM::SLOT);
     const HfaBandItem bi = ws.band_items[item];
     const int u = bi.utt, w = bi.band;
     const HfaUtt m = ws.utt[u];
@@ -326,21 +200,21 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             const int t0 = i * BLK;
             const uint32_t bar = sm0 + SM::FULL + 8u * (uint32_t)st;
             if (t0 >= T) {                                     // nothing to fetch: complete the phase
-                sk_mbar_arrive(bar);
+                hfa_mbar_arrive(bar);
                 return;
             }
             const uint32_t ebytes = (uint32_t)min(BLK, edge_len - t0) * 8u;
             const uint32_t bytes = SK_STG_B + ebytes;
-            sk_mbar_expect_tx(bar, st == 0 ? 2u * bytes : bytes);
-            sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)st * SK_STG_B, tmap, c0 & ~3, t0, bar);
-            sk_bulk_load(sm0 + SM::EDGE + (uint32_t)st * SK_EDGE_B, g_edge + t0, ebytes, bar);
+            hfa_mbar_expect_tx(bar, st == 0 ? 2u * bytes : bytes);
+            hfa_tensor_load_2d(sm0 + SM::TILE + (uint32_t)st * SK_STG_B, tmap, c0 & ~3, t0, bar);
+            hfa_bulk_load(sm0 + SM::EDGE + (uint32_t)st * SK_EDGE_B, g_edge + t0, ebytes, bar);
             if (st == 0) {                                     // the mirror behind the last stage
-                sk_tensor_load_2d(sm0 + SM::TILE + (uint32_t)NSTG * SK_STG_B, tmap, c0 & ~3, t0, bar);
-                sk_bulk_load(sm0 + SM::EDGE + (uint32_t)NSTG * SK_EDGE_B, g_edge + t0, ebytes, bar);
+                hfa_tensor_load_2d(sm0 + SM::TILE + (uint32_t)NSTG * SK_STG_B, tmap, c0 & ~3, t0, bar);
+                hfa_bulk_load(sm0 + SM::EDGE + (uint32_t)NSTG * SK_EDGE_B, g_edge + t0, ebytes, bar);
             }
         };
         static_assert(PF + 1 <= NSTG, "prologue fills distinct stages");
-        if (sk_elect_one())
+        if (hfa_elect_one())
             for (int i = 0; i <= PF && i < NB; ++i) issue(i, i);   // tiles 0 .. PF (tile b + PF + 1 follows block b)
 
         const ulonglong2 *left_x = reinterpret_cast<const ulonglong2 *>(ws.band_xchg) +
@@ -350,7 +224,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         // exchange slots of the block being prepared, fetched one block early (the left strip is normally
         // that far ahead)
         ulonglong2 xv = make_ulonglong2(0ull, 0ull);
-        if (slot_needed(0)) xv = sk_ld_slot(left_x + lane);
+        if (slot_needed(0)) xv = hfa_ld_xchg(left_x + lane);
 
         int a = 0, st_a = 0, buf_b = 0;
         uint32_t par_a = 0;
@@ -359,7 +233,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
         int st_issue = (PF + 1) % NSTG;                        // stage of the next tile to fetch
         uint32_t spins = 0;
         while (b < NB) {
-            if (b < a && __all_sync(0xffffffffu, sk_mbar_test(sm0 + SM::DONE + 8u * (uint32_t)st_b, par_b))) {
+            if (b < a && __all_sync(0xffffffffu, hfa_mbar_test_wait(sm0 + SM::DONE + 8u * (uint32_t)st_b, par_b))) {
                 if (has_right) {
                     // the advance scores lanes 31 and 30 have parked: published as tagged 64-bit words, adv31 of
                     // frame BLK b + i - 31 D into .x, adv30 of frame BLK b + i - 30 D into .y (frames 1 .. T-1 only)
@@ -367,15 +241,16 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     for (int q = lane; q < 2 * BLK; q += 32) {
                         const int half = q / BLK, i = q % BLK;
                         const int t = BLK * b + i - (31 - half) * D;
-                        if (t >= 1 && t < T)
-                            sk_st_word(reinterpret_cast<unsigned long long *>(my_x + t) + half,
-                                       sk_pack(sk_lds_f32(sm0 + SM::PUB + (uint32_t)buf_b * SK_PUB_B + 4u * (uint32_t)q),
-                                               (uint32_t)t + 1u));
+                        if (t >= 1 && t < T) {
+                            const float v = hfa_lds_f32(sm0 + SM::PUB + (uint32_t)buf_b * SK_PUB_B + 4u * (uint32_t)q);
+                            hfa_st_xchg_word(reinterpret_cast<unsigned long long *>(my_x + t) + half,
+                                             hfa_tagged(__float_as_uint(v), (uint32_t)t + 1u));
+                        }
                     }
                 }
-                if (sk_elect_one()) {
+                if (hfa_elect_one()) {
                     if (KEEP && g_dp != nullptr) {             // the block's rows of dp leave as one bulk store
-                        sk_bulk_store(g_dp + (int64_t)b * (BLK * 32), sm0 + SM::DPST + (uint32_t)buf_b * SK_DPST_B,
+                        hfa_bulk_store(g_dp + (int64_t)b * (BLK * 32), sm0 + SM::DPST + (uint32_t)buf_b * SK_DPST_B,
                                       SK_DPST_B);
                         hfa_bulk_commit();
                     }
@@ -392,7 +267,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                 continue;
             }
             if (a < NB && a <= b + SK_NBUF - 1 &&
-                __all_sync(0xffffffffu, sk_mbar_test(sm0 + SM::FULL + 8u * (uint32_t)st_a, par_a))) {
+                __all_sync(0xffffffffu, hfa_mbar_test_wait(sm0 + SM::FULL + 8u * (uint32_t)st_a, par_a))) {
                 bool go = true;
                 if (has_left) {
                     // The left strip's advance scores for frames BLK a .. BLK a + BLK - 1 go where the ghost lanes
@@ -406,22 +281,22 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     const bool ok = !need || ((uint32_t)(xv.x >> 32) == tag && (uint32_t)(xv.y >> 32) == tag);
                     go = __all_sync(0xffffffffu, ok);
                     if (!go) {
-                        if (!ok) xv = sk_ld_slot(src);
+                        if (!ok) xv = hfa_ld_xchg(src);
                     } else {
                         const ulonglong2 v = xv;
-                        xv = slot_needed(a + 1) ? sk_ld_slot(src + BLK) : make_ulonglong2(0ull, 0ull);
+                        xv = slot_needed(a + 1) ? hfa_ld_xchg(src + BLK) : make_ulonglong2(0ull, 0ull);
                         if (lane < BLK) {
                             const float a30 = need ? __uint_as_float((uint32_t)v.y) : 0.0f;
                             const float a31 = need ? __uint_as_float((uint32_t)v.x) : 0.0f;
                             const uint32_t row_sa = sm0 + SM::TILE + (uint32_t)st_a * SK_STG_B + (uint32_t)lane * SK_ROW_B +
                                                     4u * (uint32_t)(c0 & 3);
-                            sk_sts_f32(row_sa, a30);
-                            sk_sts_f32(row_sa + 4u, a31);
+                            hfa_sts_f32(row_sa, a30);
+                            hfa_sts_f32(row_sa + 4u, a31);
                             if (st_a == 0) {                                       // and its mirror
-                                sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B, a30);
-                                sk_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B + 4u, a31);
+                                hfa_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B, a30);
+                                hfa_sts_f32(row_sa + (uint32_t)NSTG * SK_STG_B + 4u, a31);
                             }
-                            if (need) sk_st_slot(src, 0ull, 0ull);                 // leave the table clean
+                            if (need) hfa_st_xchg(src, 0ull, 0ull);                 // leave the table clean
                         }
                         hfa_fence_async_smem();   // generic writes into a stage the TMA engine will refill later
                     }
@@ -429,11 +304,11 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                 if (go) {
                     // block a overwrites the dp staging of block a - SK_NBUF: that bulk store must have been read
                     // out (stores 0 .. b - 1 are in flight; a - SK_NBUF <= b - 2 unless a = b + SK_NBUF - 1)
-                    if (KEEP && a >= SK_NBUF && sk_elect_one()) {
-                        if (a == b + SK_NBUF - 1) sk_bulk_wait_read_0();
-                        else sk_bulk_wait_read_1();
+                    if (KEEP && a >= SK_NBUF && hfa_elect_one()) {
+                        if (a == b + SK_NBUF - 1) hfa_bulk_wait_read<0>();
+                        else hfa_bulk_wait_read<1>();
                     }
-                    sk_mbar_arrive(sm0 + SM::READY + 8u * (uint32_t)st_a);
+                    hfa_mbar_arrive(sm0 + SM::READY + 8u * (uint32_t)st_a);
                     if (++st_a == NSTG) {
                         st_a = 0;
                         par_a ^= 1u;
@@ -444,9 +319,9 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                 }
             }
             // neither step can go: the compute warp is inside its block, or the left strip is behind
-            if (++spins > (1u << 26)) __trap();
+            if (++spins > HFA_POLLS_EXCHANGE) __trap();
         }
-        if (KEEP && sk_elect_one()) hfa_bulk_wait_all();
+        if (KEEP && hfa_elect_one()) hfa_bulk_wait_all();
         return;
     }
 
@@ -517,7 +392,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
 
     for (int j = 0; j < NB; ++j) {
         // READY covers the producer's wait for the left strip as well as the copy: the exchange bound
-        sk_mbar_wait(sm0 + SM::READY + 8u * (uint32_t)st_wait, par_wait, 1u << 26);
+        hfa_mbar_wait(sm0 + SM::READY + 8u * (uint32_t)st_wait, par_wait, HFA_POLLS_EXCHANGE);
         const int st_cur = st_wait;                            // stage that holds frames BLK j .. BLK j + BLK - 1
         if (++st_wait == NSTG) {
             st_wait = 0;
@@ -538,8 +413,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             for (int k = 0; k < BLK; ++k) {
                 const int t = BLK * j + k - lane * D;
                 const bool live = (t >= 1) && (t < T);
-                const float e = sk_lds_f32(e_sa + SK_ROW_B * k);
-                const float2 ed = sk_lds_f2(d_sa + 8u * k);
+                const float e = hfa_lds_f32(e_sa + SK_ROW_B * k);
+                const float2 ed = hfa_lds_f2(d_sa + 8u * k);
                 const float base = __fadd_rn(dp, e);
                 const float stay = __fadd_rn(base, ed.y);
                 const float adv = __double2float_rn(__dadd_rn((double)__fadd_rn(base, ed.x), P));
@@ -553,7 +428,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
 #pragma unroll
                 for (int i = 0; i + 1 < 2 * D; ++i) q2[i] = q2[i + 1];
                 q2[2 * D - 1] = n2;
-                sk_sts_f32(p_sa + 4u * k, advx);
+                hfa_sts_f32(p_sa + 4u * k, advx);
                 const float mm = fmaxf(stay, up1);
                 const bool b1 = up1 > stay, b2 = up2 > mm;
                 const double pe = __dmul_rn((double)e, ratio);
@@ -568,7 +443,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     dp = e;                                    // until the first step has run
                     P = pe;
                 }
-                if (KEEP) sk_sts_f32(k_sa + 128u * k, dp);
+                if (KEEP) hfa_sts_f32(k_sa + 128u * k, dp);
                 if (DUMP) {
                     if (!ghost && s < S && t >= 0 && t < T) dp_dump[m.cell_off + (int64_t)t * S + s] = dp;
                 }
@@ -584,8 +459,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             float2 dv[BLK];
 #pragma unroll
             for (int k = 0; k < SK_LOOK; ++k) {
-                ev[k] = sk_lds_f32(e_sa + SK_ROW_B * k);
-                dv[k] = sk_lds_f2(d_sa + 8u * k);
+                ev[k] = hfa_lds_f32(e_sa + SK_ROW_B * k);
+                dv[k] = hfa_lds_f2(d_sa + 8u * k);
             }
             float r1[BLK + D], r2[BLK + 2 * D];
 #pragma unroll
@@ -597,8 +472,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
 #pragma unroll
                 for (int k = 0; k < BLK; ++k) {
                     if (k + SK_LOOK < BLK) {
-                        ev[k + SK_LOOK] = sk_lds_f32(e_sa + SK_ROW_B * (k + SK_LOOK));
-                        dv[k + SK_LOOK] = sk_lds_f2(d_sa + 8u * (k + SK_LOOK));
+                        ev[k + SK_LOOK] = hfa_lds_f32(e_sa + SK_ROW_B * (k + SK_LOOK));
+                        dv[k + SK_LOOK] = hfa_lds_f2(d_sa + 8u * (k + SK_LOOK));
                     }
                     const float e = ev[k];
                     const float base = __fadd_rn(dp, e);
@@ -607,11 +482,11 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     const float advx = ghost ? e : adv;
                     r1[k + D] = fminf(__shfl_up_sync(0xffffffffu, advx, 1), cap1);
                     r2[k + 2 * D] = fminf(__shfl_up_sync(0xffffffffu, advx, 2), jcap);
-                    sk_sts_f32(p_sa + 4u * k, advx);
+                    hfa_sts_f32(p_sa + 4u * k, advx);
                     const double pe = __dmul_rn((double)e, ratio);
                     sk_select(r1[k], stay, r2[k], pe, sp_hi, mr, dp, P, acc);
                     mr = __funnelshift_l(mr, mr, 1);
-                    if (KEEP) sk_sts_f32(k_sa + 128u * k, dp);
+                    if (KEEP) hfa_sts_f32(k_sa + 128u * k, dp);
                     if ((k & 15) == 15) {
                         flush_bits(acc, true);
                         acc = 0;
@@ -622,8 +497,8 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
 #pragma unroll
                 for (int k = 0; k < BLK; ++k) {
                     if (k + SK_LOOK < BLK) {
-                        ev[k + SK_LOOK] = sk_lds_f32(e_sa + SK_ROW_B * (k + SK_LOOK));
-                        dv[k + SK_LOOK] = sk_lds_f2(d_sa + 8u * (k + SK_LOOK));
+                        ev[k + SK_LOOK] = hfa_lds_f32(e_sa + SK_ROW_B * (k + SK_LOOK));
+                        dv[k + SK_LOOK] = hfa_lds_f2(d_sa + 8u * (k + SK_LOOK));
                     }
                     const int live = (unsigned)(tb + k) < (unsigned)(T - 1);     // 1 <= t <= T-1
                     const float e = ev[k];
@@ -633,11 +508,11 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     const float advx = ghost ? e : adv;
                     r1[k + D] = fminf(__shfl_up_sync(0xffffffffu, advx, 1), cap1);
                     r2[k + 2 * D] = fminf(__shfl_up_sync(0xffffffffu, advx, 2), jcap);
-                    sk_sts_f32(p_sa + 4u * k, advx);
+                    hfa_sts_f32(p_sa + 4u * k, advx);
                     const double pe = __dmul_rn((double)e, ratio);
                     sk_select_guarded(r1[k], stay, r2[k], pe, sp_hi, mr, live, dp, P, acc);
                     mr = __funnelshift_l(mr, mr, 1);
-                    if (KEEP) sk_sts_f32(k_sa + 128u * k, dp);
+                    if (KEEP) hfa_sts_f32(k_sa + 128u * k, dp);
                     if (DUMP) {
                         const int t = tb + 1 + k;
                         if (!ghost && s < S && t >= 0 && t < T) dp_dump[m.cell_off + (int64_t)t * S + s] = dp;
@@ -654,7 +529,7 @@ hfa_dp_skew_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
             for (int i = 0; i < 2 * D; ++i) q2[i] = r2[BLK + i];
         }
         if (KEEP) hfa_fence_async_smem();                      // this block's dp rows -> visible to the bulk store
-        sk_mbar_arrive(sm0 + SM::DONE + 8u * (uint32_t)st_cur);   // the stage, the staging rows: the producer's now
+        hfa_mbar_arrive(sm0 + SM::DONE + 8u * (uint32_t)st_cur);   // the stage, the staging rows: the producer's now
         if (++buf == SK_NBUF) buf = 0;
         u_row += BLK;
         if (u_row >= R) u_row -= R;
@@ -704,8 +579,8 @@ cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int item_begin, int
     // HFA_SKEW_SLOW=1: every block through the guarded body (A/B against the unrolled steady state)
     const char *sl = getenv("HFA_SKEW_SLOW");
     const int force_slow = (sl && sl[0] == '1') ? 1 : 0;
-    constexpr int NS = HFA_SKEW_BLK == 32 ? 5 : 12;            // a ring of 160 / 192 frames
-    if (d == 2) return launch_skew_d<2, NS>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
-    if (d == 3) return launch_skew_d<3, NS>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+    // a ring of 5 blocks: 160 frames
+    if (d == 2) return launch_skew_d<2, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+    if (d == 3) return launch_skew_d<3, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
     return cudaErrorInvalidValue;
 }

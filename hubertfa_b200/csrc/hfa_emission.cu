@@ -42,13 +42,6 @@ __device__ __forceinline__ void edge_logs(float p, float p_prev, float2 &out)
     out.y = (float)log(__dadd_rn(__dsub_rn(1.0, ep), 1e-6));          // :242  (1 - ep) + 1e-6
 }
 
-__device__ __forceinline__ float lds_f32(uint32_t addr)
-{
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
-
 // The emission kernels stage an utterance's ids in shared memory for at most this many states (sp_cap =
 // min(largest Sp of the batch, HFA_EMIS_ID_CAP)), so one long utterance cannot lower the occupancy of its whole
 // batch.  The ids of the states past the staged ones (S > HFA_CTA_MAX_S only) are read from global memory.
@@ -65,12 +58,7 @@ __device__ __forceinline__ int4 hfa_ids4(const int32_t *ids, int S, int V, int s
 // fetches the whole 128-byte line around it from HBM (ncu, config 4: 460 MB read for 3.7 M frames).  The 64-byte
 // fetch-granularity hint is the smallest PTX offers; the rest of the line belongs to the emission kernel's copy.
 template <typename TIn> __device__ __forceinline__ float hfa_ld_edge(const TIn *p);
-template <> __device__ __forceinline__ float hfa_ld_edge<float>(const float *p)
-{
-    float v;
-    asm volatile("ld.global.L2::64B.f32 %0, [%1];" : "=f"(v) : "l"(p));
-    return v;
-}
+template <> __device__ __forceinline__ float hfa_ld_edge<float>(const float *p) { return hfa_ldg_f32_64B(p); }
 template <> __device__ __forceinline__ float hfa_ld_edge<__half>(const __half *p)
 {
     unsigned short v;
@@ -194,7 +182,7 @@ hfa_emission_block_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
         float sum = 0.0f;
-        for (int k = part; k < n_kept; k += 4) sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(row[kept_sm[k]], mx)));
+        for (int k = part; k < n_kept; k += 4) sum = __fadd_rn(sum, expf(__fsub_rn(row[kept_sm[k]], mx)));
         sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
         sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
         if (part == 0) stat_sm[tid >> 2] = make_float2(mx, logf(sum));
@@ -223,16 +211,16 @@ hfa_emission_block_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
             const float2 st = stat_sm[rr];
             const uint32_t rb = xs_sa + (uint32_t)(rr * VP) * 4u;
             float4 o;
-            o.x = __fsub_rn(__fsub_rn(lds_f32(rb + goff[0][0]), st.x), st.y);
-            o.y = __fsub_rn(__fsub_rn(lds_f32(rb + goff[0][1]), st.x), st.y);
-            o.z = __fsub_rn(__fsub_rn(lds_f32(rb + goff[0][2]), st.x), st.y);
-            o.w = __fsub_rn(__fsub_rn(lds_f32(rb + goff[0][3]), st.x), st.y);
+            o.x = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[0][0]), st.x), st.y);
+            o.y = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[0][1]), st.x), st.y);
+            o.z = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[0][2]), st.x), st.y);
+            o.w = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[0][3]), st.x), st.y);
             if (st0) *reinterpret_cast<float4 *>(dst + r * dst_step) = o;
             if (Sp > 128) {                                                  // warp-uniform
-                o.x = __fsub_rn(__fsub_rn(lds_f32(rb + goff[1][0]), st.x), st.y);
-                o.y = __fsub_rn(__fsub_rn(lds_f32(rb + goff[1][1]), st.x), st.y);
-                o.z = __fsub_rn(__fsub_rn(lds_f32(rb + goff[1][2]), st.x), st.y);
-                o.w = __fsub_rn(__fsub_rn(lds_f32(rb + goff[1][3]), st.x), st.y);
+                o.x = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[1][0]), st.x), st.y);
+                o.y = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[1][1]), st.x), st.y);
+                o.z = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[1][2]), st.x), st.y);
+                o.w = __fsub_rn(__fsub_rn(hfa_lds_f32(rb + goff[1][3]), st.x), st.y);
                 if (st1) *reinterpret_cast<float4 *>(dst + r * dst_step + 128) = o;
             }
         }
@@ -296,7 +284,7 @@ __device__ __forceinline__ void hfa_row_stats(const TIn *row, const int (&kreg)[
     mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
 #pragma unroll
     for (int j = 0; j < NJ; ++j)             // entries past the end are -inf: exp = +0, sum unchanged
-        sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(xv[j], mx)));
+        sum = __fadd_rn(sum, expf(__fsub_rn(xv[j], mx)));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -343,12 +331,12 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
         const uint32_t bytes =
             (shift + (uint32_t)(((int64_t)(rows - 1) * in.frame_st + V) * (int64_t)sizeof(TIn)) + 15u) & ~15u;
         shift_sm[s] = (int32_t)shift;
-        hfa_mbar_expect_tx(&bar[s], bytes);
-        hfa_bulk_load(stage0 + (size_t)s * stage_bytes, src - shift, bytes, &bar[s]);
+        hfa_mbar_expect_tx(hfa_smem_u32(&bar[s]), bytes);
+        hfa_bulk_load(hfa_smem_u32(stage0 + (size_t)s * stage_bytes), src - shift, bytes, hfa_smem_u32(&bar[s]));
     };
     if (tid == 0) {
-        hfa_mbar_init(&bar[0], 1);
-        hfa_mbar_init(&bar[1], 1);
+        hfa_mbar_init(hfa_smem_u32(&bar[0]), 1);
+        hfa_mbar_init(hfa_smem_u32(&bar[1]), 1);
         hfa_fence_mbar_init();
         issue(blk0, 0);
     }
@@ -416,7 +404,8 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
         const int t_base = (blk - ws.row_blocks[u]) * HFA_EMIS_ROWS;
         const int row_st = (int)in.frame_st;
 
-        hfa_mbar_wait(&bar[s], (uint32_t)(((blk - blk0) >> 1) & 1));
+        const uint32_t parity = ((blk - blk0) >> 1) & 1;
+        hfa_mbar_wait(hfa_smem_u32(&bar[s]), parity, HFA_POLLS_COPY);
         const TIn *xs = reinterpret_cast<const TIn *>(stage0 + (size_t)s * stage_bytes + shift_sm[s]);
 
         // C. normaliser, warp-local: lane -> (row = 8 * warp + lane / 4, part = lane % 4), kept ids
@@ -443,7 +432,7 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
                 mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
                 mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
                 for (int k = part; k < n_kept; k += 4)
-                    sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(hfa_to_float<TIn>(row[kept_sm[k]]), mx)));
+                    sum = __fadd_rn(sum, expf(__fsub_rn(hfa_to_float<TIn>(row[kept_sm[k]]), mx)));
             }
             sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
             sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
@@ -584,7 +573,7 @@ hfa_emission_wide_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
         }
         mr = warp_max(mr);
         float sum = 0.0f;
-        for (int v = lane; v < V; v += 32) sum = __fadd_rn(sum, hfa_exp_neg(__fsub_rn(rowbuf[v], mr)));
+        for (int v = lane; v < V; v += 32) sum = __fadd_rn(sum, expf(__fsub_rn(rowbuf[v], mr)));
         const float l = logf(warp_sum(sum));
         __syncwarp();
         float *dst = g_out + (int64_t)t * Sp;
