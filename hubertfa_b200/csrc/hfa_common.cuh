@@ -320,6 +320,15 @@ template <> __device__ __forceinline__ float hfa_to_float<__nv_bfloat16>(__nv_bf
     return __bfloat162float(v);
 }
 
+// {max, log-sum} of one emission row from the max and the sum of exp(x - max) over the logits the
+// normaliser reads; every emission is then (x[id] - max) - log-sum.  A max of -inf means every logit read
+// is -inf: exp(-inf - -inf) made the sum NaN, so the row takes {0, 0} and every emission stays the
+// logit itself, -inf (the reference's masked logits are finite there and its emissions are -inf as well).
+__device__ __forceinline__ float2 hfa_row_stat(float mx, float sum)
+{
+    return mx == HFA_NEG_INF ? make_float2(0.0f, 0.0f) : make_float2(mx, logf(sum));
+}
+
 // typed views of the caller's result blob (layout: HfaResultLayout in include/hfa_align.h)
 struct HfaResultPtrs {
     int32_t *status, *n_seg, *end_state;

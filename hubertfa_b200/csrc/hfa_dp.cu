@@ -1072,7 +1072,7 @@ hfa_dp_band_kernel(HfaWs ws, int item_begin, int32_t *ticket, float *__restrict_
                     }
                     sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
                     sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
-                    if (part == 0) stat_sm[rr] = make_float2(mx, logf(sum));
+                    if (part == 0) stat_sm[rr] = hfa_row_stat(mx, sum);
                 }
                 __syncwarp();
                 // gather by phoneme id: K window columns per lane, the layout the compute warp reads;

@@ -185,7 +185,7 @@ hfa_emission_block_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
         for (int k = part; k < n_kept; k += 4) sum = __fadd_rn(sum, expf(__fsub_rn(row[kept_sm[k]], mx)));
         sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
         sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
-        if (part == 0) stat_sm[tid >> 2] = make_float2(mx, logf(sum));
+        if (part == 0) stat_sm[tid >> 2] = hfa_row_stat(mx, sum);
     }
     __syncthreads();
 
@@ -436,7 +436,7 @@ hfa_emission_stream_kernel(HfaWs ws, int n_blocks, int V, int sp_cap, int stage_
             }
             sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 1));
             sum = __fadd_rn(sum, __shfl_xor_sync(0xffffffffu, sum, 2));
-            if (part == 0) stat_sm[rr] = make_float2(mx, logf(sum));
+            if (part == 0) stat_sm[rr] = hfa_row_stat(mx, sum);
         }
         __syncwarp();
 
@@ -574,7 +574,10 @@ hfa_emission_wide_kernel(HfaWs ws, int n_utt, int V, int sp_cap)
         mr = warp_max(mr);
         float sum = 0.0f;
         for (int v = lane; v < V; v += 32) sum = __fadd_rn(sum, expf(__fsub_rn(rowbuf[v], mr)));
-        const float l = logf(warp_sum(sum));
+        // every logit of the row -inf: the reference's rows are NaN, ours -inf (hfa_row_stat, DESIGN 4.1)
+        const float2 st = hfa_row_stat(mr, warp_sum(sum));
+        mr = st.x;
+        const float l = st.y;
         __syncwarp();
         float *dst = g_out + (int64_t)t * Sp;
         for (int s4 = lane * 4; s4 < Sp; s4 += 128) {

@@ -19,6 +19,47 @@ def run_core_gpu(ids_list, prob_logs, els, nes, ps=None, frame_length=0.02, voca
     T = [p.shape[0] for p in prob_logs]
     S = [len(i) for i in ids_list]
     plan = ops.AlignPlan(T, S, np.concatenate(ids_list), vocab, frame_length)
+    cat = lambda xs, dt: torch.from_numpy(np.concatenate([np.asarray(x, dtype=dt).reshape(-1) for x in xs])).to(dev)
+    pl, el, ne = cat(prob_logs, np.float32), cat(els, np.float32), cat(nes, np.float32)
+    pp = cat(ps, np.float32) if ps is not None else None
+    return _run_plan(plan, lambda ws: ops.pack_emissions(ws, plan.handle, pl, el, ne, pp), dump)
+
+
+def run_core_from_logits(frames, edges, ids_list, vocab, frame_length=0.02, sample=None):
+    """Tier 1 from logits: hfa_emission fills the workspace from the logits views `frames` / `edges` (CUDA
+    tensors, one per utterance), then the DP and backtrace run as in run_core_gpu.  Returns (plan, results,
+    inputs): inputs[b] = (emissions [T, S], edge_log, not_edge_log, edge_p) exactly as the DP read them, for
+    check_core_against_oracle.  `sample`: the utterances to return (default all)."""
+    T = [int(f.shape[0]) for f in frames]
+    S = [len(i) for i in ids_list]
+    plan = ops.AlignPlan(T, S, np.concatenate(ids_list), vocab, frame_length)
+    got = {}
+
+    def fill(ws):
+        plan.set_inputs(ws, [f.data_ptr() for f in frames], [f.stride(0) for f in frames],
+                        [f.stride(1) for f in frames], [e.data_ptr() for e in edges], [e.stride(0) for e in edges])
+        ops.emission(ws, plan.handle, ops.TORCH_TO_DTYPE[frames[0].dtype])
+        got["emis"] = ops.unpack_emissions(plan, ws).cpu().numpy()
+        got["edge2"] = plan.debug_region(ws, "edge2").cpu().numpy().copy()
+        got["edge_p"] = plan.debug_region(ws, "edge_p").cpu().numpy().copy()
+
+    out = _run_plan(plan, fill, True, sample)
+    inputs, cell, eo = {}, 0, 0
+    for b in range(plan.n_utt):
+        if T[b] < 1 or S[b] < 1:
+            continue
+        if sample is None or b in sample:
+            e2 = got["edge2"][eo:eo + T[b]]
+            inputs[b] = (got["emis"][cell:cell + T[b] * S[b]].reshape(T[b], S[b]).copy(), e2[:, 0].copy(),
+                         e2[:, 1].copy(), got["edge_p"][eo:eo + T[b]].copy())
+        cell += T[b] * S[b]
+        eo += (T[b] + 15) // 16 * 16
+    return plan, out, inputs
+
+
+def _run_plan(plan, fill, dump, sample=None):
+    dev = torch.device("cuda")
+    T, S = [int(t) for t in plan.T], [int(s) for s in plan.S]
     # compute-sanitizer is closed on this pool: the workspace and the result blob sit between guard zones
     # filled with a pattern, checked after the kernels have run (an out-of-bounds write of any kernel in any
     # routing fails the test)
@@ -27,10 +68,7 @@ def run_core_gpu(ids_list, prob_logs, els, nes, ps=None, frame_length=0.02, voca
     res_all = torch.full((G + plan.result_bytes + G,), 0x5A, dtype=torch.uint8, device=dev)
     ws, res = ws_all[G:G + max(plan.workspace_bytes, 256)], res_all[G:G + plan.result_bytes]
     plan.upload(ws)
-    cat = lambda xs, dt: torch.from_numpy(np.concatenate([np.asarray(x, dtype=dt).reshape(-1) for x in xs])).to(dev)
-    pl, el, ne = cat(prob_logs, np.float32), cat(els, np.float32), cat(nes, np.float32)
-    pp = cat(ps, np.float32) if ps is not None else None
-    ops.pack_emissions(ws, plan.handle, pl, el, ne, pp)
+    fill(ws)
     dp_dump = torch.full((max(plan.total_cells, 1),), float("nan"), dtype=torch.float32, device=dev) if dump else None
     ops.viterbi_forward(ws, plan.handle, dp_dump)
     bt_dump = None
@@ -42,7 +80,8 @@ def run_core_gpu(ids_list, prob_logs, els, nes, ps=None, frame_length=0.02, voca
         bt_dump = []
         for b in range(plan.n_utt):
             try:
-                bt_dump.append(ops.unpack_backptr(plan, ws, b).cpu().numpy())
+                bt_dump.append(ops.unpack_backptr(plan, ws, b).cpu().numpy() if sample is None or b in sample
+                               else None)
             except ops.HfaError:                      # invalid utterance: no backpointers
                 bt_dump.append(None)
         plan.debug_region(ws, "bp").fill_(-1)
@@ -58,6 +97,11 @@ def run_core_gpu(ids_list, prob_logs, els, nes, ps=None, frame_length=0.02, voca
     dump_h = dp_dump.cpu().numpy() if dump else None
     out, cell = [], 0
     for b in range(plan.n_utt):
+        if sample is not None and b not in sample:
+            if int(v["status"][b]) in (0, 4):
+                cell += T[b] * S[b]
+            out.append(None)
+            continue
         o, k = int(plan.seg_off[b]), int(v["n_seg"][b])
         f0, f1 = int(plan.frame_off[b]), int(plan.frame_off[b + 1])
         d = dict(status=int(v["status"][b]), n_seg=k, end_state=int(v["end_state"][b]),
@@ -121,3 +165,19 @@ def synth_core_inputs(T, S, V, seed, style="dictionary", planted=False):
     el, ne = onp.edge_logs(ep)
     return dict(ids=ids, prob_log=np.ascontiguousarray(lp[:, ids]), el=el, ne=ne, p=p, frame=frame,
                 edge=edge, ph_seq=ph_seq, word_seq=word_seq, ph2w=ph2w, vocab=vocab)
+
+
+def pairable_ids(rng, S, lead, trail, max_word):
+    """Random sequence without adjacent SPs: [SP] word SP word ... [SP], words of 1..max_word phonemes."""
+    ids = [0] if lead else []
+    while len(ids) < S:
+        ids += [int(x) for x in rng.integers(1, 30, int(rng.integers(1, max_word + 1)))]
+        ids.append(0)
+    ids = ids[:S]
+    if trail:
+        if S >= 2 and ids[-2] == 0:
+            ids[-2] = 7
+        ids[-1] = 0
+    elif ids[-1] == 0 and (S == 1 or ids[-2] != 0):
+        ids[-1] = 9 if not (S == 1 and lead) else 0
+    return np.array(ids, dtype=np.int32)

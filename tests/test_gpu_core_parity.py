@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from conftest import golden_names
-from gpu_util import bits, check_core_against_oracle, run_core_gpu, synth_core_inputs
+from gpu_util import bits, check_core_against_oracle, pairable_ids, run_core_gpu, synth_core_inputs
 from oracle import c_oracle as oc
 from oracle import hfa_oracle_np as onp
 
@@ -115,22 +115,6 @@ def test_ties_go_to_the_earlier_candidate(routing):
         check_core_against_oracle(c[0], c[1], c[2], c[3], g)
 
 
-def _pairable_ids(rng, S, lead, trail, max_word):
-    """Random sequence without adjacent SPs: [SP] word SP word ... [SP], words of 1..max_word phonemes."""
-    ids = [0] if lead else []
-    while len(ids) < S:
-        ids += [int(x) for x in rng.integers(1, 30, int(rng.integers(1, max_word + 1)))]
-        ids.append(0)
-    ids = ids[:S]
-    if trail:
-        if S >= 2 and ids[-2] == 0:
-            ids[-2] = 7
-        ids[-1] = 0
-    elif ids[-1] == 0 and (S == 1 or ids[-2] != 0):
-        ids[-1] = 9 if not (S == 1 and lead) else 0
-    return np.array(ids, dtype=np.int32)
-
-
 @pytest.mark.parametrize("pair", ["2", "0"], ids=["pair-layout", "plain-layout"])
 def test_sp_pair_layout_edge_cases(pair, monkeypatch):
     """The SP-aware pair layout of the warp kernel (hfa_dp_pair_body) on the shapes its regrouping has to get
@@ -147,7 +131,7 @@ def test_sp_pair_layout_edge_cases(pair, monkeypatch):
               (25, 64), (40, 65), (33, 100), (64, 128), (70, 150), (50, 200), (41, 213), (90, 256), (300, 90)]
     for i, (T, S) in enumerate(shapes * 3):
         lead, trail, mw = bool(i & 1), bool(i & 2), 1 + i % 4
-        ids = _pairable_ids(rng, S, lead, trail, mw)
+        ids = pairable_ids(rng, S, lead, trail, mw)
         mode = i % 4
         if mode == 0:
             e = (-rng.exponential(3.0, (T, S))).astype(np.float32)
