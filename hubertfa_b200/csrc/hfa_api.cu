@@ -10,6 +10,7 @@
 #include <mutex>
 #include <new>
 #include <numeric>
+#include <queue>
 #include <unordered_map>
 #include <vector>
 
@@ -26,8 +27,8 @@ cudaError_t hfa_launch_dp_warp_any(const HfaLaunchCtx &c, int max_k, int max_pai
 cudaError_t hfa_launch_dp_cta(const HfaLaunchCtx &c, const int32_t *order, int n, int max_sp, float *dp_dump);
 cudaError_t hfa_launch_dp_band(const HfaLaunchCtx &c, int k, int item_begin, int n_items, int32_t *ticket,
                                bool keep_dp, int64_t fused_row_stride, float *dp_dump);
-cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int item_begin, int n_items, int32_t *ticket,
-                               bool keep_dp, float *dp_dump);
+cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int ctas_per_sm, int item_begin, int n_items,
+                               int32_t *ticket, bool keep_dp, float *dp_dump);
 cudaError_t hfa_launch_emission(const HfaLaunchCtx &c, int total_row_blocks, int max_sp, int dtype,
                                 int64_t max_row_stride, int *n_launched);
 cudaError_t hfa_launch_edge(const HfaLaunchCtx &c, int total_row_blocks, int dtype);
@@ -130,6 +131,31 @@ int sm_count()
     return n;
 }
 
+// Length in blocks of a launch of the skewed kernel when `slots` CTAs are resident: a list schedule of the strips in
+// ticket order (each claims the first slot that frees up) in which every block takes the same time and a strip's
+// blocks trail its left neighbour's by ceil(31 d / 32) + 1 blocks (block j waits for the left strip's block
+// j + ceil(31 d / 32) to be published).
+int64_t skew_makespan(const std::vector<HfaBandItem> &items, int begin, int count, const std::vector<HfaUtt> &utt,
+                      int d, int64_t slots)
+{
+    const int64_t lag = (31 * d + HFA_SKEW_BLK - 1) / HFA_SKEW_BLK + 1;
+    std::priority_queue<int64_t, std::vector<int64_t>, std::greater<int64_t>> free_at;
+    int64_t makespan = 0, left_start = 0;
+    for (int i = begin; i < begin + count; ++i) {
+        int64_t start = 0;
+        if ((int64_t)free_at.size() == slots) {
+            start = free_at.top();
+            free_at.pop();
+        }
+        if (items[i].band > 0) start = std::max(start, left_start + lag);
+        const int64_t end = start + hfa_skew_blocks(d, utt[items[i].utt].T);
+        free_at.push(end);
+        left_start = start;
+        makespan = std::max(makespan, end);
+    }
+    return makespan;
+}
+
 }  // namespace
 
 // Workspace layout (byte offsets from the workspace base, every region 256-byte aligned):
@@ -160,6 +186,8 @@ struct hfa_plan {
     // > 0: the list runs in the skewed-wavefront kernel (hfa_dp_skew.cu) with this many frames of skew
     // per state -- 32 / 30-state strips, one state per lane -- instead of the halo bands
     int32_t band_skew[2] = {0, 0};
+    // strips of the skewed kernel resident per SM (4 or 5: the kernel's ring has 6 or 5 stages)
+    int32_t skew_ctas[2] = {5, 5};
     int64_t band_xchg_elems = 0, dp_store_elems = 0;
     std::vector<int32_t> jblk_utt, jblk_first; // jump-table kernel: 256-word blocks per utterance
     int32_t n_valid = 0, n_kept = 0;           // valid utterances / utterances that keep dp
@@ -509,6 +537,25 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         };
         add_bands(lat_band, 0);
         add_bands(big_band, 1);
+        // Strips per SM.  Five 2-warp CTAs put two compute warps on one scheduler partition; four give each its
+        // own partition, which shortens the block period of the critical chain (DESIGN §4.3), but fewer strips
+        // start in the first wave.  Four when the list schedule is not longer with them (configs 1-3: the
+        // strips that miss the first wave belong to short utterances), five otherwise (512 utterances and up).
+        // HFA_SKEW_CTAS = 4 | 5 forces one residency (tests run both ring sizes on the same batches).
+        int force_ctas = 0;
+        if (const char *e = std::getenv("HFA_SKEW_CTAS")) force_ctas = std::atoi(e);
+        for (int wh = 0; wh < 2; ++wh) {
+            if (p->band_skew[wh] <= 0 || p->band_count[wh] == 0) continue;
+            if (force_ctas == 4 || force_ctas == 5) {
+                p->skew_ctas[wh] = force_ctas;
+                continue;
+            }
+            const int64_t m4 = skew_makespan(p->band_items, p->band_begin[wh], p->band_count[wh], p->utt,
+                                             p->band_skew[wh], 4LL * sm_count());
+            const int64_t m5 = skew_makespan(p->band_items, p->band_begin[wh], p->band_count[wh], p->utt,
+                                             p->band_skew[wh], 5LL * sm_count());
+            p->skew_ctas[wh] = m4 <= m5 ? 4 : 5;
+        }
         // jump-table kernel (backtrace of the utterances that keep dp): one thread per backpointer word
         p->n_valid = (int32_t)all.size();
         for (const HfaUtt &m : p->utt) p->n_kept += (m.status == 0 && m.dp_off >= 0);
@@ -742,6 +789,11 @@ int hfa_plan_routing(const hfa_plan *p, int32_t out[8])
 }
 
 int32_t hfa_plan_pair_utterances(const hfa_plan *p) { return p ? p->pair_count : 0; }
+int32_t hfa_plan_skew_ctas_per_sm(const hfa_plan *p, int32_t list)
+{
+    if (!p || list < 0 || list > 1) return 0;
+    return (p->band_skew[list] > 0 && p->band_count[list] > 0) ? p->skew_ctas[list] : 0;
+}
 int64_t hfa_plan_stored_emission_bytes(const hfa_plan *p) { return p ? p->stored_emis * 4 : 0; }
 
 int64_t hfa_plan_debug_region(const hfa_plan *p, int32_t which, int64_t *n_bytes)
@@ -753,6 +805,7 @@ int64_t hfa_plan_debug_region(const hfa_plan *p, int32_t which, int64_t *n_bytes
         case 1: off = p->o_edge2; n = p->total_edge * 8; break;
         case 2: off = p->o_edgep; n = p->total_edge * 4; break;
         case 3: off = p->o_bp; n = p->total_words * 4; break;
+        case 4: off = p->o_band_xchg; n = p->band_xchg_elems * 16; break;
         default: break;
     }
     if (n_bytes) *n_bytes = n;
@@ -969,7 +1022,7 @@ static int viterbi_forward_impl(const hfa_plan *p, void *workspace, float *dp_du
         else if (items[it].k == -3 || items[it].k == -4) {
             const int wh = items[it].k == -3 ? 0 : 1;
             if (p->band_skew[wh] > 0)
-                e = hfa_launch_dp_skew(c, p->band_skew[wh], p->band_begin[wh], p->band_count[wh],
+                e = hfa_launch_dp_skew(c, p->band_skew[wh], p->skew_ctas[wh], p->band_begin[wh], p->band_count[wh],
                                        c.ws.band_ticket + wh, p->dp_store_elems > 0, dp_dump);
             else
                 e = hfa_launch_dp_band(c, p->band_k[wh], p->band_begin[wh], p->band_count[wh],

@@ -33,12 +33,12 @@
 //
 // Emissions: ONE TMA tensor-tile copy (cp.async.bulk.tensor.2d, 32 frames x 36 columns: the box must
 // start at a 16-byte boundary, 30 w rounded down to a multiple of 4, so it is 4 columns wider than the
-// strip) per block of BLK = 32 iterations into a ring of NSTG = 5 stages (the 32 lanes of a strip span
-// 31 D frames = 2-3 tiles), plus a bulk copy of the block's 256 bytes of edge pairs; stage 0 is copied
-// twice, the second time behind the last stage, so a lane's 32 rows of a block are always contiguous and
-// every shared-memory load of the unrolled block is [per-lane base + constant].  Kept dp (for the table
-// backtrace): each iteration's 32 values form one 128-byte row of a staging tile that leaves as one 4 KB
-// bulk store per block (hfa_skew_dp_index) -- no halo columns, nothing stored twice.
+// strip) per block of BLK = 32 iterations into a ring of NSTG = 5 or 6 stages (the 32 lanes of a strip span
+// 31 D frames = 2-3 tiles; the stage count sets how many CTAs share an SM), plus a bulk copy of the block's
+// 256 bytes of edge pairs; stage 0 is copied twice, the second time behind the last stage, so a lane's 32
+// rows of a block are always contiguous and every shared-memory load of the unrolled block is
+// [per-lane base + constant].  Kept dp (for the table backtrace): each iteration's 32 values form one
+// 128-byte row of a staging tile that leaves as one 4 KB bulk store per block (hfa_skew_dp_index) -- no halo columns, nothing stored twice.
 //
 // Three block bodies: the unrolled steady-state one (all 32 lanes inside frames 1 .. T-1 for all 32
 // iterations), the same with a per-lane `live` predicate for the ramps at both ends (and for every block
@@ -570,17 +570,24 @@ cudaError_t launch_skew_d(const HfaLaunchCtx &c, int item_begin, int n_items, in
 }  // namespace
 
 // skewed kernel: items [item_begin, item_begin + n_items) of the plan's strip table, one 2-warp CTA each.
-// d = frames of skew per state (2 or 3, fixed when the plan was made: the dp store layout depends on it)
-cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int item_begin, int n_items, int32_t *ticket,
-                               bool keep_dp, float *dp_dump)
+// d = frames of skew per state (2 or 3, fixed when the plan was made: the dp store layout depends on it).
+// ctas_per_sm = strips resident per SM, the plan's choice: a ring of 5 stages (43 144 B of shared memory) lets
+// 5 CTAs share an SM, 6 stages (48 032 B) only 4 -- one compute warp per scheduler partition, one more tile
+// fetched ahead.
+cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int ctas_per_sm, int item_begin, int n_items,
+                               int32_t *ticket, bool keep_dp, float *dp_dump)
 {
     if (n_items <= 0) return cudaSuccess;
     if (c.ws.tmaps == nullptr) return cudaErrorNotSupported;
     // HFA_SKEW_SLOW=1: every block through the guarded body (A/B against the unrolled steady state)
     const char *sl = getenv("HFA_SKEW_SLOW");
     const int force_slow = (sl && sl[0] == '1') ? 1 : 0;
-    // a ring of 5 blocks: 160 frames
-    if (d == 2) return launch_skew_d<2, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
-    if (d == 3) return launch_skew_d<3, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+    if (ctas_per_sm == 4) {
+        if (d == 2) return launch_skew_d<2, 6>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+        if (d == 3) return launch_skew_d<3, 6>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+    } else if (ctas_per_sm == 5) {
+        if (d == 2) return launch_skew_d<2, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+        if (d == 3) return launch_skew_d<3, 5>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
+    }
     return cudaErrorInvalidValue;
 }

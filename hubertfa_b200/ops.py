@@ -73,6 +73,8 @@ class AlignPlan:
         return dict(warp_utts=out[0], band_warps=out[1], band_k=out[2], big_band_warps=out[3],
                     big_band_k=out[4], cta_utts=out[5], keeps_dp=bool(out[6]), skew_d=out[7],
                     pair_utts=int(self._lib.hfa_plan_pair_utterances(self._h)),
+                    skew_ctas_per_sm=int(self._lib.hfa_plan_skew_ctas_per_sm(self._h, 0)),
+                    big_skew_ctas_per_sm=int(self._lib.hfa_plan_skew_ctas_per_sm(self._h, 1)),
                     stored_emission_bytes=int(self._lib.hfa_plan_stored_emission_bytes(self._h)))
 
     def algorithmic_bytes_fused(self, dtype: int = _lib.DTYPE_F32) -> int:
@@ -147,11 +149,11 @@ class AlignPlan:
 
     def debug_region(self, workspace: torch.Tensor, which: str) -> torch.Tensor:
         """Test helper: typed view of an intermediate workspace buffer."""
-        code = {"emis": 0, "edge2": 1, "edge_p": 2, "bp": 3}[which]
+        code = {"emis": 0, "edge2": 1, "edge_p": 2, "bp": 3, "xchg": 4}[which]
         nb = C.c_int64()
         off = int(self._lib.hfa_plan_debug_region(self._h, code, C.byref(nb)))
         raw = workspace[off:off + int(nb.value)]
-        if which == "bp":
+        if which in ("bp", "xchg"):
             return raw.view(torch.int32)
         v = raw.view(torch.float32)
         return v.view(-1, 2) if which == "edge2" else v

@@ -119,6 +119,10 @@ int hfa_plan_routing(const hfa_plan *plan, int32_t out[8]);
  * {SP, phoneme} pairs so that the advance out of an SP needs no f64 arithmetic; tools/alignment_decoder.py:182-187
  * with curr == 0 at :226-228).  Chosen per utterance at hfa_plan_create. */
 int32_t hfa_plan_pair_utterances(const hfa_plan *plan);
+/* Strips of the skewed-wavefront kernel resident per SM (4 or 5), chosen per plan from a list schedule of the strips
+ * of one forward list: list 0 = the small-batch list (hfa_plan_routing out[1]), 1 = the long-sequence list (out[3]).
+ * 0 when that list does not run in the skewed kernel. */
+int32_t hfa_plan_skew_ctas_per_sm(const hfa_plan *plan, int32_t list);
 /* Bytes of emissions hfa_emission stores for this plan.  For the utterances of the pair layout the rows are
  * compacted to one column per DISTINCT phoneme id (states with the same id have the same emission,
  * prob_log[t, ids[s]], tools/alignment_decoder.py:239): fewer than the 4 bytes per DP cell of SURVEY 8(d). */
@@ -219,7 +223,8 @@ int hfa_debug_unpack_emissions(const hfa_plan *plan, const void *workspace, floa
 
 /* byte offset of a workspace region (tests peek at intermediate buffers through this):
  * which = 0 emissions f32 [sum T*Sp] (Sp = S rounded up to 4), 1 edge pairs f32x2 (per utterance
- * padded to a multiple of 16 frames), 2 edge_pred f32 (same padding), 3 backpointer words.
+ * padded to a multiple of 16 frames), 2 edge_pred f32 (same padding), 3 backpointer words, 4 the strips' and
+ * bands' exchange table (all-zero between calls).
  * Returns -1 for an unknown region. */
 int64_t hfa_plan_debug_region(const hfa_plan *plan, int32_t which, int64_t *n_bytes);
 
