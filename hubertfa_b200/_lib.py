@@ -48,6 +48,7 @@ SYMBOLS = {
     "hfa_plan_routing": (C.c_int, [_vp, C.POINTER(_i32 * 8)]),
     "hfa_plan_pair_utterances": (_i32, [_vp]),
     "hfa_plan_skew_ctas_per_sm": (_i32, [_vp, _i32]),
+    "hfa_plan_bt_walk_utterances": (_i32, [_vp]),
     "hfa_plan_stored_emission_bytes": (_i64, [_vp]),
     "hfa_debug_unpack_emissions": (C.c_int, [_vp, _vp, _vp, _vp]),
     "hfa_plan_upload": (C.c_int, [_vp, _vp, _vp]),

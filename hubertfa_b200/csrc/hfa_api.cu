@@ -44,6 +44,8 @@ cudaError_t hfa_launch_ctc_greedy(const void *logits, int dtype, int T, int V, i
 cudaError_t hfa_launch_jump_tables(const HfaLaunchCtx &c, int n_blocks);
 cudaError_t hfa_launch_backtrace_tables(const HfaLaunchCtx &c, const int32_t *order, int n,
                                         const HfaResultPtrs &res, float *frame_conf, float *dp_path);
+cudaError_t hfa_launch_backtrace_walk(const HfaLaunchCtx &c, const int32_t *order, int n, int64_t smem,
+                                      const HfaResultPtrs &res, float *frame_conf, float *dp_path);
 
 namespace {
 
@@ -189,9 +191,13 @@ struct hfa_plan {
     // strips of the skewed kernel resident per SM (4 or 5: the kernel's ring has 6 or 5 stages)
     int32_t skew_ctas[2] = {5, 5};
     int64_t band_xchg_elems = 0, dp_store_elems = 0;
-    std::vector<int32_t> jblk_utt, jblk_first; // jump-table kernel: 256-word blocks per utterance
-    int32_t n_valid = 0, n_kept = 0;           // valid utterances / utterances that keep dp
+    std::vector<int32_t> jblk_utt, jblk_first; // jump-table kernel: 256-word blocks per utterance of the table set
+    int32_t n_kept = 0;                        // utterances that keep dp
     int32_t bt_begin = 0;
+    // the kept-dp utterances split into the walk set (backpointers staged in shared memory, hfa_backtrace_walk_kernel)
+    // and the table set (jump tables + hfa_backtrace_tables_kernel); both lists follow the backtrace list in `order`
+    int32_t walk_begin = 0, n_walk = 0, tab_begin = 0, n_tab = 0;
+    int64_t walk_smem = 0;                     // dynamic shared memory of the walk launch: its largest utterance
     std::vector<int32_t> row_blocks;           // [n+1]
     std::vector<int32_t> block_utt;            // [row_blocks[n]]
     int64_t total_frames = 0, total_states = 0, total_cells = 0, padded_cells = 0;
@@ -556,13 +562,35 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                                              p->band_skew[wh], 5LL * sm_count());
             p->skew_ctas[wh] = m4 <= m5 ? 4 : 5;
         }
-        // jump-table kernel (backtrace of the utterances that keep dp): one thread per backpointer word
-        p->n_valid = (int32_t)all.size();
-        for (const HfaUtt &m : p->utt) p->n_kept += (m.status == 0 && m.dp_off >= 0);
+        // Backtrace of the utterances that keep dp.  The walk stages an utterance's backpointer words in shared
+        // memory and walks them serially, one CTA per utterance; the jump tables make the serial part one lookup
+        // per 16 frames but cost a kernel that walks every word.  Measured (profiles/r5_bt_routes.jsonl, B200): the
+        // walk wins on every batch it fits, 256 utterances of T = 500-6000 and S = 40-256 up to 192 KB of words
+        // at one CTA per SM, so an utterance takes it whenever its words fit in one CTA's shared memory; giants
+        // (S > 8192) keep the tables.  HFA_BT_WALK = 0: never (tests compare the two routes).
+        int bt_walk = 2;
+        if (const char *e = std::getenv("HFA_BT_WALK")) bt_walk = std::atoi(e);
+        std::vector<int32_t> walk_list, tab_list;
+        std::vector<char> walks((size_t)n_utt, 0);
+        for (int32_t b : all) {
+            const HfaUtt &m = p->utt[b];
+            if (m.dp_off < 0) continue;
+            p->n_kept += 1;
+            const bool walk = bt_walk != 0 && m.S <= HFA_CTA_MAX_S &&
+                              hfa_bt_walk_smem(m.T, m.S, m.Sp) <= HFA_BT_WALK_SMEM_LIMIT;
+            (walk ? walk_list : tab_list).push_back(b);
+            if (walk) {
+                walks[(size_t)b] = 1;
+                p->walk_smem = std::max(p->walk_smem, hfa_bt_walk_smem(m.T, m.S, m.Sp));
+            }
+        }
+        p->n_walk = (int32_t)walk_list.size();
+        p->n_tab = (int32_t)tab_list.size();
+        // jump-table kernel (the table set): one thread per backpointer word
         p->jblk_first.assign((size_t)n_utt + 1, 0);
         for (int32_t b = 0; b < n_utt; ++b) {
             const HfaUtt &m = p->utt[b];
-            const int64_t w = (m.status == 0 && m.dp_off >= 0) ? (int64_t)((m.T + 15) / 16) * m.Sp : 0;
+            const int64_t w = (m.status == 0 && m.dp_off >= 0 && !walks[(size_t)b]) ? (int64_t)((m.T + 15) / 16) * m.Sp : 0;
             const int32_t nblk = (int32_t)((w + 255) / 256);
             p->jblk_first[b + 1] = p->jblk_first[b] + nblk;
             p->jblk_utt.insert(p->jblk_utt.end(), (size_t)nblk, b);
@@ -652,6 +680,10 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         p->bt_begin = (int32_t)p->order.size();
         p->order.insert(p->order.end(), all.begin(), all.end());
         p->order.insert(p->order.end(), invalid.begin(), invalid.end());
+        p->walk_begin = (int32_t)p->order.size();
+        p->order.insert(p->order.end(), walk_list.begin(), walk_list.end());
+        p->tab_begin = (int32_t)p->order.size();
+        p->order.insert(p->order.end(), tab_list.begin(), tab_list.end());
 
         // workspace layout
         int64_t o = 0;
@@ -681,7 +713,7 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         p->o_last = region((int64_t)n_utt * 8);
         p->o_emode = region(p->n_compact > 0 ? (int64_t)n_utt * 4 : 0);
         p->o_dpst = region(p->dp_store_elems * 4);
-        const bool jump_tables = p->dp_store_elems > 0;      // latency plans: parallel backtrace
+        const bool jump_tables = p->n_tab > 0;              // kept-dp utterances the walk does not take
         p->o_jump = region(jump_tables ? words : 0);
         p->o_moves = region(jump_tables ? words : 0);
         p->o_rowent = region(jump_tables ? edge / 16 * 4 : 0);
@@ -789,6 +821,7 @@ int hfa_plan_routing(const hfa_plan *p, int32_t out[8])
 }
 
 int32_t hfa_plan_pair_utterances(const hfa_plan *p) { return p ? p->pair_count : 0; }
+int32_t hfa_plan_bt_walk_utterances(const hfa_plan *p) { return p ? p->n_walk : 0; }
 int32_t hfa_plan_skew_ctas_per_sm(const hfa_plan *p, int32_t list)
 {
     if (!p || list < 0 || list > 1) return 0;
@@ -1053,16 +1086,23 @@ int hfa_backtrace(const hfa_plan *p, void *workspace, void *result, float *frame
     if (p->n_utt == 0) return HFA_OK;
     HfaLaunchCtx c = make_ctx(p, workspace, stream);
     const HfaResultPtrs r = make_res(p, result);
-    if (!p->jblk_utt.empty()) {
-        // utterances whose forward pass kept dp (latency plans): jump tables (parallel), then one CTA
-        // per utterance; the warp-per-utterance kernel below skips them (and they skip the others)
+    // utterances whose forward pass kept dp (latency plans): one CTA per utterance, the walk set straight from
+    // its staged backpointers, the table set after the jump tables; the warp-per-utterance kernel below skips
+    // them (and they skip the others)
+    if (p->n_walk > 0) {
+        cudaError_t ew = hfa_launch_backtrace_walk(c, c.ws.order + p->walk_begin, p->n_walk, p->walk_smem, r,
+                                                   frame_conf, dp_path);
+        if (ew != cudaSuccess) return cuda_fail(ew, "hfa_backtrace: walk kernel");
+        g_launches += 1;
+    }
+    if (p->n_tab > 0) {
         cudaError_t ej = hfa_launch_jump_tables(c, (int)p->jblk_utt.size());
         if (ej == cudaSuccess)
-            ej = hfa_launch_backtrace_tables(c, c.ws.order + p->bt_begin, p->n_valid, r, frame_conf, dp_path);
+            ej = hfa_launch_backtrace_tables(c, c.ws.order + p->tab_begin, p->n_tab, r, frame_conf, dp_path);
         if (ej != cudaSuccess) return cuda_fail(ej, "hfa_backtrace: table kernels");
         g_launches += 2;
-        if (p->n_kept == p->n_utt) return HFA_OK;           // nothing left for the warp kernel
     }
+    if (p->n_kept > 0 && p->n_kept == p->n_utt) return HFA_OK;   // nothing left for the warp kernel
     cudaError_t e = hfa_launch_backtrace(c, c.ws.order + p->bt_begin, p->n_utt, r, frame_conf,
                                          dp_path);
     if (e != cudaSuccess) return cuda_fail(e, "hfa_backtrace: launch");

@@ -99,7 +99,7 @@ hfa_backtrace_kernel(HfaWs ws, const int32_t *__restrict__ order, int n, HfaResu
         }
         return;
     }
-    if (m.dp_off >= 0) return;                 // kept dp + jump tables: hfa_backtrace_tables_kernel
+    if (m.dp_off >= 0) return;                 // kept dp: hfa_backtrace_walk_kernel / hfa_backtrace_tables_kernel
     const int T = m.T, S = m.S, Sp = m.Sp;
     const int32_t *ids = ws.ids + m.seg_off;
     const uint32_t *bp = ws.bp + m.bp_off;
@@ -374,6 +374,55 @@ hfa_backtrace_kernel(HfaWs ws, const int32_t *__restrict__ order, int n, HfaResu
 //   2  (thread = frame)  frame confidence, log-sum;   3 (thread = segment)  seconds.
 // ---------------------------------------------------------------------------------------------
 #define HFA_BTT_THREADS 256
+#define HFA_BTW_CHUNKS 8         // bulk copies (and mbarriers) the walk kernel stages an utterance's words in
+
+// Phases 2 and 3 of the kept-dp backtraces, for a CTA of HFA_BTT_THREADS threads: frame confidence, log-sum and
+// total confidence from dp[t, s_t] (dp_at(t)), segment seconds from the segment frames in forward order
+// (seg_t(k)), then the utterance's scalar results.  Both kernels call this, so their results are the same bits.
+template <typename FDp, typename FSegT>
+__device__ __forceinline__ void hfa_bt_finish(const HfaUtt &m, int u, int n_seg, int s_end, float final_score,
+                                              const float *p, const HfaResultPtrs &res, float *frame_conf,
+                                              float *dp_path, double frame_length, double *warp_log, FDp dp_at,
+                                              FSegT seg_t)
+{
+    constexpr int NW = HFA_BTT_THREADS / 32;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int T = m.T;
+
+    // ---- 2: frame confidence (:284-288), total confidence (:97) ----
+    double log_sum = 0.0;
+    for (int t = tid; t < T; t += HFA_BTT_THREADS) {
+        const float cur = dp_at(t);
+        const float prev = (t > 0) ? dp_at(t - 1) : 0.0f;          // dp_path[-1] := 0 (:286)
+        const float fc = expf(__fsub_rn(cur, prev));
+        if (frame_conf != nullptr) frame_conf[m.frame_off + t] = fc;
+        if (dp_path != nullptr) dp_path[m.frame_off + t] = cur;
+        log_sum += (double)logf(__fadd_rn(fc, 1e-6f));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) log_sum += __shfl_xor_sync(0xffffffffu, log_sum, o);
+    if (lane == 0) warp_log[warp] = log_sum;
+
+    // ---- 3: segments -> seconds ----
+    double *out_iv = res.intervals + 2 * m.seg_off;
+    for (int k = tid; k < n_seg; k += HFA_BTT_THREADS) {
+        out_iv[2 * k] = seg_time(p, seg_t(k), T, frame_length);
+        out_iv[2 * k + 1] = (k + 1 < n_seg) ? seg_time(p, seg_t(k + 1), T, frame_length)
+                                            : __dmul_rn(frame_length, (double)T);
+    }
+    __syncthreads();
+    if (tid == 0) {
+        double tot = 0.0;
+        for (int q = 0; q < NW; ++q) tot += warp_log[q];
+        const float mean = (float)(tot / (double)T);
+        res.status[u] = (final_score == HFA_NEG_INF) ? 4 : 0;
+        res.n_seg[u] = n_seg;
+        res.end_state[u] = s_end;
+        res.final_score[u] = final_score;
+        res.total_conf[u] = expf(__fdiv_rn(mean, 3.0f));
+    }
+}
+
 
 __global__ void __launch_bounds__(HFA_BTT_THREADS)
 hfa_backtrace_tables_kernel(HfaWs ws, const int32_t *__restrict__ order, int n, HfaResultPtrs res,
@@ -488,40 +537,122 @@ hfa_backtrace_tables_kernel(HfaWs ws, const int32_t *__restrict__ order, int n, 
         __syncthreads();
     }
     const int n_seg = min(carry_sm, S);
+    hfa_bt_finish(m, u, n_seg, s_end, final_score, ws.edge_p + m.edge_off, res, frame_conf, dp_path, frame_length,
+                  warp_log, [&](int t) { return __int_as_float(path_state[t]); }, [&](int k) { return out_t[k]; });
+}
 
-    // ---- 2: frame confidence (:284-288), total confidence (:97) ----
-    double log_sum = 0.0;
-    for (int t = tid; t < T; t += HFA_BTT_THREADS) {
-        const float cur = __int_as_float(path_state[t]);
-        const float prev = (t > 0) ? __int_as_float(path_state[t - 1]) : 0.0f;   // dp_path[-1] := 0 (:286)
-        const float fc = expf(__fsub_rn(cur, prev));
-        if (frame_conf != nullptr) frame_conf[m.frame_off + t] = fc;
-        if (dp_path != nullptr) dp_path[m.frame_off + t] = cur;
-        log_sum += (double)logf(__fadd_rn(fc, 1e-6f));
+// ---------------------------------------------------------------------------------------------
+// Backtrace of the kept-dp utterances whose backpointers fit in shared memory: ONE CTA per utterance,
+// no jump tables.  The utterance's ceil(T/16) x Sp backpointer words are staged by bulk copies, last
+// rows first (one mbarrier per chunk of rows), and warp 0 walks the path from move to move straight out
+// of shared memory (hfa_walk_row: one LDS + clz per move, one per row without a move), all 32 lanes in
+// lock step: lane f writes the state of frame f of the row.  Then every thread gathers dp[t, s_t] of its
+// frames and hfa_bt_finish does the rest exactly as in the table backtrace.
+// Dynamic shared memory (hfa_bt_walk_smem): [n_rows][Sp] words, [16 n_rows] frame state -> dp bits,
+// [S] segment states and [S] segment frames in backward order.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(HFA_BTT_THREADS)
+hfa_backtrace_walk_kernel(HfaWs ws, const int32_t *__restrict__ order, HfaResultPtrs res,
+                          float *__restrict__ frame_conf, float *__restrict__ dp_path, double frame_length)
+{
+    constexpr int NW = HFA_BTT_THREADS / 32;
+    extern __shared__ __align__(16) unsigned char walk_sm[];
+    __shared__ __align__(8) uint64_t bars[HFA_BTW_CHUNKS];
+    __shared__ double warp_log[NW];
+    __shared__ int n_seg_sm;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int u = order[blockIdx.x];
+    const HfaUtt m = ws.utt[u];                  // the planner sends valid utterances with kept dp only
+    const int T = m.T, S = m.S, Sp = m.Sp;
+    const int n_rows = (T + 15) >> 4;
+    const uint32_t *words = reinterpret_cast<const uint32_t *>(walk_sm);
+    int32_t *fr = reinterpret_cast<int32_t *>(walk_sm + (size_t)n_rows * Sp * 4);
+    int32_t *rev_idx = fr + 16 * n_rows;
+    int32_t *rev_t = rev_idx + S;
+    const int rows_per = (n_rows + HFA_BTW_CHUNKS - 1) / HFA_BTW_CHUNKS;
+    const uint32_t bar0 = hfa_smem_u32(bars);
+
+    if (tid == 0) {
+        for (int c = 0; c < HFA_BTW_CHUNKS; ++c) hfa_mbar_init(bar0 + 8 * c, 1);
+        hfa_fence_mbar_init();
+        // chunk c = rows [hi - rows_per, hi), hi = n_rows - c rows_per: the walk needs the last rows first
+        for (int c = 0; c * rows_per < n_rows; ++c) {
+            const int hi = n_rows - c * rows_per, lo = max(hi - rows_per, 0);
+            const uint32_t bytes = (uint32_t)(hi - lo) * Sp * 4;
+            hfa_mbar_expect_tx(bar0 + 8 * c, bytes);
+            hfa_bulk_load(hfa_smem_u32(words) + (uint32_t)lo * Sp * 4, ws.bp + m.bp_off + (int64_t)lo * Sp, bytes,
+                          bar0 + 8 * c);
+        }
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) log_sum += __shfl_xor_sync(0xffffffffu, log_sum, o);
-    if (lane == 0) warp_log[warp] = log_sum;
 
-    // ---- 3: segments -> seconds ----
-    const float *p = ws.edge_p + m.edge_off;
-    double *out_iv = res.intervals + 2 * m.seg_off;
-    for (int k = tid; k < n_seg; k += HFA_BTT_THREADS) {
-        out_iv[2 * k] = seg_time(p, out_t[k], T, frame_length);
-        out_iv[2 * k + 1] = (k + 1 < n_seg) ? seg_time(p, out_t[k + 1], T, frame_length)
-                                            : __dmul_rn(frame_length, (double)T);
+    // ---- end state (:269-272) ----
+    const int32_t *ids = ws.ids + m.seg_off;
+    const float last1 = ws.dp_last[2 * u];
+    const float last2 = (S >= 2) ? ws.dp_last[2 * u + 1] : HFA_NEG_INF;
+    int s_end = S - 1;
+    float final_score = last1;
+    if (S >= 2 && last2 > last1 && ids[S - 1] == 0) {
+        s_end = S - 2;
+        final_score = last2;
+    }
+    __syncthreads();                             // the barriers are initialised
+
+    // ---- 1: the walk (warp 0) ----
+    if (warp == 0) {
+        int cur = s_end, n_seg = 0, c = 0;
+        hfa_mbar_wait(bar0, 0, HFA_POLLS_COPY);
+        for (int w = n_rows - 1; w >= 0; --w) {
+            if (w < n_rows - (c + 1) * rows_per) {
+                ++c;
+                hfa_mbar_wait(bar0 + 8 * c, 0, HFA_POLLS_COPY);
+            }
+            const int tt = (w == n_rows - 1) ? ((T - 1) & 15) : 15;
+            cur = hfa_walk_row(words + (size_t)w * Sp, cur, tt, w == 0,
+                               [&](int st, int f) {
+                                   if (lane == 0 && n_seg < S) {
+                                       rev_idx[n_seg] = st;
+                                       rev_t[n_seg] = 16 * w + f;
+                                   }
+                                   ++n_seg;
+                               },
+                               [&](int st, int f_lo, int f_hi) {
+                                   if (lane >= f_lo && lane <= f_hi) fr[16 * w + lane] = st;
+                               });
+        }
+        if (lane == 0) n_seg_sm = min(n_seg, S);   // n_seg > S cannot happen with valid backpointers
     }
     __syncthreads();
-    if (tid == 0) {
-        double tot = 0.0;
-        for (int q = 0; q < NW; ++q) tot += warp_log[q];
-        const float mean = (float)(tot / (double)T);
-        res.status[u] = (final_score == HFA_NEG_INF) ? 4 : 0;
-        res.n_seg[u] = n_seg;
-        res.end_state[u] = s_end;
-        res.final_score[u] = final_score;
-        res.total_conf[u] = expf(__fdiv_rn(mean, 3.0f));
+    const int n_seg = n_seg_sm;
+
+    // ---- dp[t, s_t] in place of s_t, segments in forward order ----
+    const float *dps = ws.dp_store + m.dp_off;
+    constexpr int G = 8;                         // independent gathers in flight per thread
+    for (int base = 0; base < T; base += G * HFA_BTT_THREADS) {
+        float dv[G];
+#pragma unroll
+        for (int j = 0; j < G; ++j) {
+            const int t = min(base + j * HFA_BTT_THREADS + tid, T - 1);
+            const int st = fr[t];
+            dv[j] = hfa_ldg_f32_64B(dps + (m.skew_d > 0 ? hfa_skew_dp_index(m.skew_d, T, t, st)
+                                                        : hfa_dp_store_index(m.band_k, T, t, st)));
+        }
+        __syncthreads();                         // every state of this batch is read before any is replaced
+#pragma unroll
+        for (int j = 0; j < G; ++j) {
+            const int t = base + j * HFA_BTT_THREADS + tid;
+            if (t < T) fr[t] = __float_as_int(dv[j]);
+        }
     }
+    int32_t *out_idx = res.ph_idx_seq + m.seg_off;
+    int32_t *out_t = res.ph_time_int + m.seg_off;
+    for (int k = tid; k < n_seg; k += HFA_BTT_THREADS) {
+        out_idx[k] = rev_idx[n_seg - 1 - k];
+        out_t[k] = rev_t[n_seg - 1 - k];
+    }
+    __syncthreads();
+    hfa_bt_finish(m, u, n_seg, s_end, final_score, ws.edge_p + m.edge_off, res, frame_conf, dp_path, frame_length,
+                  warp_log, [&](int t) { return __int_as_float(fr[t]); },
+                  [&](int k) { return rev_t[n_seg - 1 - k]; });
 }
 
 // test helper: unpack one utterance's backpointers to int8 [T][S] (row 0 = -1, :247)
@@ -584,6 +715,18 @@ cudaError_t hfa_launch_backtrace_tables(const HfaLaunchCtx &c, const int32_t *or
     if (n <= 0) return cudaSuccess;
     hfa_backtrace_tables_kernel<<<n, HFA_BTT_THREADS, 0, c.stream>>>(c.ws, order, n, res, frame_conf, dp_path,
                                                                     c.frame_length);
+    return cudaGetLastError();
+}
+
+cudaError_t hfa_launch_backtrace_walk(const HfaLaunchCtx &c, const int32_t *order, int n, int64_t smem,
+                                      const HfaResultPtrs &res, float *frame_conf, float *dp_path)
+{
+    if (n <= 0) return cudaSuccess;
+    cudaError_t e = cudaFuncSetAttribute(hfa_backtrace_walk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem);
+    if (e != cudaSuccess) return e;
+    hfa_backtrace_walk_kernel<<<n, HFA_BTT_THREADS, (size_t)smem, c.stream>>>(c.ws, order, res, frame_conf, dp_path,
+                                                                             c.frame_length);
     return cudaGetLastError();
 }
 

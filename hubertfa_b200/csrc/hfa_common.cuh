@@ -136,6 +136,15 @@ __host__ __device__ __forceinline__ int64_t hfa_skew_dp_index(int D, int T, int 
     return ((int64_t)w * hfa_skew_blocks(D, T) * HFA_SKEW_BLK + t + p * D) * 32 + p;
 }
 
+// Shared memory of the walk backtrace (hfa_backtrace_walk_kernel) for one utterance: its ceil(T/16) x Sp
+// backpointer words, 16 frames of state / dp per word row, and S segment states + S segment frames.
+__host__ __device__ __forceinline__ int64_t hfa_bt_walk_smem(int T, int S, int Sp)
+{
+    const int64_t rows = (T + 15) / 16;
+    return rows * Sp * 4 + rows * 64 + ((int64_t)S * 8 + 15) / 16 * 16;
+}
+#define HFA_BT_WALK_SMEM_LIMIT (227 * 1024 - 1024)   // dynamic shared memory of one CTA, less the static part
+
 // ---------------------------------------------------------------------------------------------
 // PTX primitives.  Shared memory is addressed through 32-bit shared::cta window addresses: a generic
 // pointer costs an S2UR + ULEA at every use on sm_100, so a kernel converts once (hfa_smem_u32) and

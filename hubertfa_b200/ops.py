@@ -75,6 +75,7 @@ class AlignPlan:
                     pair_utts=int(self._lib.hfa_plan_pair_utterances(self._h)),
                     skew_ctas_per_sm=int(self._lib.hfa_plan_skew_ctas_per_sm(self._h, 0)),
                     big_skew_ctas_per_sm=int(self._lib.hfa_plan_skew_ctas_per_sm(self._h, 1)),
+                    bt_walk_utts=int(self._lib.hfa_plan_bt_walk_utterances(self._h)),
                     stored_emission_bytes=int(self._lib.hfa_plan_stored_emission_bytes(self._h)))
 
     def algorithmic_bytes_fused(self, dtype: int = _lib.DTYPE_F32) -> int:

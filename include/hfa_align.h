@@ -123,6 +123,10 @@ int32_t hfa_plan_pair_utterances(const hfa_plan *plan);
  * of one forward list: list 0 = the small-batch list (hfa_plan_routing out[1]), 1 = the long-sequence list (out[3]).
  * 0 when that list does not run in the skewed kernel. */
 int32_t hfa_plan_skew_ctas_per_sm(const hfa_plan *plan, int32_t list);
+/* How many of the utterances that keep dp (out[6]) are backtraced by walking their backpointers out of shared
+ * memory instead of through jump tables: those whose backpointer words fit in one CTA's shared memory, giants
+ * (S > HFA_CTA_MAX_S) excepted.  HFA_BT_WALK=0 routes none there. */
+int32_t hfa_plan_bt_walk_utterances(const hfa_plan *plan);
 /* Bytes of emissions hfa_emission stores for this plan.  For the utterances of the pair layout the rows are
  * compacted to one column per DISTINCT phoneme id (states with the same id have the same emission,
  * prob_log[t, ids[s]], tools/alignment_decoder.py:239): fewer than the 4 bytes per DP cell of SURVEY 8(d). */
