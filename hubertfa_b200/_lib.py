@@ -65,6 +65,8 @@ SYMBOLS = {
     "hfa_debug_unpack_backptr": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "hfa_debug_unpack_dp": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "hfa_ctc_greedy": (C.c_int, [_vp, _i32, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
+    "hfa_ctc_greedy_batch": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
+    "hfa_frame_states": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
 }
 
 _lib = None

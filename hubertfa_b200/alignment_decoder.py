@@ -40,16 +40,42 @@ def _as_1d(edge: torch.Tensor) -> torch.Tensor:
     return edge
 
 
+def _masked_logits(frame_logits: torch.Tensor, ph_seq_id, vocab_size: int) -> torch.Tensor:
+    """ad:53-59: the frame logits with every phoneme outside the sequence (SP excepted) pushed down by 1e9."""
+    drop = np.ones(vocab_size, dtype=bool)
+    drop[ph_seq_id] = False
+    drop[0] = False
+    pen = torch.from_numpy(drop).to(frame_logits.device)[None, None, :] * 1e9
+    return frame_logits.float() - pen.float()
+
+
+def _ph_frame_pred(frame_logits: torch.Tensor, ph_seq_id, vocab_size: int) -> np.ndarray:
+    """ad:56-59,73: softmax of the masked [1,T,V] logits -> f32 [T, V]."""
+    return torch.nn.functional.softmax(_masked_logits(frame_logits, ph_seq_id, vocab_size), dim=-1
+                                       ).squeeze(0).cpu().numpy().astype("float32")
+
+
+def _edge_prob(edge_logits: torch.Tensor) -> np.ndarray:
+    """ad:68-71,84: the edge probability of the [1,T] edge logits, spread onto the frame after it."""
+    p = (((torch.sigmoid(edge_logits.float()) - 0.1) / 0.8).clamp(0.0, 1.0)).squeeze(0).cpu().numpy().astype("float32")
+    return (p + np.concatenate(([0], p[:-1]))).clip(0, 1)
+
+
 class BatchAlignment:
     """Result of :meth:`AlignmentDecoder.decode_batch` (host resident, numeric part vectorised).
 
     Ragged arrays are indexed by ``seg_off`` (raw segments, capacity S per utterance),
     ``ph_off`` (phonemes kept after the SP filter, ad:123) and ``word_off`` (merged words, ad:128).
     ``result[b]`` gives utterance ``b`` as the reference's 5-tuple.
+
+    What ``validation_step`` reads after ``decode()`` (forced_alignment.py:407-414) is here per utterance too:
+    ``ctc(b)`` (with ``ctc_logits``), ``ph_idx_frame(b)`` (``frame_state``, with ``want_frame_states``),
+    ``ph_frame_pred(b)`` / ``edge_prob(b)`` (computed on demand, like the decoder's attributes) and
+    ``plot(b, melspec)``.
     """
 
     def __init__(self, plan: ops.AlignPlan, views: dict, ph_seqs, word_seqs, ph2word, is_sp, word_idx,
-                 frame_conf=None):
+                 frame_conf=None, ctc=None, frame_state=None, inputs=None):
         self.n_utt = plan.n_utt
         self.T = plan.T
         self.S = plan.S
@@ -64,6 +90,14 @@ class BatchAlignment:
         self.ph_time_int = views["ph_time_int"]
         self.raw_intervals = views["intervals"]
         self.frame_confidence = frame_conf
+        # ctc(): ids of utterance b at ctc_ids[frame_off[b] : frame_off[b] + ctc_len[b]]
+        self.ctc_ids, self.ctc_len = ctc if ctc is not None else (None, None)
+        self.frame_state = frame_state            # int32 [sum T]: state index of the best path at every frame
+        self.frame_length = plan.frame_length
+        self.vocab_size = plan.vocab_size
+        # (frame logits, edge logits, ph_seq_id) per utterance, trimmed, on the device: for ph_frame_pred / edge_prob.
+        # Kept only for validation batches (ctc_logits / want_frame_states): they hold the logits alive.
+        self._inputs = inputs
         self._ph_seqs, self._word_seqs, self._ph2word = ph_seqs, word_seqs, ph2word
         self._filter_and_merge(is_sp, word_idx)
 
@@ -109,10 +143,13 @@ class BatchAlignment:
         return (self.ph_idx_seq[o:o + k].astype(np.int64), self.ph_time_int[o:o + k].astype(np.int64),
                 self.raw_intervals[o:o + k])
 
-    def __getitem__(self, b: int):
-        """Utterance b as the reference's 5-tuple (ad:143)."""
+    def _require_aligned(self, b: int) -> None:
         if self.status[b] not in (_lib.UTT_OK, _lib.UTT_INFEASIBLE):
             raise HfaError(f"utterance {b} was not aligned (status {int(self.status[b])})")
+
+    def __getitem__(self, b: int):
+        """Utterance b as the reference's 5-tuple (ad:143)."""
+        self._require_aligned(b)
         ph_seq, word_seq = self._ph_seqs[b], self._word_seqs[b]
         p0, p1 = int(self.ph_off[b]), int(self.ph_off[b + 1])
         w0, w1 = int(self.word_off[b]), int(self.word_off[b + 1])
@@ -121,6 +158,51 @@ class BatchAlignment:
         ph_iv = self.ph_intervals[p0:p1] if p1 > p0 else np.array([]).clip(min=0)
         word_iv = self.word_intervals[w0:w1] if w1 > w0 else np.array([]).clip(min=0)
         return ph_pred, ph_iv, word_pred, word_iv, np.float32(self.total_confidence[b])
+
+    def ctc(self, b: int) -> np.ndarray:
+        """Greedy CTC ids of utterance b, int64: what ``decode(); ctc()`` returns (ad:145-150)."""
+        self._require_aligned(b)
+        if self.ctc_ids is None:
+            raise HfaError("ctc() needs decode_batch(..., ctc_logits=...)")
+        f0 = int(self.frame_off[b])
+        return self.ctc_ids[f0:f0 + int(self.ctc_len[b])].astype(np.int64)
+
+    def ph_idx_frame(self, b: int) -> np.ndarray:
+        """State index of the best path at every frame of utterance b: the ph_idx_frame plot() builds
+        (ad:156-161)."""
+        self._require_aligned(b)
+        if self.frame_state is None:
+            raise HfaError("ph_idx_frame() needs decode_batch(..., want_frame_states=True)")
+        return self.frame_state[int(self.frame_off[b]):int(self.frame_off[b + 1])].astype(np.int64)
+
+    def _inputs_of(self, b: int):
+        self._require_aligned(b)
+        if self._inputs is None:
+            raise HfaError("the logits are kept for decode_batch(..., ctc_logits=... or want_frame_states=True) only")
+        return self._inputs[b]
+
+    def ph_frame_pred(self, b: int) -> np.ndarray:
+        """f32 [T, V] masked softmax of utterance b's frame logits (the decoder's ``ph_frame_pred``, ad:73)."""
+        frame, _, ids = self._inputs_of(b)
+        return _ph_frame_pred(frame[None], ids, self.vocab_size)
+
+    def edge_prob(self, b: int) -> np.ndarray:
+        """f32 [T] edge probability of utterance b (the decoder's ``edge_prob``, ad:84)."""
+        return _edge_prob(self._inputs_of(b)[1][None])
+
+    def plot(self, b: int, melspec):
+        """ad:152-168 for utterance b: plot_for_valid with the arguments ``decode(); plot()`` passes.  Needs
+        ``want_frame_confidence`` and ``want_frame_states``, and the reference's ``tools.plot`` on the path."""
+        from tools.plot import plot_for_valid  # provided by the reference checkout
+
+        ph_pred, ph_iv = self[b][:2]
+        if self.frame_confidence is None:
+            raise HfaError("plot() needs decode_batch(..., want_frame_confidence=True)")
+        f0, f1 = int(self.frame_off[b]), int(self.frame_off[b + 1])
+        ids = self._inputs_of(b)[2]
+        return plot_for_valid(melspec.cpu().numpy(), ph_pred, (ph_iv / self.frame_length).round().astype("int32"),
+                              self.frame_confidence[f0:f1].copy(), self.ph_frame_pred(b)[:, ids],
+                              self.ph_idx_frame(b), self.edge_prob(b))
 
 
 class AlignmentDecoder:
@@ -176,8 +258,10 @@ class AlignmentDecoder:
         n = int((wav_length * self.melspec_config["sample_rate"] + 0.5) / self.melspec_config["hop_length"])
         return min(T, n) if n >= 0 else max(T + n, 0)      # python slice semantics of ad:48
 
-    def _run(self, frames, edges, ids_list, want_frame_conf: bool):
-        """frames/edges: per-utterance 2-D / 1-D CUDA tensors (views allowed, already trimmed)."""
+    def _run(self, frames, edges, ids_list, want_frame_conf: bool, ctcs=None, want_states: bool = False):
+        """frames/edges: per-utterance 2-D / 1-D CUDA tensors (views allowed, already trimmed).  ctcs: None or
+        per-utterance 2-D ctc logits (one dtype and width, T rows each) for hfa_ctc_greedy_batch; want_states:
+        hfa_frame_states after the alignment.  Both run on the same stream, before the one synchronise."""
         dev = frames[0].device
         dtype = frames[0].dtype
         if dtype not in ops.TORCH_TO_DTYPE:
@@ -214,19 +298,46 @@ class AlignmentDecoder:
             else:
                 _lib.check(lib.hfa_align_batch(h, wp, ops.TORCH_TO_DTYPE[dtype], res.data_ptr(),
                                                fc.data_ptr() if fc is not None else None, sp), "hfa_align_batch")
+            nf = max(plan.total_frames, 1)
+            extra = {}                     # device outputs of the validation kernels -> pinned host copies
+            if ctcs is not None:
+                ctab = torch.from_numpy(plan.ctc_table(
+                    np.fromiter((c.data_ptr() for c in ctcs), dtype=np.int64, count=n),
+                    np.fromiter((c.stride(0) for c in ctcs), dtype=np.int64, count=n),
+                    np.fromiter((c.stride(1) for c in ctcs), dtype=np.int64, count=n))).to(dev)
+                ids_d = torch.empty(nf, dtype=torch.int32, device=dev)
+                len_d = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+                scratch = torch.empty(nf, dtype=torch.int32, device=dev)
+                Vc = int(ctcs[0].shape[1]) if n else 1
+                _lib.check(lib.hfa_ctc_greedy_batch(h, wp, ctab.data_ptr(), Vc, ops.TORCH_TO_DTYPE[ctcs[0].dtype],
+                                                    scratch.data_ptr(), ids_d.data_ptr(), len_d.data_ptr(), sp),
+                           "hfa_ctc_greedy_batch")
+                extra["ctc_ids"], extra["ctc_len"] = ids_d, len_d
+            if want_states:
+                st_d = torch.empty(nf, dtype=torch.int32, device=dev)
+                _lib.check(lib.hfa_frame_states(h, wp, res.data_ptr(), st_d.data_ptr(), sp), "hfa_frame_states")
+                extra["states"] = st_d
             host = self._pinned("res", plan.result_bytes, torch.uint8)
             host.copy_(res, non_blocking=True)
             fc_host = None
             if fc is not None:
                 fc_host = self._pinned("fc", fc.numel(), torch.float32)
                 fc_host.copy_(fc, non_blocking=True)
+            for k, d in extra.items():
+                extra[k] = self._pinned(k, d.numel(), d.dtype)
+                extra[k].copy_(d, non_blocking=True)
             stream.synchronize()
         # the pinned buffers are reused by the next call: hand out copies
         host = host.numpy().copy()
         if fc_host is not None:
             fc_host = fc_host.numpy().copy()
         views = plan.views(host)
-        return plan, views, (fc_host[:plan.total_frames] if fc_host is not None else None), ws
+        out = dict(frame_conf=fc_host[:plan.total_frames] if fc_host is not None else None)
+        if ctcs is not None:
+            out["ctc"] = (extra["ctc_ids"].numpy()[:plan.total_frames].copy(), extra["ctc_len"].numpy()[:n].copy())
+        if want_states:
+            out["frame_state"] = extra["states"].numpy()[:plan.total_frames].copy()
+        return plan, views, out, ws
 
     def _pinned(self, key: str, numel: int, dtype) -> torch.Tensor:
         cache = self.__dict__.setdefault("_pin_cache", {})
@@ -266,7 +377,8 @@ class AlignmentDecoder:
         if T < 1 or len(ph_seq_id) < 1:
             raise IndexError("index 0 is out of bounds for axis 0 with size 0")    # ad:250
 
-        plan, v, fc, _ = self._run([frame], [edge], [ph_seq_id.astype(np.int32)], True)
+        plan, v, out, _ = self._run([frame], [edge], [ph_seq_id.astype(np.int32)], True)
+        fc = out["frame_conf"]
         if v["status"][0] not in (_lib.UTT_OK, _lib.UTT_INFEASIBLE):
             raise HfaError(f"alignment failed with status {int(v['status'][0])}")
         k = int(v["n_seg"][0])
@@ -300,12 +412,19 @@ class AlignmentDecoder:
     # ----------------------------------------------------------------------------------------
     def decode_batch(self, ph_frame_logits, ph_edge_logits, ph_seqs: Sequence[Sequence[str]],
                      word_seqs=None, ph_idx_to_word_idxs=None, wav_lengths=None, lengths=None,
-                     want_frame_confidence: bool = False) -> BatchAlignment:
+                     want_frame_confidence: bool = False, ctc_logits=None,
+                     want_frame_states: bool = False) -> BatchAlignment:
         """Aligns a ragged batch in one pass.
 
         ph_frame_logits / ph_edge_logits: either lists of per-utterance tensors ([1,T,V] / [1,T], the
         shapes ``decode`` takes, strided views allowed), or one packed tensor [sum T, V] / [sum T]
         with ``lengths`` giving T per utterance.  Host tensors are copied to the device first.
+
+        For validation (what ``decode(); ctc(); plot()`` give per utterance): ``ctc_logits`` in the same form
+        as the frame logits (one width for the batch) is decoded greedily for every utterance in one launch,
+        ``want_frame_states`` expands the best paths into per-frame state indices in one more; both run on the
+        alignment's stream and come back with its single synchronise.  See ``BatchAlignment.ctc`` /
+        ``ph_idx_frame`` / ``plot``.
         """
         n = len(ph_seqs)
         ids_list = [self._ids_of(seq).astype(np.int32) for seq in ph_seqs]        # same checks as decode()
@@ -318,10 +437,17 @@ class AlignmentDecoder:
             offs = np.concatenate([[0], np.cumsum(np.asarray(lengths, dtype=np.int64))])
             frames = [fcat[offs[b]:offs[b + 1]] for b in range(n)]
             edges = [ecat[offs[b]:offs[b + 1]] for b in range(n)]
+            if ctc_logits is not None:
+                ccat = ctc_logits.to(dev, non_blocking=True)
+                ctcs = [ccat[offs[b]:offs[b + 1]] for b in range(n)]
         else:
             dev = self._device_for(ph_frame_logits[0])
             frames = [_as_2d(f).to(dev, non_blocking=True) for f in ph_frame_logits]
             edges = [_as_1d(e).to(dev, non_blocking=True) for e in ph_edge_logits]
+            if ctc_logits is not None:
+                if len(ctc_logits) != n:
+                    raise ValueError("ctc_logits must hold one tensor per utterance")
+                ctcs = [_as_2d(c).to(dev, non_blocking=True) for c in ctc_logits]
         # the reference applies .float() to both streams (ad:57,69): one element type per batch
         dt0 = frames[0].dtype if n else torch.float32
         if any(f.dtype != dt0 for f in frames) or dt0 not in ops.TORCH_TO_DTYPE:
@@ -332,6 +458,21 @@ class AlignmentDecoder:
             for b in range(n):
                 nf = self._num_frames(wav_lengths[b], frames[b].shape[0])
                 frames[b], edges[b] = frames[b][:nf], edges[b][:nf]
+                if ctc_logits is not None:                                       # ad:50
+                    ctcs[b] = ctcs[b][:self._num_frames(wav_lengths[b], ctcs[b].shape[0])]
+        if ctc_logits is None:
+            ctcs = None
+        elif n:
+            # one element type and one width per batch; ctc() decodes the frames decode() aligns
+            for b in range(n):
+                if ctcs[b].shape[0] != frames[b].shape[0]:
+                    raise ValueError(f"utterance {b}: {ctcs[b].shape[0]} frames of ctc logits, "
+                                     f"{frames[b].shape[0]} of frame logits")
+                if ctcs[b].shape[1] != ctcs[0].shape[1]:
+                    raise ValueError("the ctc logits of a batch must share one width")
+            ct = ctcs[0].dtype
+            if any(c.dtype != ct for c in ctcs) or ct not in ops.TORCH_TO_DTYPE:
+                ctcs = [c.float() for c in ctcs]
         if word_seqs is None:
             word_seqs = ph_seqs
             ph_idx_to_word_idxs = [np.arange(len(s)) for s in ph_seqs]
@@ -339,8 +480,10 @@ class AlignmentDecoder:
                                 for s in ph_seqs]) if n else np.zeros(0, bool)
         word_idx = np.concatenate([np.asarray(w, dtype=np.int64) for w in ph_idx_to_word_idxs]) \
             if n else np.zeros(0, np.int64)
-        plan, views, fc, _ = self._run(frames, edges, ids_list, want_frame_confidence)
-        return BatchAlignment(plan, views, ph_seqs, word_seqs, ph_idx_to_word_idxs, is_sp, word_idx, fc)
+        plan, views, out, _ = self._run(frames, edges, ids_list, want_frame_confidence, ctcs, want_frame_states)
+        return BatchAlignment(plan, views, ph_seqs, word_seqs, ph_idx_to_word_idxs, is_sp, word_idx,
+                              out["frame_conf"], out.get("ctc"), out.get("frame_state"),
+                              list(zip(frames, edges, ids_list)) if ctcs is not None or want_frame_states else None)
 
     # ----------------------------------------------------------------------------------------
     # attributes the reference fills eagerly (ad:73-78,86) and only validation consumes: lazily here
@@ -351,29 +494,18 @@ class AlignmentDecoder:
             self._lazy[key] = fn()
         return self._lazy[key]
 
-    def _masked_logits(self):
-        drop = np.ones(self.vocab["vocab_size"], dtype=bool)
-        drop[self.ph_seq_id] = False
-        drop[0] = False
-        pen = torch.from_numpy(drop).to(self._frame_logits.device)[None, None, :] * 1e9
-        return self._frame_logits.float() - pen.float()
-
     def __getattribute__(self, name):
         if name in ("ph_frame_pred", "ctc_logits", "edge_prob"):
             d = object.__getattribute__(self, "__dict__")
             if d.get("_lazy") is not None:
                 if name == "ph_frame_pred":                                        # ad:56-59,73
-                    return self._lazy_get(name, lambda: torch.nn.functional.softmax(
-                        self._masked_logits(), dim=-1).squeeze(0).cpu().numpy().astype("float32"))
+                    return self._lazy_get(name, lambda: _ph_frame_pred(self._frame_logits, self.ph_seq_id,
+                                                                       self.vocab["vocab_size"]))
                 if name == "ctc_logits":                                           # ad:76-78
                     return self._lazy_get(name, lambda: None if self._ctc_src is None else
                                           self._ctc_src.float().squeeze(0).cpu().numpy().astype("float32"))
                 if name == "edge_prob":                                            # ad:68-71,84
-                    def _edge():
-                        p = (((torch.sigmoid(self._edge_logits.float()) - 0.1) / 0.8).clamp(0.0, 1.0)
-                             ).squeeze(0).cpu().numpy().astype("float32")
-                        return (p + np.concatenate(([0], p[:-1]))).clip(0, 1)
-                    return self._lazy_get(name, _edge)
+                    return self._lazy_get(name, lambda: _edge_prob(self._edge_logits))
         return object.__getattribute__(self, name)
 
     def ctc(self):

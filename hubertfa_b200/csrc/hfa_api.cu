@@ -19,8 +19,6 @@
 #include "../../include/hfa_align.h"
 #include "hfa_common.cuh"
 
-#define HFA_EMIS_ROWS 64
-
 cudaError_t hfa_launch_unpack_emissions(const HfaLaunchCtx &c, int total_row_blocks, float *out);
 cudaError_t hfa_launch_dp_warp_any(const HfaLaunchCtx &c, int max_k, int max_pair_k, const int32_t *order, int n,
                                    float *dp_dump);
@@ -41,6 +39,10 @@ cudaError_t hfa_launch_unpack_bp(const HfaLaunchCtx &c, int utt, int8_t *out);
 cudaError_t hfa_launch_unpack_dp(const HfaLaunchCtx &c, int utt, float *out);
 cudaError_t hfa_launch_ctc_greedy(const void *logits, int dtype, int T, int V, int64_t st_t, int64_t st_v,
                                   int32_t *arg, int32_t *out_ids, int32_t *out_len, cudaStream_t stream);
+cudaError_t hfa_launch_ctc_batch(const HfaLaunchCtx &c, int total_row_blocks, const HfaCtcDesc *table, int V,
+                                 int dtype, int32_t *arg, int32_t *out_ids, int32_t *out_len);
+cudaError_t hfa_launch_frame_states(const HfaLaunchCtx &c, int total_row_blocks, const HfaResultPtrs &res,
+                                    int32_t *out);
 cudaError_t hfa_launch_jump_tables(const HfaLaunchCtx &c, int n_blocks);
 cudaError_t hfa_launch_backtrace_tables(const HfaLaunchCtx &c, const int32_t *order, int n,
                                         const HfaResultPtrs &res, float *frame_conf, float *dp_path);
@@ -1183,6 +1185,38 @@ int hfa_ctc_greedy(const void *logits, int32_t dtype, int64_t T, int64_t V, int6
     cudaError_t e = hfa_launch_ctc_greedy(logits, dtype, (int)T, (int)V, stride_t, stride_v, scratch, out_ids,
                                           out_len, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return cuda_fail(e, "hfa_ctc_greedy: launch");
+    g_launches += 1;
+    return HFA_OK;
+}
+
+int hfa_ctc_greedy_batch(const hfa_plan *p, void *workspace, const HfaCtcDesc *table, int64_t V, int32_t dtype,
+                         int32_t *scratch, int32_t *out_ids, int32_t *out_len, void *stream)
+{
+    if (!p || !workspace) return fail(HFA_ERR_ARG, "hfa_ctc_greedy_batch: NULL plan/workspace");
+    if (V < 1 || V > INT32_MAX || dtype < 0 || dtype > 2)
+        return fail(HFA_ERR_ARG, "hfa_ctc_greedy_batch: bad width / dtype (V=%lld, dtype=%d)", (long long)V, dtype);
+    if (p->n_utt == 0) return HFA_OK;
+    if (!table || !scratch || !out_ids || !out_len) return fail(HFA_ERR_ARG, "hfa_ctc_greedy_batch: NULL argument");
+    HfaLaunchCtx c = make_ctx(p, workspace, stream);
+    // out_len is the kernel's per-utterance count of finished frames before it holds the lengths
+    cudaError_t e = cudaMemsetAsync(out_len, 0, (size_t)p->n_utt * sizeof(int32_t), c.stream);
+    if (e != cudaSuccess) return cuda_fail(e, "hfa_ctc_greedy_batch: out_len reset");
+    if (p->total_frames == 0) return HFA_OK;
+    e = hfa_launch_ctc_batch(c, p->row_blocks[p->n_utt], table, (int)V, dtype, scratch, out_ids, out_len);
+    if (e != cudaSuccess) return cuda_fail(e, "hfa_ctc_greedy_batch: launch");
+    g_launches += 1;
+    return HFA_OK;
+}
+
+int hfa_frame_states(const hfa_plan *p, void *workspace, const void *result, int32_t *out, void *stream)
+{
+    if (!p || !workspace) return fail(HFA_ERR_ARG, "hfa_frame_states: NULL plan/workspace");
+    if (p->n_utt == 0 || p->total_frames == 0) return HFA_OK;
+    if (!result || !out) return fail(HFA_ERR_ARG, "hfa_frame_states: NULL argument");
+    HfaLaunchCtx c = make_ctx(p, workspace, stream);
+    cudaError_t e = hfa_launch_frame_states(c, p->row_blocks[p->n_utt],
+                                            make_res(p, const_cast<void *>(result)), out);
+    if (e != cudaSuccess) return cuda_fail(e, "hfa_frame_states: launch");
     g_launches += 1;
     return HFA_OK;
 }

@@ -16,6 +16,7 @@
 #include <stdint.h>
 
 #define HFA_TILE_T 16            // frames per emission tile == frames per backpointer word
+#define HFA_EMIS_ROWS 64         // frames per row block (HfaWs::row_blocks / block_utt)
 #define HFA_WARP_MAX_K 8         // states per lane in the warp-per-utterance kernel
 #define HFA_WARP_MAX_S (32 * HFA_WARP_MAX_K)
 #define HFA_CTA_K 8              // states per thread in the CTA-per-utterance kernel

@@ -8,7 +8,6 @@
 // Algorithmic HBM bytes per frame: V*sizeof(in) + sizeof(in) (edge logit) read, 4*S + 12 written.
 #include "hfa_common.cuh"
 
-#define HFA_EMIS_ROWS 64
 #define HFA_EMIS_WARPS 8
 
 namespace {

@@ -135,6 +135,16 @@ class AlignPlan:
             check(self._lib.hfa_set_inputs_device(self._h, workspace.data_ptr(), table.data_ptr(),
                                                   int(max_row_stride), _stream_ptr()), "hfa_set_inputs_device")
 
+    CTC_DESC = np.dtype([("logits", np.int64), ("stride_t", np.int64), ("stride_v", np.int64)])   # = HfaCtcDesc
+
+    def ctc_table(self, ptrs, stride_t, stride_v) -> np.ndarray:
+        """Host image of the per-utterance ctc logits table (HfaCtcDesc[n_utt], uint8 array) that
+        ``ctc_greedy_batch`` reads from the device: pointers and element strides, one entry per utterance."""
+        tab = np.zeros(self.n_utt, dtype=self.CTC_DESC)
+        for name, a in zip(self.CTC_DESC.names, (ptrs, stride_t, stride_v)):
+            tab[name] = np.asarray(a, dtype=np.int64)
+        return tab.view(np.uint8)
+
     def views(self, blob: np.ndarray) -> dict:
         """Typed numpy views into a host copy of the result blob."""
         L, n, ns = self.layout, self.n_utt, self.total_states
@@ -228,6 +238,33 @@ def forward_fused(workspace: torch.Tensor, plan: int, dtype: int) -> None:
     raises HfaError when the plan / inputs do not qualify)."""
     with torch.cuda.device(workspace.device):
         check(_lib.load().hfa_forward_fused(plan, workspace.data_ptr(), dtype, _stream_ptr()), "hfa_forward_fused")
+
+
+@torch.library.custom_op("hfa::ctc_greedy_batch", mutates_args=("scratch", "out_ids", "out_len"),
+                         device_types="cuda")
+def ctc_greedy_batch(workspace: torch.Tensor, plan: int, table: torch.Tensor, V: int, dtype: int,
+                     scratch: torch.Tensor, out_ids: torch.Tensor, out_len: torch.Tensor) -> None:
+    """Greedy CTC decode of every utterance of the plan in one launch (hfa_ctc_greedy_batch).  table: device
+    uint8 tensor with HfaCtcDesc[n_utt] (``AlignPlan.ctc_table``); scratch / out_ids: int32 [sum T]; out_len:
+    int32 [n_utt].  Utterance b's ids: out_ids[frame_off[b] : frame_off[b] + out_len[b]]."""
+    for t, what in ((scratch, "scratch"), (out_ids, "out_ids"), (out_len, "out_len")):
+        if t.dtype != torch.int32:
+            raise HfaError(f"ctc_greedy_batch: {what} must be int32")
+    with torch.cuda.device(workspace.device):
+        check(_lib.load().hfa_ctc_greedy_batch(plan, workspace.data_ptr(), table.data_ptr(), V, dtype,
+                                               scratch.data_ptr(), out_ids.data_ptr(), out_len.data_ptr(),
+                                               _stream_ptr()), "hfa_ctc_greedy_batch")
+
+
+@torch.library.custom_op("hfa::frame_states", mutates_args=("out",), device_types="cuda")
+def frame_states(workspace: torch.Tensor, plan: int, result: torch.Tensor, out: torch.Tensor) -> None:
+    """Per-frame state index of the best paths in ``result`` (hfa_frame_states): out int32 [sum T], ragged by
+    the plan's frame offsets."""
+    if out.dtype != torch.int32:
+        raise HfaError("frame_states: out must be int32")
+    with torch.cuda.device(workspace.device):
+        check(_lib.load().hfa_frame_states(plan, workspace.data_ptr(), result.data_ptr(), out.data_ptr(),
+                                           _stream_ptr()), "hfa_frame_states")
 
 
 class GraphedStep:

@@ -210,6 +210,31 @@ int64_t hfa_plan_algorithmic_bytes_fused(const hfa_plan *plan, int32_t dtype);
 int hfa_ctc_greedy(const void *logits, int32_t dtype, int64_t T, int64_t V, int64_t stride_t,
                    int64_t stride_v, int32_t *scratch, int32_t *out_ids, int32_t *out_len, void *stream);
 
+/* ---- validation of a whole batch (validation_step, networks/task/forced_alignment.py:407-414) ---- */
+/* The same greedy decode for every utterance of a plan in one launch (:145-150, what ctc() returns after
+ * decode() of each utterance).  table: [dev] HfaCtcDesc[n_utt]: utterance b's ctc logits, element (t, v) at
+ * logits[t*stride_t + v*stride_v] (elements; views of the head output are fine), with at least T[b] rows; one
+ * width V and one dtype (HFA_DTYPE_*) for the batch.  scratch: [dev] int32 [sum T] (the per-frame argmax).
+ * out_ids: [dev] int32 [sum T], ragged by hfa_plan_frame_offsets(): utterance b's ids are
+ * out_ids[frame_off[b] .. frame_off[b] + out_len[b]).  out_len: [dev] int32 [n_utt]; 0 for the utterances the
+ * plan did not accept.  Reads only the plan's uploaded tables besides its arguments: capturable into a CUDA
+ * graph (a memset of out_len and one kernel). */
+typedef struct HfaCtcDesc {
+    const void *logits;       /* [dev] ctc logits of the utterance */
+    int64_t stride_t, stride_v;   /* in elements */
+} HfaCtcDesc;
+int hfa_ctc_greedy_batch(const hfa_plan *plan, void *workspace, const HfaCtcDesc *table /*[dev]*/, int64_t V,
+                         int32_t dtype, int32_t *scratch /*[dev] sum T*/, int32_t *out_ids, int32_t *out_len,
+                         void *stream);
+
+/* The state index the best path occupies at every frame (:152-161, the ph_idx_frame plot() builds with a
+ * cumsum): out[frame_off[b] + t] = ph_idx_seq[k] of the largest k with ph_time_int[k] <= t, for every utterance
+ * the plan accepted, infeasible ones included (the others have no frames).  result: [dev] the blob
+ * hfa_align_batch / hfa_backtrace wrote with this plan; out: [dev] int32 [sum T].  Reads only the blob and the
+ * plan's uploaded tables: one kernel, capturable into a CUDA graph after hfa_align_batch. */
+int hfa_frame_states(const hfa_plan *plan, void *workspace, const void *result /*[dev]*/,
+                     int32_t *out /*[dev] sum T*/, void *stream);
+
 /* ---- introspection for tests: unpacked backpointers of one utterance ------------------------ */
 /* out: [dev] int8 [T_b][S_b], codes 0/1/2 (row 0 is -1 like the reference, :247). */
 int hfa_debug_unpack_backptr(const hfa_plan *plan, const void *workspace, int32_t utt, int8_t *out,
