@@ -26,7 +26,7 @@ cudaError_t hfa_launch_dp_cta(const HfaLaunchCtx &c, const int32_t *order, int n
 cudaError_t hfa_launch_dp_band(const HfaLaunchCtx &c, int k, int item_begin, int n_items, int32_t *ticket,
                                bool keep_dp, int64_t fused_row_stride, float *dp_dump);
 cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int ctas_per_sm, int item_begin, int n_items,
-                               int32_t *ticket, bool keep_dp, float *dp_dump);
+                               int32_t *ticket, bool keep_dp, int force_slow, float *dp_dump);
 cudaError_t hfa_launch_emission(const HfaLaunchCtx &c, int total_row_blocks, int max_sp, int dtype,
                                 int64_t max_row_stride, int *n_launched);
 cudaError_t hfa_launch_edge(const HfaLaunchCtx &c, int total_row_blocks, int dtype);
@@ -75,10 +75,6 @@ typedef CUresult (*HfaEncodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_
                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 HfaEncodeTiled tensor_map_encoder()
 {
-    // HFA_NO_TENSORMAP=1 (read on every call, so tests can flip it): the band kernel's producer falls
-    // back to one 1-D bulk copy per frame row
-    if (const char *e = std::getenv("HFA_NO_TENSORMAP"))
-        if (e[0] == '1') return nullptr;
     static const HfaEncodeTiled fn = [] {
         void *f = nullptr;
         cudaDriverEntryPointQueryResult q;
@@ -192,6 +188,10 @@ struct hfa_plan {
     int32_t band_skew[2] = {0, 0};
     // strips of the skewed kernel resident per SM (4 or 5: the kernel's ring has 6 or 5 stages)
     int32_t skew_ctas[2] = {5, 5};
+    int32_t skew_slow = 0;                     // 1: every block of the skewed kernel through its guarded body
+    // true: the strips and bands read their emission tiles through TMA tensor maps, which hfa_plan_upload writes;
+    // false: the halo bands take the strips' place and their producers copy one frame row at a time
+    bool use_tmaps = false;
     int64_t band_xchg_elems = 0, dp_store_elems = 0;
     std::vector<int32_t> jblk_utt, jblk_first; // jump-table kernel: 256-word blocks per utterance of the table set
     int32_t n_kept = 0;                        // utterances that keep dp
@@ -257,7 +257,7 @@ HfaWs make_ws(const hfa_plan *p, void *workspace)
     w.row_entry = reinterpret_cast<int32_t *>(b + p->o_rowent);
     w.jblk_utt = reinterpret_cast<const int32_t *>(b + p->o_jblk_utt);
     w.jblk_first = reinterpret_cast<const int32_t *>(b + p->o_jblk_first);
-    w.tmaps = (p->n_tmaps > 0 && tensor_map_encoder() != nullptr) ? b + p->o_tmaps : nullptr;
+    w.tmaps = (p->n_tmaps > 0 && p->use_tmaps) ? b + p->o_tmaps : nullptr;
     w.col_ids = reinterpret_cast<const int32_t *>(b + p->o_colids);
     w.colmap = reinterpret_cast<const uint8_t *>(b + p->o_colmap);
     w.emis_mode = reinterpret_cast<int32_t *>(b + p->o_emode);
@@ -311,6 +311,46 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                     vocab_size);
     hfa_plan *p = new (std::nothrow) hfa_plan();
     if (!p) return fail(HFA_ERR_NOMEM, "hfa_plan_create: out of host memory");
+
+    // Routing overrides (DESIGN §4.6), read here and nowhere else: the plan keeps what it read, and no call made
+    // with it looks at the environment again.  Unset, each leaves the planner's own choice.
+    // HFA_LATENCY_MODE: 0 never cut utterances with S <= 256 into strips / bands, 2 always, -1: by the budget below
+    int lat_mode = -1;
+    if (const char *e = std::getenv("HFA_LATENCY_MODE")) lat_mode = e[0] - '0';
+    // HFA_BAND_MAX: strip / band budget of the latency route and of the S > 256 list (3072: the measured crossover)
+    int64_t band_max = 3072;
+    if (const char *e = std::getenv("HFA_BAND_MAX")) band_max = std::atoll(e);
+    // HFA_SKEW_D = 2 | 3: frames of skew per state of the skewed kernel; HFA_LAT_KERNEL = band: halo bands instead
+    int skew_d = 2;
+    if (const char *e = std::getenv("HFA_SKEW_D")) skew_d = (std::atoi(e) == 3) ? 3 : 2;
+    if (const char *e = std::getenv("HFA_LAT_KERNEL")) { if (e[0] == 'b') skew_d = 0; }
+    // HFA_SKEW_SLOW = 1: every block of the skewed kernel through its guarded body
+    if (const char *e = std::getenv("HFA_SKEW_SLOW")) p->skew_slow = e[0] == '1' ? 1 : 0;
+    // HFA_SKEW_CTAS = 4 | 5: strips resident per SM, instead of the list schedule's choice
+    int force_ctas = 0;
+    if (const char *e = std::getenv("HFA_SKEW_CTAS")) force_ctas = std::atoi(e);
+    // HFA_BIG_KERNEL = cta | band: kernel of the S > 256 list (-1: by the budget); HFA_BIG_K = 2 | 4 | 8: states
+    // per lane of its halo bands
+    int big_mode = -1;
+    if (const char *e = std::getenv("HFA_BIG_KERNEL")) big_mode = (e[0] == 'b');
+    int big_k = 0;
+    if (const char *e = std::getenv("HFA_BIG_K")) big_k = std::atoi(e);
+    // HFA_KEEP_DP = 0: the strips and bands keep no dp (the backtrace re-scores the path)
+    bool keep_dp = true;
+    if (const char *e = std::getenv("HFA_KEEP_DP")) keep_dp = (e[0] != '0');
+    // HFA_BT_WALK = 0: jump tables instead of the shared-memory walk for every kept-dp utterance
+    int bt_walk = 2;
+    if (const char *e = std::getenv("HFA_BT_WALK")) bt_walk = std::atoi(e);
+    // HFA_PAIR = 0: never the SP-aware pair layout, 2: wherever possible, 1: where the cost rule picks it
+    int pair_mode = 1;
+    if (const char *e = std::getenv("HFA_PAIR")) pair_mode = std::atoi(e);
+    // HFA_COMPACT = 0: plain [T][Sp] emission rows for the pair layout
+    bool compact = true;
+    if (const char *e = std::getenv("HFA_COMPACT")) compact = e[0] != '0';
+    // HFA_NO_TENSORMAP = 1: no TMA tensor maps, as when the driver lacks cuTensorMapEncodeTiled
+    p->use_tmaps = tensor_map_encoder() != nullptr;
+    if (const char *e = std::getenv("HFA_NO_TENSORMAP")) { if (e[0] == '1') p->use_tmaps = false; }
+
     try {
         p->n_utt = n_utt;
         p->vocab = vocab_size;
@@ -398,15 +438,8 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         // its longest utterances.  Such batches go to the banded kernel (hfa_dp_band_kernel): every
         // utterance becomes several 2-states-per-lane warps on different SMs.  Big batches keep
         // one warp per utterance (no redundant halo work).
-        //   HFA_LATENCY_MODE = 0: never band (S <= 256) | 2: always band
-        //   | unset: strips / bands when the batch needs <= HFA_BAND_MAX
-        //   (default 3072) of them.   HFA_BIG_KERNEL = cta | band, HFA_BIG_K = 2|4|8.
         // Latency-regime kernel: the skewed wavefront (default; needs the TMA tensor maps) or the halo bands.
-        //   HFA_LAT_KERNEL = skew | band,   HFA_SKEW_D = 2 | 3 (frames of skew per state)
-        int skew_d = 2;
-        if (const char *e = std::getenv("HFA_SKEW_D")) skew_d = (std::atoi(e) == 3) ? 3 : 2;
-        if (const char *e = std::getenv("HFA_LAT_KERNEL")) { if (e[0] == 'b') skew_d = 0; }
-        if (tensor_map_encoder() == nullptr) skew_d = 0;
+        if (!p->use_tmaps) skew_d = 0;
         auto n_bands = [&](int32_t b, int k) {
             if (k == 1) return hfa_skew_strips(p->utt[b].Sp);
             const int w = 32 * k, own = w - 32, sp = p->utt[b].Sp;
@@ -415,12 +448,7 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         // measured crossover (profiles/r2_routing_crossover.json, B200): strips win for 256 / 512 utterances
         // (820 / 1674 strips: 0.22 vs 0.44 ms, 0.33 vs 0.48 ms per step), tie at 1024 (3310 strips: 0.550 vs
         // 0.553 ms), one warp per utterance wins at 2048 (6582 strips: 1.03 vs 0.73 ms)
-        int64_t band_max = 3072;
-        if (const char *e = std::getenv("HFA_BAND_MAX")) band_max = std::atoll(e);
-        int lat_mode = -1;
-        if (const char *e = std::getenv("HFA_LATENCY_MODE")) lat_mode = e[0] - '0';
         std::vector<int32_t> lat_band;
-        bool hybrid = false;             // lat_band holds only the costliest utterances of a big batch
         if (lat_mode != 0) {
             int64_t nb = 0;
             for (int c = 0; c < HFA_NUM_CLASSES; ++c)
@@ -436,57 +464,17 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                     p->class_count[c] = 0;
                 }
                 std::sort(lat_band.begin(), lat_band.end(), by_len);
-            } else if (skew_d > 0 && nb > 0) {
-                // Big batch, one warp per utterance -- except for its costliest utterances.  A single warp runs
-                // the recurrence of T frames x K states per lane at well under one instruction per cycle, so
-                // the few longest / widest utterances alone last about as long as the whole batch would on a
-                // perfectly filled machine, and the launch ends in a long, empty tail.  Those utterances are cut
-                // into strips of the skewed kernel instead (no redundant work, 2-5 warps each, no dp kept: they
-                // share the warp-per-utterance backtrace).  Cost unit: frames x states per lane; threshold =
-                // HFA_HYBRID x the per-scheduler share of the whole batch.
-                // MEASURED (B200, config 4): a loss -- DP stage 0.458 ms with no strips, 0.659 ms at 0.26 (2306
-                // strips), 0.917 ms at 0.15 (6758 strips): a strip spends ~1.5x the instructions per cell of the
-                // K-states-per-lane warp and holds 38 KB of shared memory.  Off by default; the knob stays.
-                double alpha = 0.0;
-                if (const char *e = std::getenv("HFA_HYBRID")) alpha = std::atof(e);
-                auto ucost = [&](int32_t b) { return (int64_t)p->utt[b].T * ((p->utt[b].Sp + 31) / 32); };
-                int64_t sum_cost = 0;
-                for (int c = 0; c < HFA_NUM_CLASSES; ++c)
-                    for (int32_t b : lists[c]) sum_cost += ucost(b);
-                const double thresh = alpha * (double)sum_cost / (4.0 * sm_count());
-                if (alpha > 0.0) {
-                    int64_t strips = 0;
-                    for (int c = 1; c < HFA_NUM_CLASSES; ++c) {   // class 0 (S <= 32) is a single strip anyway
-                        std::vector<int32_t> keep;
-                        for (int32_t b : lists[c]) {
-                            if ((double)ucost(b) >= thresh && strips + n_bands(b, 1) <= 8 * band_max) {
-                                lat_band.push_back(b);
-                                strips += n_bands(b, 1);
-                            } else {
-                                keep.push_back(b);
-                            }
-                        }
-                        lists[c].swap(keep);
-                        p->class_count[c] = (int32_t)lists[c].size();
-                    }
-                    std::sort(lat_band.begin(), lat_band.end(), by_len);
-                    hybrid = !lat_band.empty();
-                }
             }
         }
         std::vector<int32_t> big_band;
         {
             // states per lane of the long-sequence bands: as few as the band budget allows (measured on
             // config 3: 2.5 ms with 2, 3.8 ms with 4, 9.9 ms with 8, 17 ms in the CTA kernel)
-            int big_mode = -1;                               // -1 auto, 0 cta, 1 band
-            if (const char *e = std::getenv("HFA_BIG_KERNEL")) big_mode = (e[0] == 'b');
             auto count = [&](int k) {
                 int64_t nb = 0;
                 for (int32_t b : lists[HFA_NUM_CLASSES]) nb += n_bands(b, k);
                 return nb;
             };
-            int big_k = 0;
-            if (const char *e = std::getenv("HFA_BIG_K")) big_k = std::atoi(e);
             if (big_k != 2 && big_k != 4 && big_k != 8) {
                 big_k = 8;
                 for (int k : {2, 4, 8})
@@ -513,8 +501,6 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                 std::sort(big_band.begin(), big_band.end(), by_len);
             }
         }
-        bool keep_dp = true;
-        if (const char *e = std::getenv("HFA_KEEP_DP")) keep_dp = (e[0] != '0');
         auto add_bands = [&](const std::vector<int32_t> &utts, int which) {
             const int k = p->band_k[which];
             const int sd = p->band_skew[which];
@@ -528,7 +514,7 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
                 // instead of re-running the serial chain along the path
                 p->utt[b].band_k = k;
                 p->utt[b].tmap = p->n_tmaps++;
-                if (keep_dp && !(hybrid && which == 0)) {
+                if (keep_dp) {
                     p->utt[b].dp_off = p->dp_store_elems;
                     // bands: one [T][32 k] block per band; strips: one 128-byte row per iteration
                     p->dp_store_elems += sd > 0 ? (int64_t)nb * hfa_skew_blocks(sd, p->utt[b].T) * HFA_SKEW_BLK * 32
@@ -550,8 +536,6 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         // start in the first wave.  Four when the list schedule is not longer with them (configs 1-3: the
         // strips that miss the first wave belong to short utterances), five otherwise (512 utterances and up).
         // HFA_SKEW_CTAS = 4 | 5 forces one residency (tests run both ring sizes on the same batches).
-        int force_ctas = 0;
-        if (const char *e = std::getenv("HFA_SKEW_CTAS")) force_ctas = std::atoi(e);
         for (int wh = 0; wh < 2; ++wh) {
             if (p->band_skew[wh] <= 0 || p->band_count[wh] == 0) continue;
             if (force_ctas == 4 || force_ctas == 5) {
@@ -570,8 +554,6 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         // walk wins on every batch it fits, 256 utterances of T = 500-6000 and S = 40-256 up to 192 KB of words
         // at one CTA per SM, so an utterance takes it whenever its words fit in one CTA's shared memory; giants
         // (S > 8192) keep the tables.  HFA_BT_WALK = 0: never (tests compare the two routes).
-        int bt_walk = 2;
-        if (const char *e = std::getenv("HFA_BT_WALK")) bt_walk = std::atoi(e);
         std::vector<int32_t> walk_list, tab_list;
         std::vector<char> walks((size_t)n_utt, 0);
         for (int32_t b : all) {
@@ -607,8 +589,6 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         // So: if the frames-weighted instruction count of the possible utterances is lower in pairs, all of them
         // go there.  Instructions per frame counted in the SASS (loop bodies + the per-tile work / 8):
         // 16 + 21 K plain, 17 + 25 KP in pairs.   HFA_PAIR = 0: never | 2: whenever possible | unset: as above.
-        int pair_mode = 1;
-        if (const char *e = std::getenv("HFA_PAIR")) pair_mode = std::atoi(e);
         std::vector<int32_t> warp_all;
         std::vector<std::pair<int32_t, int>> pairable;          // (utterance, pairs per lane)
         int64_t sum_pair = 0, sum_plain = 0;
@@ -634,9 +614,8 @@ int hfa_plan_create(int32_t n_utt, int32_t vocab_size, const int32_t *T, const i
         }
         // Compacted emission rows for those utterances (HfaWs::colmap): every slot of the pair layout reads its
         // column through its own address register, so pointing states with the same id at ONE column is free.
-        // HFA_COMPACT=0 keeps the plain [T][Sp] rows.
-        bool compact = vocab_size <= 255;
-        if (const char *e = std::getenv("HFA_COMPACT")) compact = compact && e[0] != '0';
+        // HFA_COMPACT=0 keeps the plain [T][Sp] rows, and so does V > 255 (a colmap entry is one byte).
+        compact = compact && vocab_size <= 255;
         p->col_ids.assign((size_t)(p->total_states + 4 * (int64_t)n_utt), vocab_size);
         p->colmap.assign((size_t)p->total_states, 0);
         if (pair_mode >= 2 || sum_pair < sum_plain)
@@ -854,7 +833,7 @@ int hfa_plan_upload(const hfa_plan *p, void *workspace, void *stream)
     cudaError_t e = cudaMemcpyAsync(workspace, p->head.data(), (size_t)p->head_bytes,
                                     cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return cuda_fail(e, "hfa_plan_upload");
-    if (p->n_tmaps > 0 && tensor_map_encoder() != nullptr) try {
+    if (p->n_tmaps > 0 && p->use_tmaps) try {
         // TMA tensor maps over emis[t][s] of the banded utterances (they hold the workspace address, so
         // they are built here): rank 2, f32, dims {Sp, T}, row pitch Sp * 4 B, box {32 K, 16}
         std::vector<CUtensorMap> maps((size_t)p->n_tmaps);
@@ -971,8 +950,7 @@ int hfa_emission(const hfa_plan *p, void *workspace, int32_t dtype, void *stream
     if (p->n_utt == 0 || p->total_frames == 0) return HFA_OK;
     if (dtype < 0 || dtype > 2) return fail(HFA_ERR_ARG, "hfa_emission: bad dtype %d", dtype);
     HfaLaunchCtx c = make_ctx(p, workspace, stream);
-    static const bool no_tma = [] { const char *v = std::getenv("HFA_EMISSION_NO_TMA"); return v && v[0] == '1'; }();
-    const int64_t row_stride = no_tma ? 0 : p->row_stride_of(workspace);
+    const int64_t row_stride = p->row_stride_of(workspace);
     // The persistent (TMA) emission kernel leaves the edge stream to its own small kernel, forked
     // onto a side stream so that the two overlap and joined before anything downstream.  The fork
     // point has to be recorded BEFORE the emission launch is queued.
@@ -1058,7 +1036,7 @@ static int viterbi_forward_impl(const hfa_plan *p, void *workspace, float *dp_du
             const int wh = items[it].k == -3 ? 0 : 1;
             if (p->band_skew[wh] > 0)
                 e = hfa_launch_dp_skew(c, p->band_skew[wh], p->skew_ctas[wh], p->band_begin[wh], p->band_count[wh],
-                                       c.ws.band_ticket + wh, p->dp_store_elems > 0, dp_dump);
+                                       c.ws.band_ticket + wh, p->dp_store_elems > 0, p->skew_slow, dp_dump);
             else
                 e = hfa_launch_dp_band(c, p->band_k[wh], p->band_begin[wh], p->band_count[wh],
                                        c.ws.band_ticket + wh, p->dp_store_elems > 0, fused_row_stride, dp_dump);
@@ -1155,17 +1133,16 @@ int hfa_align_batch(const hfa_plan *p, void *workspace, int32_t dtype, void *res
     // Fused route (small batches): when every utterance is in the banded kernel, keeps its dp, and
     // the logits are f32 rows the TMA engine can fetch, the emission stage disappears -- only the
     // edge stream is computed up front, the emissions are produced inside the DP kernel's producer
-    // warps and never written to HBM.  HFA_FUSED=0 keeps the three-stage route.
+    // warps and never written to HBM.
     // Measured (B200): the fused route wins when no utterance is split into several bands (config 1:
     // 0.137 vs 0.173 ms per decode) and loses otherwise -- every band of an utterance recomputes the
     // softmax normaliser of its frames, and a single producer warp then cannot keep up with its
-    // compute warp (config 2: 0.29 vs 0.22 ms).  HFA_FUSED=0 / 1 forces the choice.
-    static const int fused_mode = [] { const char *v = std::getenv("HFA_FUSED"); return v ? (v[0] == '1' ? 1 : 0) : -1; }();
+    // compute warp (config 2: 0.29 vs 0.22 ms).
     int64_t n_valid = 0;
     for (const HfaUtt &m : p->utt) n_valid += (m.status == 0);
     const bool unsplit = (int64_t)p->band_items.size() == n_valid;
     int rc;
-    if ((fused_mode == 1 || (fused_mode == -1 && unsplit)) && fused_ok(p, workspace, dtype)) {
+    if (unsplit && fused_ok(p, workspace, dtype)) {
         rc = hfa_forward_fused(p, workspace, dtype, stream);
     } else {
         rc = hfa_emission(p, workspace, dtype, stream);

@@ -1326,13 +1326,10 @@ cudaError_t hfa_launch_dp_warp_any(const HfaLaunchCtx &c, int max_k, int max_pai
                                     hfa_warp_smem_bytes<3>(), hfa_warp_smem_bytes<4>(),
                                     hfa_warp_smem_bytes<5>(), hfa_warp_smem_bytes<6>(),
                                     hfa_warp_smem_bytes<7>(), hfa_warp_smem_bytes<8>()};
-    size_t smem = (bytes[max_k] + 127) & ~(size_t)127;
-    // HFA_DP_WARPS_PER_SM=n caps the resident warps per SM by padding the shared-memory request
-    // (experiment knob; measured on config 4: flat from 13 warps per SM upwards)
-    static const int cap = [] { const char *e = getenv("HFA_DP_WARPS_PER_SM"); return e ? atoi(e) : 0; }();
-    if (cap > 0) smem = std::max(smem, ((size_t)(227 * 1024) / (size_t)cap - 1024) & ~(size_t)127);
-    // (register-leaner variants compiled for the largest class present -- 72 registers for K <= 5 --
-    // and 2 instead of 3 emission stages were measured on config 4: no gain, 0.465 vs 0.459 ms)
+    const size_t smem = (bytes[max_k] + 127) & ~(size_t)127;
+    // Measured on config 4, no gain: capping the resident warps per SM by padding this request (flat from 13 warps
+    // per SM upwards); register-leaner variants compiled for the largest class present (72 registers for K <= 5)
+    // with 2 instead of 3 emission stages (0.465 vs 0.459 ms).
     if (dp_dump != nullptr) return launch_any<true, 8>(c, smem, order, n, dp_dump);
     return launch_any<false, 8>(c, smem, order, n, dp_dump);
 }

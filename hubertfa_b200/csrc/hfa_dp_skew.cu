@@ -573,15 +573,13 @@ cudaError_t launch_skew_d(const HfaLaunchCtx &c, int item_begin, int n_items, in
 // d = frames of skew per state (2 or 3, fixed when the plan was made: the dp store layout depends on it).
 // ctas_per_sm = strips resident per SM, the plan's choice: a ring of 5 stages (43 144 B of shared memory) lets
 // 5 CTAs share an SM, 6 stages (48 032 B) only 4 -- one compute warp per scheduler partition, one more tile
-// fetched ahead.
+// fetched ahead.  force_slow = 1: every block through the guarded body (tests compare it with the unrolled steady
+// state).
 cudaError_t hfa_launch_dp_skew(const HfaLaunchCtx &c, int d, int ctas_per_sm, int item_begin, int n_items,
-                               int32_t *ticket, bool keep_dp, float *dp_dump)
+                               int32_t *ticket, bool keep_dp, int force_slow, float *dp_dump)
 {
     if (n_items <= 0) return cudaSuccess;
     if (c.ws.tmaps == nullptr) return cudaErrorNotSupported;
-    // HFA_SKEW_SLOW=1: every block through the guarded body (A/B against the unrolled steady state)
-    const char *sl = getenv("HFA_SKEW_SLOW");
-    const int force_slow = (sl && sl[0] == '1') ? 1 : 0;
     if (ctas_per_sm == 4) {
         if (d == 2) return launch_skew_d<2, 6>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);
         if (d == 3) return launch_skew_d<3, 6>(c, item_begin, n_items, ticket, keep_dp, dp_dump, force_slow);

@@ -7,7 +7,7 @@ all -inf gives -inf emissions, as in the reference (its masked logits stay finit
 logit is -inf gives -inf too, where the reference gives NaN (a deliberate divergence).  NaN, +inf and
 |x| >= 5e8 are out of contract.
 
-Which kernel runs follows from the inputs (HFA_EMISSION_NO_TMA and HFA_FUSED are read once per process):
+Which kernel runs follows from the inputs alone (no environment variable selects one):
   stream  unit column stride and a 64-row stage of at most 48 KiB (f32 head views [T, V+2] up to V = 189)
   block   column stride != 1 (a transposed view), or a larger stage (f32 head views, V = 190 .. 255)
   wide    V >= 256
